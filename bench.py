@@ -2,6 +2,7 @@
 """bench.py -- benchmark of the photomosaic best-fit path on the BASELINE.json configurations.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg4|cfg2|cfg3|cfg5|...] [--configs all|none]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[3], SURVEY.md section 8d "Config 4"): synthetic 7680x4320 main image x 10,000-image
 library of 128x128 tiles, CIEDE2000, square cells 128, detail 100 %, repeat range 8 / addition 500. A "step" is one complete
@@ -22,6 +23,10 @@ roofline: the binding EXECUTED pipe of the difference kernel (FP32 lane-ops or M
           against the pipe rates measured live by the in-library micro-benchmark).
 The CPU oracle package (the reference's own generator compiled into oracle/_ref) is imported ONLY by the cpu_baseline leg and
 by --impl reference; the B200 arm builds everything it needs with the product.
+--dump-outputs DIR: after the run, DIR/<workload>_best_fits<step>.npy (float64) holds the best-fit grid of every size step that the
+last timed step of each B200 workload returned (getBestFits: library index per cell, -1 outside the grid state). The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
+bench.py writes nothing into the source tree (no bytecode either), so it runs from a read-only checkout.
 """
 import argparse
 import hashlib
@@ -34,6 +39,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the modules imported below (package, oracle, tools/) leave no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -89,7 +95,28 @@ def parse():
                     help="all: after the headline workload also run BASELINE configs 2, 3 and 5 (a few steps each) into the `configs` object")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=45.0, help="target CPU time of the full-library cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the best-fit grids of the last timed step of every B200 workload to DIR/<workload>_best_fits<step>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        # that arm times the CPU generator on a sample of cells per step, not the whole grid: there is no grid to compare
+        ap.error("--dump-outputs writes the B200 arm's best-fit grids; --impl reference computes no whole grid")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, grids_of):
+    """grids_of: workload name -> list of best-fit grids (one per size step), written as float64 .npy files (exact for indices)."""
+    arrays = {"%s_best_fits%d" % (name, i): g.astype(np.float64) for name, grids in grids_of.items() for i, g in enumerate(grids)}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs to dump: %d bytes" % total  # a grid has one entry per cell: a few hundred KB at most
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- shared by both arms (no oracle, no GPU)
@@ -163,6 +190,7 @@ class ClockSampler:
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait(timeout=10)
         self.t.join(timeout=2)
         num = lambda s: s.replace(".", "").isdigit()
         sm = [float(r[1]) for r in self.rows if len(r) >= 9 and num(r[1])]
@@ -491,6 +519,7 @@ class B200Run:
             launches += tm["kernel_launches"]
         self.barrier()
         elapsed = time.perf_counter() - t0
+        timed_grids = grids
         clk = clocks.stop() if clocks else None
         pixel_diffs = tm["pixel_diffs"]  # whole job (every rank counts all cells of the step)
         local_share = 1.0
@@ -512,7 +541,7 @@ class B200Run:
         return {"elapsed": elapsed, "steps": steps, "phase": phase, "launches": int(launches), "pixel_diffs": pixel_diffs,
                 "pixel_diffs_nominal": tm["pixel_diffs_nominal"], "local_share": local_share, "clocks": clk, "e2e_elapsed": e2e_elapsed,
                 "e2e_steps": e2e_steps, "checksum": checksum, "h2d": int(self.h2d_main + self.h2d_lib),
-                "d2h": int(sum(g.size * 8 for g in grids))}
+                "d2h": int(sum(g.size * 8 for g in grids)), "grids": timed_grids}
 
     def tie_band(self):
         """cells whose best two penalised candidates are within an FP32-explainable tolerance (untimed, 1 GPU)"""
@@ -620,6 +649,7 @@ def main():
     run = B200Run(args.workload, cfg, rank, world, local_rank)
     m = run.measure(args.steps, args.warmup, max(1, min(args.steps, 3)), sample_clocks=True)
     m["valid_cells"] = run.valid_cells
+    outputs = {args.workload: m["grids"]}
     mb = np.zeros(12)
     capi().mosaic_kernel_microbench(local_rank, mb.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), 12)
     head = summarise(args.workload, cfg, m, world, roofline_of(args.workload, cfg, m, mb, peaks, sass, world))
@@ -645,6 +675,7 @@ def main():
             (one,) = r2.allmax([max(time.perf_counter() - t_w, 1e-3)])
             m2 = r2.measure(min(args.steps, 5), max(3, min(50, int(0.5 / one))), 2, sample_clocks=True)
             m2["valid_cells"] = r2.valid_cells
+            outputs[name] = m2["grids"]
             s2 = summarise(name, c2, m2, world, roofline_of(name, c2, m2, mb, peaks, sass, world))
             s2["clocks"] = m2["clocks"]
             if world == 1:
@@ -669,6 +700,8 @@ def main():
             out["cpu_baseline"] = cpu
         if configs:
             out["configs"] = configs
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

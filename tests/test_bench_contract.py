@@ -36,6 +36,33 @@ def test_other_ranks_of_the_reference_arm_do_nothing():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_reference_arm_refuses_to_dump_outputs(tmp_path):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "d")],
+                       capture_output=True, text=True, timeout=120, env=dict(os.environ, RANK="0", WORLD_SIZE="1"))
+    assert p.returncode != 0 and "--dump-outputs" in p.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_b200_arm_dumps_the_same_outputs_on_every_run(tmp_path):
+    """--dump-outputs: the best-fit grid of the last timed step, float64, identical for two runs with the same arguments."""
+    import numpy as np
+    grids = []
+    for run in range(2):
+        out = tmp_path / ("run%d" % run)
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                            "--workload", "cfg4-small", "--configs", "none", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=600, env=dict(os.environ, RANK="0", WORLD_SIZE="1"))
+        assert p.returncode == 0, p.stderr[-2000:]
+        line = json.loads(p.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 2
+        assert sorted(os.listdir(out)) == ["cfg4-small_best_fits0.npy"]
+        g = np.load(out / "cfg4-small_best_fits0.npy")
+        assert g.dtype == np.float64 and g.shape == (11, 17)  # 1080 x 1920 in 128 px cells (GridGenerator's grid, edge ring included)
+        assert int((g >= 0).sum()) == line["valid_cells"] and g.max() < 1000 and np.array_equal(g, np.round(g))
+        grids.append(g)
+    assert np.array_equal(grids[0], grids[1])
+
+
 def test_b200_arm_fails_loudly_without_a_device():
     import torch
     if torch.cuda.is_available():

@@ -1,6 +1,6 @@
 """File formats either side of the path (.mil library, .mcs cell shape): round trips like the reference's
 ImageLibrary.SaveAndLoad / CellShape.SaveAndLoad tests (test/tst_ImageLibrary.h, test/tst_CellShape.h), and the
-reference's own Cells/*.mcs fixtures when the checkout is present."""
+reference's own Cells/*.mcs files (committed under tests/golden/cells)."""
 import glob
 import os
 
@@ -8,6 +8,8 @@ import numpy as np
 import pytest
 
 pytest.importorskip("cv2")
+
+CELLS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cells")
 
 
 def test_mil_round_trip(tmp_path):
@@ -42,9 +44,7 @@ def test_mcs_round_trip(tmp_path):
 
 
 def test_reference_cell_fixtures(oracle):
-    files = sorted(glob.glob("/root/reference/Cells/*.mcs"))
-    if not files:
-        pytest.skip("reference checkout not present")
+    files = sorted(glob.glob(os.path.join(CELLS, "*.mcs")))
     from mosaicmagnifique_b200 import formats
     assert len(files) == 10
     for p in files:
@@ -53,7 +53,7 @@ def test_reference_cell_fixtures(oracle):
         assert f["version"] == 8 and f["mask"].shape == (512, 512)
         assert np.array_equal(np.where(f["mask"] > 127, 255, 0), o.mask)
         assert [f[k] for k in ("row_spacing", "col_spacing", "alt_row_spacing", "alt_col_spacing", "alt_row_offset", "alt_col_offset")] == o.params()[1:7]
-    hexa = formats.load_mcs("/root/reference/Cells/Hexagon.mcs")
+    hexa = formats.load_mcs(os.path.join(CELLS, "Hexagon.mcs"))
     assert (hexa["row_spacing"], hexa["col_spacing"], hexa["alt_row_offset"]) == (385, 440, 220)  # SURVEY.md section 8a
 
 

@@ -2,8 +2,8 @@
 
 The ten `Cells/*.mcs` of the reference are committed under tests/golden/cells/ (reference-held fixtures) and read with the
 product's own reader (mosaic_mcs_load: QDataStream layout + PNG codec in csrc/containers.cpp). The CUDA path is compared with
-the reference's OWN generator object code (oracle/_ref/libref_core.so, which travels to the GPU box prebuilt) exactly as
-tests/test_gpu_generator.py::_direct_reference_case does: identical grid states, identical best-fit grids outside the tie band.
+the reference generator's answer -- its own object code where oracle/_ref/libref_core.so is built, else the stored answer in
+tests/golden/reference_grids.npz (which records its source) -- exactly as tests/test_gpu_generator.py::_direct_reference_case does: identical grid states, identical best-fit grids outside the tie band.
 
   config 2  Hexagon.mcs @128 (spacing 96/110, odd-row offset 55), detail 50 %, CIEDE2000, SampleImages main image
             (tst_Generator.h:80-90, 327-371: CreateHexagonCellGroup(128, 0, 50)); IsocelesTriangle(-45deg) as the flip case
@@ -44,11 +44,6 @@ def sample_image(scale):
     return cv2.resize(img, None, fx=scale, fy=scale, interpolation=cv2.INTER_AREA)
 
 
-def _need_ref(oracle):
-    if not oracle.reference_generator_available():
-        pytest.skip("oracle/_ref/libref_core.so (reference object code) not present / not loadable")
-
-
 def test_product_reader_equals_checker_reader(oracle):
     """mosaic_mcs_load (own PNG codec) against the cv2-based checker on every committed shape file (no GPU work, but kept with the
     config tests so that the fixtures the GPU cases run on are known to be read correctly on the box)."""
@@ -62,7 +57,6 @@ def test_config2_hexagon_mcs_ciede2000_detail50_sample_image(oracle):
     """configs[1]: SampleImages main image (x0.25 so that the CPU reference finishes in seconds), Hexagon.mcs resized to 128,
     detail 50 %, CIEDE2000, a 160-image substitute library (big-lib.mil is absent from the reference checkout: seeded crops of the
     sample image itself through the reference-equivalent ingest + synthetic images), repeats on."""
-    _need_ref(oracle)
     from mosaicmagnifique_b200 import synthetic
     o, _ = load_shape(oracle, "Hexagon")
     sh = o.resized(128)
@@ -70,14 +64,13 @@ def test_config2_hexagon_mcs_ciede2000_detail50_sample_image(oracle):
     main = sample_image(0.25)
     lib = synthetic.make_photo_library(sample_image(0.5), 96, 128, seed=2002)
     lib = np.concatenate([lib, synthetic.make_library(64, 128, 2003)])
-    n, n_diff = _direct_reference_case(oracle, main, lib, sh, 2, 50, 0, 2, 500)
+    n, n_diff = _direct_reference_case(oracle, "baseline-config2_hexagon", main, lib, sh, 2, 50, 0, 2, 500)
     assert n > 100
     print("config 2 (Hexagon.mcs, sample image): %d of %d cells differ from the reference (tie band)" % (n_diff, n))
 
 
 def test_config5_puzzle_mcs_rgb_detail50(oracle):
     """configs[4] shape: Puzzle.mcs resized to 128 (spacing 108, 72 % active), detail 50 %, RGB Euclidean."""
-    _need_ref(oracle)
     from mosaicmagnifique_b200 import synthetic
     o, _ = load_shape(oracle, "Puzzle")
     sh = o.resized(128)
@@ -85,7 +78,7 @@ def test_config5_puzzle_mcs_rgb_detail50(oracle):
     main = synthetic.make_main_image(1100, 1500, 505, block=64)
     lib = synthetic.make_library(300, 128, 506)
     for rr, ra in ((0, 0), (3, 2000)):  # BASELINE's config 5 has no repeats (fused argmin epilogue); and with the wavefront
-        n, n_diff = _direct_reference_case(oracle, main, lib, sh, 0, 50, 0, rr, ra)
+        n, n_diff = _direct_reference_case(oracle, "baseline-config5_puzzle-rr%d" % rr, main, lib, sh, 0, 50, 0, rr, ra)
         assert n > 120
         print("config 5 shape (Puzzle.mcs) repeats %d/%d: %d of %d cells differ from the reference (tie band)" % (rr, ra, n_diff, n))
 
@@ -94,7 +87,6 @@ def test_config5_puzzle_mcs_rgb_detail50(oracle):
 def test_every_reference_cell_shape(oracle, name):
     """All ten shipped shapes (flips on IsocelesTriangle: colV/rowV, IsocelesTriangle-45deg: all four, YinAndYang: colH/colV with
     alternate column spacing 0 -> clamped to 1 by resized()), resized to 64, detail 50 % and 100 %, one size step for half of them."""
-    _need_ref(oracle)
     from mosaicmagnifique_b200 import synthetic
     o, _ = load_shape(oracle, name)
     k = ALL_SHAPES.index(name)
@@ -104,7 +96,7 @@ def test_every_reference_cell_shape(oracle, name):
     diff = (2, 0, 1)[k % 3]
     detail = 50 if k % 2 == 0 else 100
     steps = 1 if k % 4 == 1 else 0
-    n, n_diff = _direct_reference_case(oracle, main, lib, sh, diff, detail, steps, 2, 300)
+    n, n_diff = _direct_reference_case(oracle, "baseline-shape-" + name, main, lib, sh, diff, detail, steps, 2, 300)
     assert n > 10
     print("%s: %d of %d cells differ from the reference (tie band)" % (name, n_diff, n))
 
@@ -114,7 +106,6 @@ def test_isoceles_45deg_flips_config2_style(oracle, all_four):
     """The flip case of config 2 at its own size: IsocelesTriangle-45deg.mcs @128, detail 50 %, CIEDE2000. The file switches all four
     flip flags on, which (column and row flips XOR-ed, GridUtility.cpp:101-132) yields the unflipped and the doubly flipped mask;
     with the alternate-row vertical flip switched off all four flipped masks occur in the grid (checked)."""
-    _need_ref(oracle)
     import ctypes
 
     from mosaicmagnifique_b200 import capi, synthetic
@@ -130,6 +121,6 @@ def test_isoceles_45deg_flips_config2_style(oracle, all_four):
     assert flips == ({0, 1, 2, 3} if all_four else {0, 3})
     main = synthetic.make_main_image(700, 900, 811, block=64)
     lib = synthetic.make_library(80, 128, 812)
-    n, n_diff = _direct_reference_case(oracle, main, lib, sh, 2, 50, 0, 2, 500)
+    n, n_diff = _direct_reference_case(oracle, "baseline-isoceles45-all_four%d" % all_four, main, lib, sh, 2, 50, 0, 2, 500)
     assert n > 60
     print("IsocelesTriangle-45deg @128 (flip states %s): %d of %d cells differ from the reference (tie band)" % (sorted(flips), n_diff, n))

@@ -10,7 +10,7 @@ import os
 import numpy as np
 import pytest
 
-CELLS = "/root/reference/Cells"
+CELLS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cells")  # the reference's Cells/*.mcs
 FIELDS = ("row_spacing", "col_spacing", "alt_row_spacing", "alt_col_spacing", "alt_row_offset", "alt_col_offset",
           "alt_col_flip_h", "alt_col_flip_v", "alt_row_flip_h", "alt_row_flip_v")
 
@@ -86,7 +86,6 @@ def test_product_group_matches_reference_object_code(ref):
         assert [g.shape for g in got] == [g.shape for g in want]
 
 
-@pytest.mark.skipif(not os.path.isdir(CELLS), reason="reference Cells/*.mcs not present")
 def test_mcs_files_of_the_reference(ref, tmp_path):
     """Every Cells/*.mcs of the reference: the reference's own loadFromFile vs the product reader (formats.load_mcs) and the
     oracle reader; then both writers round-trip through the other side's reader."""
@@ -253,7 +252,6 @@ def _capi_mcs_load(L, path):
     return c, mask, name.value.decode()
 
 
-@pytest.mark.skipif(not os.path.isdir(CELLS), reason="reference Cells/*.mcs not present")
 def test_capi_mcs_reader_and_writer_against_reference_object_code(ref, tmp_path):
     """mosaic_mcs_load / mosaic_mcs_save (own QDataStream layout, own PNG codec incl. inflate) on every Cells/*.mcs of the
     reference: equal to the reference's loadFromFile; the library's writer is read back by the reference."""
