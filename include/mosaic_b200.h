@@ -68,6 +68,8 @@ typedef struct mosaic_timings {
     double pixel_diffs;         /* active, in-bound mask pixels x library images x variants, all steps */
     double pixel_diffs_nominal; /* bounding-box pixels (detail size squared) x library x variants x valid cells */
     int64_t kernel_launches;    /* kernels this library launched inside the call */
+    double evaluated_pixel_diffs; /* pixel_diffs scaled by the share of the difference work actually executed: below pixel_diffs
+                                   * when exact pruning skipped pairs that cannot be selected */
 } mosaic_timings;
 
 typedef void (*mosaic_progress_fn)(int progress, void *user); /* signal progress(int), PhotomosaicGeneratorBase.h:78 */

@@ -21,7 +21,7 @@ class Timings(ctypes.Structure):
     _fields_ = [("preprocess_ms", ctypes.c_double), ("diff_ms", ctypes.c_double), ("select_ms", ctypes.c_double),
                 ("total_ms", ctypes.c_double), ("h2d_bytes", ctypes.c_double), ("d2h_bytes", ctypes.c_double),
                 ("pixel_diffs", ctypes.c_double), ("pixel_diffs_nominal", ctypes.c_double),
-                ("kernel_launches", ctypes.c_int64)]
+                ("kernel_launches", ctypes.c_int64), ("evaluated_pixel_diffs", ctypes.c_double)]
 
 
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_int, ctypes.c_void_p)

@@ -26,6 +26,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <cub/device/device_scan.cuh>
 
 #include "colour_math.cuh"
 #include "kernels.h"
@@ -79,6 +80,57 @@ constexpr int kThreads = (kConsumerWarps + 1) * 32;
 constexpr uint32_t kLibBlockBytes = MM_TNB * MM_KP * 16;
 constexpr uint32_t kCellBlockBytes = MM_TCB * MM_KP * 20;
 constexpr uint32_t kStageBytes = kLibBlockBytes + kCellBlockBytes;
+
+// Consumer side of the ring: warp `warp` walks nk chunks of its cell slot against the 8 library images of the stage and leaves,
+// per lane, the TNB running sums of the pixels it strode over. Shared by both kernels below, so that a pair's arithmetic (and the
+// measured loop body, DESIGN.md 4.1) is the same whichever launch computes it.
+template <int DIFF>
+__device__ __forceinline__ void consume_ring(const unsigned char *smem, uint64_t *full_bar, uint64_t *empty_bar, int nk, int warp,
+                                             int lane, float (&acc)[MM_TNB])
+{
+#pragma unroll
+    for (int i = 0; i < MM_TNB; ++i)
+        acc[i] = 0.0f;
+
+    for (int k = 0; k < nk; ++k) {
+        const int s = k % kStages;
+        mbar_wait(&full_bar[s], (k / kStages) & 1);
+        if (MM_STRESS_SKEW)
+            __nanosleep((unsigned)((warp * 97 + k * 29 + blockIdx.x * 7) % 400));
+        const float4 *lib_s = reinterpret_cast<const float4 *>(smem + (size_t)s * kStageBytes);
+        const float4 *cell_s = reinterpret_cast<const float4 *>(smem + (size_t)s * kStageBytes + kLibBlockBytes) + warp * MM_KP;
+        const float *w_s = reinterpret_cast<const float *>(smem + (size_t)s * kStageBytes + kLibBlockBytes + MM_TCB * MM_KP * 16) + warp * MM_KP;
+#pragma unroll kPixelUnroll
+        for (int j = 0; j < MM_KP / 32; ++j) {
+            const int p = j * 32 + lane;
+            const float4 c = cell_s[p];
+            const float w = w_s[p];
+            if (DIFF == MM_DIFF_CIEDE2000) {
+                // packed FP32: two library images per lane vector. The tile stores image pairs interleaved:
+                // [pair][0][p] = (L0, L1, a0, a1), [pair][1][p] = (b0, b1, C0, C1)  (prep_kernels.cu)
+#pragma unroll
+                for (int i = 0; i < MM_TNB / 2; ++i) {
+                    const float4 la = lib_s[(i * 2 + 0) * MM_KP + p];
+                    const float4 lb = lib_s[(i * 2 + 1) * MM_KP + p];
+                    const mm_f2 d = mm_ciede2000_stored_v<mm_f2>(c.x, c.y, c.z, c.w, mm_f2{la.x, la.y}, mm_f2{la.z, la.w},
+                                                               mm_f2{lb.x, lb.y}, mm_f2{lb.z, lb.w});
+                    const mm_f2 a2 = v_fma(mm_f2{w, w}, d, mm_f2{acc[2 * i], acc[2 * i + 1]});
+                    acc[2 * i] = a2.x;
+                    acc[2 * i + 1] = a2.y;
+                }
+            } else {
+#pragma unroll
+                for (int i = 0; i < MM_TNB; ++i) {
+                    const float4 l = lib_s[i * MM_KP + p];
+                    acc[i] = fmaf(w, mm_euclid(c.x, c.y, c.z, l.x, l.y, l.z), acc[i]);
+                }
+            }
+        }
+        __syncwarp();
+        if (lane == 0)
+            mbar_arrive(&empty_bar[s]);
+    }
+}
 
 template <int DIFF>
 __global__ void __launch_bounds__(kThreads, MM_MIN_CTAS)
@@ -143,48 +195,7 @@ diff_sum_kernel(const unsigned char *__restrict__ cells, const unsigned char *__
 
     // ---------------- consumer warps: warp = cell within the tile, lanes stride pixels
     float acc[MM_TNB];
-#pragma unroll
-    for (int i = 0; i < MM_TNB; ++i)
-        acc[i] = 0.0f;
-
-    for (int k = 0; k < nk; ++k) {
-        const int s = k % kStages;
-        mbar_wait(&full_bar[s], (k / kStages) & 1);
-        if (MM_STRESS_SKEW)
-            __nanosleep((unsigned)((warp * 97 + k * 29 + blockIdx.x * 7) % 400));
-        const float4 *lib_s = reinterpret_cast<const float4 *>(smem + (size_t)s * kStageBytes);
-        const float4 *cell_s = reinterpret_cast<const float4 *>(smem + (size_t)s * kStageBytes + kLibBlockBytes) + warp * MM_KP;
-        const float *w_s = reinterpret_cast<const float *>(smem + (size_t)s * kStageBytes + kLibBlockBytes + MM_TCB * MM_KP * 16) + warp * MM_KP;
-#pragma unroll kPixelUnroll
-        for (int j = 0; j < MM_KP / 32; ++j) {
-            const int p = j * 32 + lane;
-            const float4 c = cell_s[p];
-            const float w = w_s[p];
-            if (DIFF == MM_DIFF_CIEDE2000) {
-                // packed FP32: two library images per lane vector. The tile stores image pairs interleaved:
-                // [pair][0][p] = (L0, L1, a0, a1), [pair][1][p] = (b0, b1, C0, C1)  (prep_kernels.cu)
-#pragma unroll
-                for (int i = 0; i < MM_TNB / 2; ++i) {
-                    const float4 la = lib_s[(i * 2 + 0) * MM_KP + p];
-                    const float4 lb = lib_s[(i * 2 + 1) * MM_KP + p];
-                    const mm_f2 d = mm_ciede2000_stored_v<mm_f2>(c.x, c.y, c.z, c.w, mm_f2{la.x, la.y}, mm_f2{la.z, la.w},
-                                                               mm_f2{lb.x, lb.y}, mm_f2{lb.z, lb.w});
-                    const mm_f2 a2 = v_fma(mm_f2{w, w}, d, mm_f2{acc[2 * i], acc[2 * i + 1]});
-                    acc[2 * i] = a2.x;
-                    acc[2 * i + 1] = a2.y;
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < MM_TNB; ++i) {
-                    const float4 l = lib_s[i * MM_KP + p];
-                    acc[i] = fmaf(w, mm_euclid(c.x, c.y, c.z, l.x, l.y, l.z), acc[i]);
-                }
-            }
-        }
-        __syncwarp();
-        if (lane == 0)
-            mbar_arrive(&empty_bar[s]);
-    }
+    consume_ring<DIFF>(smem, full_bar, empty_bar, nk, warp, lane, acc);
 
     // ---------------- epilogue: warp-shuffle reduction, D store, fused argmin
 #pragma unroll
@@ -217,7 +228,7 @@ diff_sum_kernel(const unsigned char *__restrict__ cells, const unsigned char *__
 template <int DIFF>
 static cudaError_t launch(const void *cells, const void *lib, float *D, unsigned long long *best_key, int n_cell_tiles,
                           int n_lib_tiles, int n_chunks, int n_lib, int n_cells, cudaStream_t stream, const int *cancel,
-                          unsigned long long *progress, Raster raster, size_t seg_stride)
+                          unsigned long long *progress, Raster raster)
 {
     const size_t smem = (size_t)kStages * kStageBytes;
     // per device (context) attribute: set on every launch, it is cheap
@@ -225,97 +236,232 @@ static cudaError_t launch(const void *cells, const void *lib, float *D, unsigned
     if (e != cudaSuccess)
         return e;
     const unsigned grid = (unsigned)n_cell_tiles * (unsigned)n_lib_tiles;  // 1-D, super-block rasterisation (kernels.h)
-    // One launch per pixel segment (split-K across LAUNCHES): the kernel itself only learns how many chunks to walk (nk) and gets
-    // its tensors pre-offset to the segment's first chunk; the tile stride inside the packed tensors stays n_chunks. Keeping the
-    // segment out of the kernel keeps its inner loop's instruction schedule exactly the one measured fastest in round 1 -- ptxas
-    // re-orders the 461-instruction loop body on the slightest change of the surrounding code, worth +-1 % (DESIGN.md 4.1).
-    for (int seg = 0; seg < raster.n_segs; ++seg) {
-        const int k0 = raster.n_segs > 1 ? seg * raster.seg_chunks : 0;
-        const int nk = raster.n_segs > 1 ? std::min(n_chunks, k0 + raster.seg_chunks) - k0 : n_chunks;
-        diff_sum_kernel<DIFF><<<grid, kThreads, smem, stream>>>(
-            (const unsigned char *)cells + (size_t)k0 * kCellBlockBytes, (const unsigned char *)lib + (size_t)k0 * kLibBlockBytes,
-            D ? D + (size_t)seg * seg_stride : nullptr, best_key, n_chunks, n_lib, n_lib_tiles * MM_TNB, n_cells, n_cell_tiles,
-            n_lib_tiles, cancel, progress, nk, raster.sb_a, raster.sb_b);
-        e = cudaGetLastError();
-        if (e != cudaSuccess)
-            return e;
-    }
-    return cudaSuccess;
+    diff_sum_kernel<DIFF><<<grid, kThreads, smem, stream>>>((const unsigned char *)cells, (const unsigned char *)lib, D, best_key, n_chunks,
+                                                            n_lib, n_lib_tiles * MM_TNB, n_cells, n_cell_tiles, n_lib_tiles, cancel,
+                                                            progress, n_chunks, raster.sb_a, raster.sb_b);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_diff_sum(int diff_type, const void *cells, const void *lib, float *D, unsigned long long *best_key,
                             int n_cell_tiles, int n_lib_tiles, int n_chunks, int n_lib, int n_cells, cudaStream_t stream,
-                            const int *cancel, unsigned long long *progress, Raster raster, size_t seg_stride)
+                            const int *cancel, unsigned long long *progress)
 {
     if (n_cell_tiles <= 0 || n_lib_tiles <= 0 || n_chunks <= 0)
         return cudaSuccess;
     if (diff_type != MM_DIFF_CIEDE2000)
         return cudaErrorInvalidValue;  // RGB Euclidean / CIE76 run diff_euclid_kernel (diff_euclid.cu)
-    if (raster.n_segs < 1 || raster.sb_a < 1 || raster.sb_b < 1 || (raster.n_segs > 1 && (best_key || !D || raster.seg_chunks < 1)))
-        return cudaErrorInvalidValue;
-    return launch<MM_DIFF_CIEDE2000>(cells, lib, D, best_key, n_cell_tiles, n_lib_tiles, n_chunks, n_lib, n_cells, stream, cancel, progress,
-                                     raster, seg_stride);
-}
-
-// ---------------------------------------------------------------- raster choice + segment reduction
-
-Raster choose_raster(int n_cell_tiles, int n_lib_tiles, int n_chunks, bool can_split)
-{
     auto env = [](const char *name) -> int {
         const char *v = getenv(name);
         return v ? atoi(v) : 0;
     };
-    // Measured on config 4 (ncu dram__bytes_read, profiles/r2_raster_sweep.txt), segments / sb_a x sb_b -> DRAM reads, kernel time:
-    //   1 / 16 x 16: 47.4 GB, 893.8 ms     2 / 32 x 8: 30.6 GB, 894.4 ms     3 / 32 x 8: 22.5 GB, 895.2 ms     4 / 32 x 8: 22.0 GB, 895.7 ms
-    //   2 / 16 x 16: 42.8 GB               1 / 24 x 12: 102.5 GB             1 / 32 x 8: 233 GB                 2 / 64 x 4: 251 GB
-    // i.e. a hot set (sb_a cell tiles x one segment x 20 KB per chunk) of 42 MB survives in the 126 MB L2, 63 MB and more do not,
-    // and every extra launch costs ~0.6 ms of tail. Default: segments of <= 64 chunks (8,192 pixels), the widest column whose hot
-    // set stays <= 42 MB.
-    Raster r{1, n_chunks, kSuperTiles, kSuperTiles};
-    if (can_split && n_chunks > 64)
-        r.n_segs = (n_chunks + 63) / 64;
-    if (env("MM_SPLITK") > 0 && can_split)
-        r.n_segs = std::min(env("MM_SPLITK"), std::max(n_chunks, 1));
-    r.seg_chunks = (n_chunks + r.n_segs - 1) / r.n_segs;
-    r.n_segs = (n_chunks + r.seg_chunks - 1) / std::max(r.seg_chunks, 1);
-    const size_t seg_bytes = (size_t)std::max(r.seg_chunks, 1) * kCellBlockBytes;
-    int a = (int)((size_t)(42u << 20) / seg_bytes);
-    a = a >= 64 ? 64 : (a >= 32 ? 32 : 16);
+    // Measured on config 4 (ncu dram__bytes_read, profiles/r2_raster_sweep.txt): whole cells per CTA, 16 x 16 super-blocks:
+    // 47.4 GB at the kernel's compute-bound time. MM_SB_A / MM_SB_B in the environment override the shape (tuning).
+    Raster r{std::min(kSuperTiles, n_cell_tiles), std::min(kSuperTiles, n_lib_tiles)};
     if (env("MM_SB_A") > 0)
-        a = env("MM_SB_A");
-    r.sb_a = std::max(1, std::min(a, n_cell_tiles));
-    r.sb_b = std::max(1, 256 / r.sb_a);
+        r.sb_a = std::min(env("MM_SB_A"), n_cell_tiles);
     if (env("MM_SB_B") > 0)
-        r.sb_b = env("MM_SB_B");
-    r.sb_b = std::max(1, std::min(r.sb_b, n_lib_tiles));
-    return r;
+        r.sb_b = std::min(env("MM_SB_B"), n_lib_tiles);
+    return launch<MM_DIFF_CIEDE2000>(cells, lib, D, best_key, n_cell_tiles, n_lib_tiles, n_chunks, n_lib, n_cells, stream, cancel, progress,
+                                     r);
 }
 
-__global__ void sum_segments_kernel(float4 *__restrict__ D, int n_segs, size_t seg_stride4, size_t n4)
+// ---------------------------------------------------------------- row work lists (segment passes, exact pruning)
+
+// One CTA = one group of up to 8 rows (cell x library tile) that share a library tile. Bucket b = column * n_lib_tiles + lib_tile
+// holds the bucket's listed cells (in cell order) at cells[b * col_cells ...]; groups[] is the exclusive scan of its group counts.
+// The producer streams the tile's 16 KB library block and, per warp, that cell's 2 KB pixel slice + 512 B weight slice of its cell
+// block: the shared-memory stage has exactly the layout of diff_sum_kernel's, so the consumer loop is the same code. A group with
+// fewer than 8 rows repeats its first cell in the empty warps and does not store them.
+__global__ void __launch_bounds__(kThreads, MM_MIN_CTAS)
+diff_rows_kernel(const unsigned char *__restrict__ cells, const unsigned char *__restrict__ lib, float *__restrict__ D, int n_chunks,
+                 int nk, int n_lib_pad, int n_lib_tiles, RowList rows, const int *__restrict__ perm, const int *cancel,
+                 unsigned long long *__restrict__ progress)
 {
-    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
-        float4 v = D[i];
-        for (int s = 1; s < n_segs; ++s) {  // fixed order: the result does not depend on how the launch was scheduled
-            const float4 w = D[(size_t)s * seg_stride4 + i];
-            v.x += w.x;
-            v.y += w.y;
-            v.z += w.z;
-            v.w += w.w;
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ uint64_t full_bar[kStages];
+    __shared__ uint64_t empty_bar[kStages];
+    __shared__ int s_cancelled, s_cell[kConsumerWarps], s_lib_tile, s_n_rows;
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        const int cancelled = cancel ? load_cancel_flag(cancel) : 0;  // device word (L2 hit), in flight during the set-up
+        // bucket of this group: last b with groups[b] <= blockIdx.x (groups is non-decreasing, groups[0] = 0)
+        int lo = 0, hi = rows.n_buckets;
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (rows.groups[mid] <= (int)blockIdx.x)
+                lo = mid;
+            else
+                hi = mid;
         }
-        D[i] = v;
+        const int g = (int)blockIdx.x - rows.groups[lo];
+        const int n_in = min(kConsumerWarps, rows.count[lo] - g * kConsumerWarps);
+        const int *list = rows.cells + (size_t)lo * rows.col_cells + g * kConsumerWarps;
+        for (int w = 0; w < kConsumerWarps; ++w)
+            s_cell[w] = list[w < n_in ? w : 0];
+        s_lib_tile = lo % n_lib_tiles;
+        s_n_rows = n_in;
+        for (int s = 0; s < kStages; ++s) {
+            mbar_init(&full_bar[s], 1);
+            mbar_init(&empty_bar[s], kConsumerWarps);
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        s_cancelled = cancelled;
+    }
+    __syncthreads();
+    if (s_cancelled)
+        return;  // cancel(): nothing has been issued yet, the whole CTA leaves
+    const int lib_tile = s_lib_tile;
+
+    if (warp == kConsumerWarps) {
+        if (lane == 0) {
+            const unsigned char *lib_src = lib + (size_t)lib_tile * n_chunks * kLibBlockBytes;
+            constexpr uint32_t kSlice = MM_KP * 16, kWSlice = MM_KP * 4;
+            for (int k = 0; k < nk; ++k) {
+                const int s = k % kStages;
+                if (k >= kStages)
+                    mbar_wait(&empty_bar[s], ((k / kStages) - 1) & 1);
+                unsigned char *dst = smem + (size_t)s * kStageBytes;
+                if (MM_STRESS_SKEW)
+                    __nanosleep((unsigned)((k * 131 + blockIdx.x * 17) % 300));
+                mbar_expect_tx(&full_bar[s], kLibBlockBytes + kConsumerWarps * (kSlice + kWSlice));
+                bulk_g2s(dst, lib_src + (size_t)k * kLibBlockBytes, kLibBlockBytes, &full_bar[s]);
+                for (int w = 0; w < kConsumerWarps; ++w) {
+                    const int c = s_cell[w];
+                    const unsigned char *blk = cells + ((size_t)(c / MM_TCB) * n_chunks + k) * kCellBlockBytes;
+                    const int slot = c % MM_TCB;
+                    bulk_g2s(dst + kLibBlockBytes + w * kSlice, blk + slot * kSlice, kSlice, &full_bar[s]);
+                    bulk_g2s(dst + kLibBlockBytes + MM_TCB * kSlice + w * kWSlice, blk + MM_TCB * kSlice + slot * kWSlice, kWSlice,
+                             &full_bar[s]);
+                }
+            }
+        }
+        return;
+    }
+
+    float acc[MM_TNB];
+    consume_ring<MM_DIFF_CIEDE2000>(smem, full_bar, empty_bar, nk, warp, lane, acc);
+#pragma unroll
+    for (int i = 0; i < MM_TNB; ++i) {
+        float v = acc[i];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+            v += __shfl_xor_sync(0xffffffffu, v, o);
+        acc[i] = v;
+    }
+    if (warp < s_n_rows && lane < MM_TNB) {
+        float v = 0.0f;
+#pragma unroll
+        for (int i = 0; i < MM_TNB; ++i)
+            v = (lane == i) ? acc[i] : v;
+        // segments are added in pass order, one pass at a time: D = ((seg 0 + seg 1) + seg 2) + ... for every pair
+        float *d = D + (size_t)s_cell[warp] * n_lib_pad + perm[lib_tile * MM_TNB + lane];
+        *d += v;
+    }
+    if (progress && threadIdx.x == 0)
+        atomicAdd(progress, (unsigned long long)s_n_rows);
+}
+
+cudaError_t launch_diff_rows(const void *cells, const void *lib, float *D, int n_groups, int n_lib_tiles, int n_chunks, int k0, int nk,
+                             RowList rows, const int *perm, cudaStream_t stream, const int *cancel, unsigned long long *progress)
+{
+    if (n_groups <= 0 || nk <= 0)
+        return cudaSuccess;
+    const size_t smem = (size_t)kStages * kStageBytes;
+    cudaError_t e = cudaFuncSetAttribute(diff_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess)
+        return e;
+    // the kernel gets its tensors pre-offset to the segment's first chunk; the tile stride inside them stays n_chunks
+    diff_rows_kernel<<<(unsigned)n_groups, kThreads, smem, stream>>>(
+        (const unsigned char *)cells + (size_t)k0 * kCellBlockBytes, (const unsigned char *)lib + (size_t)k0 * kLibBlockBytes, D, n_chunks, nk,
+        n_lib_tiles * MM_TNB, n_lib_tiles, rows, perm, cancel, progress);
+    return cudaGetLastError();
+}
+
+// One CTA per bucket (column of col_cells cells x one library tile), one thread per cell. A cell is listed when its row is in
+// state `want`; with a threshold T (pruning) an active row is listed only while one of its pairs still has a partial sum <= T[cell]
+// -- otherwise it dies: its pairs become +inf (their complete sums are > T, top-K can never take them) and its remaining segments
+// count as done. Listing keeps cell order, so the lists do not depend on scheduling.
+__global__ void __launch_bounds__(1024)
+list_rows_kernel(float *__restrict__ D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *__restrict__ state, int want,
+                 const float *__restrict__ T, const int *__restrict__ perm, int segs_left, RowList rows,
+                 int *__restrict__ group_count, unsigned long long *__restrict__ listed, unsigned long long *__restrict__ progress)
+{
+    __shared__ int warp_sum[32];
+    const int lib_tile = blockIdx.x, col = blockIdx.y;
+    const int b = col * n_lib_tiles + lib_tile;
+    const int cell = col * rows.col_cells + threadIdx.x;
+    bool on = false;
+    if (threadIdx.x < rows.col_cells && cell < n_rows) {
+        uint8_t *st = state ? state + (size_t)cell * n_lib_tiles + lib_tile : nullptr;
+        on = !st || *st == want;
+        if (on && T) {
+            const float t = T[cell];
+            float *row = D + (size_t)cell * n_lib_pad;
+            bool alive = false;
+            for (int i = 0; i < MM_TNB; ++i) {
+                const int j = perm[lib_tile * MM_TNB + i];
+                alive = alive || (j < n_lib && row[j] <= t);
+            }
+            if (!alive) {
+                for (int i = 0; i < MM_TNB; ++i)
+                    row[perm[lib_tile * MM_TNB + i]] = __int_as_float(0x7f800000);
+                *st = kRowDead;
+                if (progress)
+                    atomicAdd(progress, (unsigned long long)segs_left);
+                on = false;
+            }
+        }
+    }
+    // block-wide exclusive rank of the listed cells, in thread (= cell) order
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned ballot = __ballot_sync(0xffffffffu, on);
+    if (lane == 0)
+        warp_sum[warp] = __popc(ballot);
+    __syncthreads();
+    int before = 0, total = 0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+        before += w < warp ? warp_sum[w] : 0;
+        total += warp_sum[w];
+    }
+    if (on)
+        rows.cells[(size_t)b * rows.col_cells + before + __popc(ballot & ((1u << lane) - 1u))] = cell;
+    if (threadIdx.x == 0) {
+        rows.count[b] = total;
+        group_count[b] = (total + MM_TCB - 1) / MM_TCB;
+        if (total)
+            atomicAdd(listed, (unsigned long long)total);
     }
 }
 
-cudaError_t launch_sum_segments(float *D, int n_segs, size_t seg_stride, size_t n, cudaStream_t stream)
+size_t list_rows_scratch_bytes(int n_buckets)
 {
-    if (n_segs <= 1 || n == 0)
+    size_t temp = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, temp, (const int *)nullptr, (int *)nullptr, n_buckets + 1);
+    return ((size_t)(n_buckets + 1) * sizeof(int) + 255 & ~(size_t)255) + temp;
+}
+
+cudaError_t launch_list_rows(float *D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *state, int want, const float *T,
+                             const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
+                             unsigned long long *listed, unsigned long long *progress, cudaStream_t stream)
+{
+    const int n_cols = (n_rows + rows.col_cells - 1) / rows.col_cells;
+    if (n_cols <= 0 || n_lib_tiles <= 0)
         return cudaSuccess;
-    if ((seg_stride | n) & 3)
-        return cudaErrorInvalidValue;  // rows are padded to the library tile (8 floats), so both are multiples of 4
-    const size_t n4 = n / 4;
-    const unsigned blocks = (unsigned)((n4 + 255) / 256 > 148 * 16 ? 148 * 16 : (n4 + 255) / 256);
-    sum_segments_kernel<<<blocks, 256, 0, stream>>>(reinterpret_cast<float4 *>(D), n_segs, seg_stride / 4, n4);
-    return cudaGetLastError();
+    if (rows.col_cells > 1024 || rows.col_cells % 32 || rows.n_buckets != n_cols * n_lib_tiles)
+        return cudaErrorInvalidValue;
+    // group counts in scratch[0 .. n_buckets], the last one stays 0 so that the scan's last entry is the total
+    int *group_count = (int *)scratch;
+    const size_t head = (size_t)(rows.n_buckets + 1) * sizeof(int) + 255 & ~(size_t)255;
+    cudaError_t e = cudaMemsetAsync(group_count + rows.n_buckets, 0, sizeof(int), stream);
+    if (e != cudaSuccess)
+        return e;
+    list_rows_kernel<<<dim3((unsigned)n_lib_tiles, (unsigned)n_cols), rows.col_cells, 0, stream>>>(
+        D, n_lib_pad, n_lib, n_rows, n_lib_tiles, state, want, T, perm, segs_left, rows, group_count, listed, progress);
+    if ((e = cudaGetLastError()) != cudaSuccess)
+        return e;
+    size_t temp = scratch_bytes - head;
+    return cub::DeviceScan::ExclusiveSum((unsigned char *)scratch + head, temp, group_count, rows.groups, rows.n_buckets + 1, stream);
 }
 
 }  // namespace mm

@@ -95,12 +95,20 @@ struct DevBuf {
     }
 };
 
+// segment passes of the CIEDE2000 difference sums (kernels.h: RowList): 8 passes over the pixel axis, work lists of columns of
+// 256 cells (config 4: 16 chunks per segment, a column's hot set 10 MB of L2)
+constexpr int kPruneSegments = 8;
+constexpr int kColumnCells = 256;
+
 // persistent device workspace of one generator (see DevBuf)
 struct Workspace {
     DevBuf main_f32, main_var_u8, lib_small, lib_work, lib_half;
     DevBuf pix_list, masks4, descs, cells_packed, lib_packed, best_key;
     DevBuf grid, pos, next, prog, counts;
     DevBuf tab_start, tab_si, tab_alpha;  // fractional INTER_AREA table of the current step
+    // segment passes over row work lists (kernels.h: RowList) and exact pruning
+    DevBuf perm, inv_perm, order_scratch, row_cells, row_count, row_groups, list_scratch, row_state, listed, prune_score, prune_idx,
+        threshold;
 };
 
 struct StepPlan {
@@ -157,7 +165,7 @@ struct mosaic_generator {
     // progress(int) while a launch runs: device counter of finished CTAs, polled over a second stream into pinned memory
     cudaStream_t poll_stream = nullptr;
     DevBuf d_progress;
-    unsigned long long *h_progress = nullptr;
+    unsigned long long *h_progress = nullptr;  // [0] progress poll, [1] [2] row-list counts
 
     bool is_cancelled() const { return h_cancel && __atomic_load_n(h_cancel, __ATOMIC_RELAXED) != 0; }
 
@@ -598,6 +606,19 @@ void run_pipeline(G *g, bool candidates_only)
     g->cand_k.assign(n_steps, 0);
 
     const bool penalise = g->repeat_range > 0 && g->repeat_addition != 0;
+    const bool fused_argmin = !penalise && V == 1 && !candidates_only && g->world == 1 && !g->report_margins;
+    // CIEDE2000 steps that need D run as segment passes over row work lists; the library tiles then hold the library in colour
+    // order (kernels.h: RowList), which is what lets exact pruning drop whole tiles of a cell
+    const bool row_passes = layout == kLayoutCiede && !fused_argmin;
+    if (row_passes) {
+        g->ws.perm.alloc((size_t)n_lib_pad * sizeof(int), st);
+        g->ws.inv_perm.alloc((size_t)n_lib_pad * sizeof(int), st);
+        g->ws.order_scratch.alloc(library_order_scratch_bytes(N), st);
+        const uint8_t *src = g->d_lib_u8.as<uint8_t>();
+        CU(launch_library_order(src, g->lib_stored_size, N, n_lib_pad, g->ws.perm.as<int>(), g->ws.inv_perm.as<int>(), g->ws.order_scratch.p,
+                                g->ws.order_scratch.bytes, st));
+        tm.kernel_launches += 3;
+    }
     int progress = 0;
     // cancel(): polled by the host before every phase it enqueues and by every CTA of the difference kernels when it starts
     // (the reference polls per step, row and cell, CPUPhotomosaicGenerator.cpp:52, 66, 73). Work already enqueued drains first.
@@ -663,15 +684,16 @@ void run_pipeline(G *g, bool candidates_only)
 
         // library tiles
         d.lib_packed.alloc((size_t)n_lib_tiles * p.n_chunks * tg.lib_block, st);
+        const int *perm = row_passes ? d.perm.as<int>() : nullptr;
         if (fuse_lib_conversion && layout == kLayoutCiede)
             CU(launch_pack_library_ciede(lib_u8_at_ds, true, d.lib_packed.p, N, P, d.pix_list.as<int>(), p.n_active, p.n_chunks,
-                                         n_lib_tiles, g->d_lut.as<short4>(), st, ds * fused_k, fused_k));
+                                         n_lib_tiles, g->d_lut.as<short4>(), st, ds * fused_k, fused_k, perm));
         else if (fuse_lib_conversion)
             CU(launch_pack_library_euclid_u8(lib_u8_at_ds, ds * fused_k, fused_k, is_lab, d.lib_packed.p, N, P, d.pix_list.as<int>(),
                                              p.n_active, p.n_chunks, n_lib_tiles, g->d_lut.as<short4>(), st));
         else
             CU(launch_pack_library(d_lib_work.as<float>(), d.lib_packed.p, N, P, d.pix_list.as<int>(), p.n_active, p.n_chunks,
-                                   n_lib_tiles, layout, st));
+                                   n_lib_tiles, layout, st, perm));
         tm.kernel_launches++;
 
         // cell descriptors of this rank's cells (getCellAt, PhotomosaicGeneratorBase.cpp:293-329)
@@ -719,18 +741,12 @@ void run_pipeline(G *g, bool candidates_only)
         tm.kernel_launches++;
         clock.end();
 
-        // ---- DiffReduce: one fused launch for the whole step
+        // ---- DiffReduce
         clock.begin(kDiff);
-        const bool fused_argmin = !penalise && V == 1 && !candidates_only && g->world == 1 && !g->report_margins;
         const bool need_D = !fused_argmin || g->keep_D;
         DevBuf &D = g->d_D[s];
-        // CIEDE2000 launches that write D split the pixel axis into segments for L2 locality (kernels.h: Raster); the partial
-        // matrices sit seg_stride floats apart and are added in a fixed order right after the launch
-        const Raster raster = layout == kLayoutCiede ? choose_raster(n_cell_tiles, n_lib_tiles, p.n_chunks, need_D && !fused_argmin)
-                                                      : Raster{1, p.n_chunks, kSuperTiles, kSuperTiles};
-        const size_t seg_stride = (size_t)std::max(n_rows_pad, 1) * n_lib_pad;
         if (need_D) {
-            D.alloc(seg_stride * raster.n_segs * sizeof(float), st);
+            D.alloc((size_t)std::max(n_rows_pad, 1) * n_lib_pad * sizeof(float), st);
             g->have_D[s] = true;
         }
         if (fused_argmin) {
@@ -738,38 +754,43 @@ void run_pipeline(G *g, bool candidates_only)
             CU(launch_fill_u64(d.best_key.as<unsigned long long>(), (size_t)std::max(n_rows_pad, 1), ~0ull, st));
             tm.kernel_launches++;
         }
-        check_cancel();
-        if (d_tiles_done)
-            CU(cudaMemsetAsync(d_tiles_done, 0, sizeof(unsigned long long), st));
-        if (layout == kLayoutCiede)
-            CU(launch_diff_sum(MM_DIFF_CIEDE2000, d.cells_packed.p, d.lib_packed.p, need_D ? D.as<float>() : nullptr,
-                               fused_argmin ? d.best_key.as<unsigned long long>() : nullptr, n_cell_tiles, n_lib_tiles, p.n_chunks,
-                               (int)N, n_rows_local, st, g->d_cancel, d_tiles_done, raster, seg_stride));
-        else
-            CU(launch_diff_euclid(d.cells_packed.p, d.lib_packed.p, need_D ? D.as<float>() : nullptr,
-                                  fused_argmin ? d.best_key.as<unsigned long long>() : nullptr, n_cell_tiles, n_lib_tiles, p.n_chunks,
-                                  (int)N, n_rows_local, st, g->d_cancel, d_tiles_done));
-        if (n_cell_tiles > 0)
-            tm.kernel_launches += layout == kLayoutCiede ? raster.n_segs : 1;
-        if (raster.n_segs > 1 && n_cell_tiles > 0) {
-            CU(launch_sum_segments(D.as<float>(), raster.n_segs, seg_stride, seg_stride, st));
-            tm.kernel_launches++;
+        // top-K count of the selection below; when D only feeds top-K (and need not be complete), pairs that cannot be among the
+        // k_need smallest are pruned (launch_prune_threshold)
+        const int64_t rr = g->repeat_range;
+        const int64_t k_need = candidates_only ? (penalise ? std::min<int64_t>(N, 2 * rr * rr + 2 * rr + 1) : 1)
+                                               : std::min<int64_t>(N, 2 * rr * rr + 2 * rr + 1 + (g->report_margins ? 1 : 0));
+        const bool via_topk = candidates_only || (penalise && k_need * 4 <= N);
+        const int M = (int)std::min<int64_t>(N, k_need + k_need / 4 + 8);  // candidates of the first segment: 1.25 k_need + 8
+        const bool prune = row_passes && via_topk && V == 1 && !g->keep_D && k_need * 4 <= N && M <= 4096 && n_rows_local > 0;
+        // segments: 8 (or MM_SPLITK) passes over the pixel axis, chunk-aligned
+        int n_segs = 1, seg_chunks = p.n_chunks;
+        if (row_passes) {
+            const char *ev = getenv("MM_SPLITK");
+            const int want = ev && atoi(ev) > 0 ? atoi(ev) : kPruneSegments;
+            seg_chunks = (p.n_chunks + std::min(want, p.n_chunks) - 1) / std::min(want, p.n_chunks);
+            n_segs = (p.n_chunks + seg_chunks - 1) / seg_chunks;
         }
-        clock.end();
+        const unsigned long long prog_total = row_passes ? (unsigned long long)std::max(n_rows_local, 1) * n_lib_tiles * n_segs
+                                                         : (unsigned long long)std::max(n_cell_tiles, 1) * n_lib_tiles;
         const int step_weight = (int)pow(4.0, (double)(n_steps - 1 - s));
         const int positions = p.rows * p.cols;
-        if (g->progress_fn) {
-            // the host watches the launch from here (before anything that could block it, e.g. the pageable D2H copy of the grid)
+        int last = progress;
+        // waits for the stream; with a callback the host polls the device's count of finished rows / tiles meanwhile and emits
+        // base + weight * floor(positions * done / total) (see the end of the step)
+        auto watch = [&]() {
+            if (!g->progress_fn) {
+                wait_stream(g, st);
+                check_cancel();
+                return;
+            }
             cudaEvent_t done;
             CU(cudaEventCreateWithFlags(&done, cudaEventDisableTiming));
             cudaEventRecord(done, st);
-            const unsigned long long total = (unsigned long long)std::max(n_cell_tiles, 1) * (unsigned long long)n_lib_tiles * raster.n_segs;
-            int last = progress;
             while (cudaEventQuery(done) == cudaErrorNotReady) {
                 if (cudaMemcpyAsync(g->h_progress, d_tiles_done, sizeof(unsigned long long), cudaMemcpyDeviceToHost, g->poll_stream) == cudaSuccess &&
                     cudaStreamSynchronize(g->poll_stream) == cudaSuccess && !g->is_cancelled()) {
-                    const unsigned long long dn = std::min(*g->h_progress, total);
-                    const int v = progress + step_weight * (int)((unsigned long long)positions * dn / total);
+                    const unsigned long long dn = std::min(*g->h_progress, prog_total);
+                    const int v = progress + step_weight * (int)((unsigned long long)positions * dn / prog_total);
                     if (v > last && v < progress + step_weight * positions) {
                         last = v;
                         g->progress_fn(v, g->progress_user);  // may call mosaic_cancel(): the running kernel then drains
@@ -781,7 +802,97 @@ void run_pipeline(G *g, bool candidates_only)
             cudaEventDestroy(done);
             cudaGetLastError();
             check_cancel();
+        };
+        check_cancel();
+        if (d_tiles_done)
+            CU(cudaMemsetAsync(d_tiles_done, 0, sizeof(unsigned long long), st));
+        double evaluated = 1.0;  // executed share of the step's (row, chunk) work
+        if (row_passes && n_rows_local > 0) {
+            CU(cudaMemsetAsync(D.p, 0, D.bytes, st));
+            int col_cells = kColumnCells;
+            if (const char *ev = getenv("MM_SB_A"))
+                col_cells = std::max(32, std::min(1024, atoi(ev) * MM_TCB / 32 * 32));
+            const int n_cols = (n_rows_local + col_cells - 1) / col_cells;
+            RowList rows{nullptr, nullptr, nullptr, n_cols * n_lib_tiles, col_cells};
+            d.row_cells.alloc((size_t)rows.n_buckets * col_cells * sizeof(int), st);
+            d.row_count.alloc((size_t)rows.n_buckets * sizeof(int), st);
+            d.row_groups.alloc((size_t)(rows.n_buckets + 1) * sizeof(int), st);
+            d.list_scratch.alloc(list_rows_scratch_bytes(rows.n_buckets), st);
+            d.listed.alloc(sizeof(unsigned long long), st);
+            rows.cells = d.row_cells.as<int>();
+            rows.count = d.row_count.as<int>();
+            rows.groups = d.row_groups.as<int>();
+            const int *perm = d.perm.as<int>();
+            uint8_t *state = nullptr;
+            if (prune) {
+                d.row_state.alloc((size_t)n_rows_local * n_lib_tiles, st);
+                CU(cudaMemsetAsync(d.row_state.p, kRowActive, d.row_state.bytes, st));
+                state = d.row_state.as<uint8_t>();
+            }
+            double units = 0;  // rows x chunks evaluated
+            int n_groups = 0;
+            auto list = [&](uint8_t *st8, int want, const float *T, int segs_left) {
+                CU(cudaMemsetAsync(d.listed.p, 0, sizeof(unsigned long long), st));
+                CU(launch_list_rows(D.as<float>(), n_lib_pad, (int)N, n_rows_local, n_lib_tiles, st8, want, T, perm, segs_left, rows,
+                                    d.list_scratch.p, d.list_scratch.bytes, d.listed.as<unsigned long long>(), d_tiles_done, st));
+                CU(cudaMemcpyAsync(g->h_progress + 1, rows.groups + rows.n_buckets, sizeof(int), cudaMemcpyDeviceToHost, st));
+                CU(cudaMemcpyAsync(g->h_progress + 2, d.listed.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+                tm.kernel_launches += 2;
+                watch();  // the pass size is needed on the host to size the next launch
+                n_groups = (int)*reinterpret_cast<const int *>(g->h_progress + 1);
+                return (double)g->h_progress[2];
+            };
+            auto pass = [&](int seg, double n_listed) {
+                const int k0 = seg * seg_chunks, nk = std::min(p.n_chunks, k0 + seg_chunks) - k0;
+                CU(launch_diff_rows(d.cells_packed.p, d.lib_packed.p, D.as<float>(), n_groups, n_lib_tiles, p.n_chunks, k0, nk, rows, perm,
+                                    st, g->d_cancel, d_tiles_done));
+                tm.kernel_launches += n_groups > 0;
+                units += n_listed * nk;
+            };
+            double n_listed = list(nullptr, kRowActive, nullptr, 0);  // every row
+            if (!prune) {
+                for (int seg = 0; seg < n_segs; ++seg)
+                    pass(seg, n_listed);
+            } else {
+                pass(0, n_listed);
+                // candidates = the M smallest partial sums of segment 0; their tiles are completed first, T[cell] = the k_need-th
+                // smallest of their complete sums, and every later pass lists only the rows that still have a pair <= T
+                d.prune_score.alloc((size_t)n_rows_local * M * sizeof(float), st);
+                d.prune_idx.alloc((size_t)n_rows_local * M * sizeof(int), st);
+                d.threshold.alloc((size_t)n_rows_local * sizeof(float), st);
+                CU(launch_topk(D.as<float>(), n_lib_pad, (int)N, n_rows_local, M, d.prune_score.as<float>(), d.prune_idx.as<int>(), st));
+                CU(launch_prune_threshold(D.as<float>(), n_lib_pad, d.prune_idx.as<int>(), n_rows_local, M, (int)k_need,
+                                          d.inv_perm.as<int>(), n_lib_tiles, state, nullptr, true, st));
+                tm.kernel_launches += 2;
+                if (n_segs > 1) {
+                    n_listed = list(state, kRowComplete, nullptr, 0);
+                    for (int seg = 1; seg < n_segs; ++seg)
+                        pass(seg, n_listed);
+                }
+                CU(launch_prune_threshold(D.as<float>(), n_lib_pad, d.prune_idx.as<int>(), n_rows_local, M, (int)k_need,
+                                          d.inv_perm.as<int>(), n_lib_tiles, state, d.threshold.as<float>(), false, st));
+                tm.kernel_launches++;
+                for (int seg = 1; seg < n_segs; ++seg) {
+                    n_listed = list(state, kRowActive, d.threshold.as<float>(), n_segs - seg);
+                    pass(seg, n_listed);
+                }
+            }
+            evaluated = units / ((double)n_rows_local * n_lib_tiles * p.n_chunks);
+        } else if (layout == kLayoutCiede) {
+            CU(launch_diff_sum(MM_DIFF_CIEDE2000, d.cells_packed.p, d.lib_packed.p, need_D ? D.as<float>() : nullptr,
+                               fused_argmin ? d.best_key.as<unsigned long long>() : nullptr, n_cell_tiles, n_lib_tiles, p.n_chunks,
+                               (int)N, n_rows_local, st, g->d_cancel, d_tiles_done));
+            tm.kernel_launches += n_cell_tiles > 0;
+        } else {
+            CU(launch_diff_euclid(d.cells_packed.p, d.lib_packed.p, need_D ? D.as<float>() : nullptr,
+                                  fused_argmin ? d.best_key.as<unsigned long long>() : nullptr, n_cell_tiles, n_lib_tiles, p.n_chunks,
+                                  (int)N, n_rows_local, st, g->d_cancel, d_tiles_done));
+            tm.kernel_launches += n_cell_tiles > 0;
         }
+        tm.evaluated_pixel_diffs += p.pixel_diffs * evaluated;
+        clock.end();
+        if (g->progress_fn)
+            watch();  // the host watches the launch from here (before anything that could block it, e.g. the pageable D2H copy)
 
         // ---- Repeats + FindLowest
         clock.begin(kSel);
@@ -791,9 +902,7 @@ void run_pipeline(G *g, bool candidates_only)
         }
         if (candidates_only) {
             // K = min(N, 2r^2 + 2r + 1) smallest entries always contain the penalised winner (SURVEY.md 8e)
-            const int64_t r = g->repeat_range;
-            const int64_t kk = penalise ? std::min<int64_t>(N, 2 * r * r + 2 * r + 1) : 1;
-            const int K = (int)kk;
+            const int K = (int)k_need;
             g->cand_k[s] = K;
             // one block per rank: float scores [per_rank][K] followed by int32 indices [per_rank][K]; every rank's block has the
             // same size, so ONE all-gather assembles the candidates of the whole step (rank r's rows start at r * per_rank)
@@ -832,9 +941,7 @@ void run_pipeline(G *g, bool candidates_only)
                 }
                 // With a penalty the winner (and the runner-up) lies among the K (+1) smallest unpenalised scores
                 // (SURVEY.md 8e), so the wavefront scans candidate lists instead of whole D rows when that is shorter.
-                const int64_t r = g->repeat_range;
-                const int64_t k_need = std::min<int64_t>(N, 2 * r * r + 2 * r + 1 + (g->report_margins ? 1 : 0));
-                if (penalise && k_need * 4 <= N) {
+                if (via_topk) {
                     const int K = (int)k_need;
                     g->d_cand_score[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(float), st);
                     g->d_cand_idx[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(int), st);
@@ -905,7 +1012,7 @@ int mosaic_create(int device, mosaic_generator **out)
     if (cudaStreamCreateWithFlags(&g->poll_stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaHostAlloc((void **)&g->h_cancel, sizeof(int), cudaHostAllocDefault) != cudaSuccess ||
         cudaMalloc((void **)&g->d_cancel, 256) != cudaSuccess || cudaMemset(g->d_cancel, 0, 256) != cudaSuccess ||
-        cudaHostAlloc((void **)&g->h_progress, sizeof(unsigned long long), cudaHostAllocDefault) != cudaSuccess) {
+        cudaHostAlloc((void **)&g->h_progress, 4 * sizeof(unsigned long long), cudaHostAllocDefault) != cudaSuccess) {
         mosaic_destroy(g);
         return MOSAIC_ERR_CUDA;
     }

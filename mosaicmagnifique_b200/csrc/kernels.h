@@ -48,12 +48,9 @@ namespace mm {
 //     chunks (sb_a x seg_chunks x 20 KB) stay hot in the 126 MB L2 for the whole sweep: the library is streamed from HBM once per
 //     cell column, the cells once.
 // Config 4 history (ncu dram__bytes_read): plain order 842 GB; round 1 (16 x 16 super-blocks, library band kept, whole cells per
-// CTA) 124-132 GB = 40 x the 3.3 GB the launch needs; cell column kept instead 47.4 GB; plus two pixel segments of 64 chunks
-// (one launch each, partial sums added in a fixed order by sum_segments_kernel) and 32 x 8 super-blocks 30.6 GB, four segments
-// 22.0 GB (profiles/r2_raster_sweep.txt).
+// CTA) 124-132 GB = 40 x the 3.3 GB the launch needs; cell column kept instead 47.4 GB (profiles/r2_raster_sweep.txt). Launches
+// that write D run as row work lists instead (RowList).
 struct Raster {
-    int n_segs;      // pixel segments = launches (split-K); 1 = whole cells per CTA
-    int seg_chunks;  // chunks per segment
     int sb_a, sb_b;  // super-block: cell tiles x library tiles
 };
 constexpr int kSuperTiles = 16;
@@ -103,19 +100,36 @@ inline TileGeom tile_geom(PackLayout l)
 cudaError_t launch_diff_euclid(const void *cells, const void *lib, float *D, unsigned long long *best_key, int n_cell_tiles,
                                int n_lib_tiles, int n_chunks, int n_lib, int n_cells, cudaStream_t stream,
                                const int *cancel = nullptr, unsigned long long *progress = nullptr);
-// Raster of a CIEDE2000 launch (see above): segments only when the partial sums have somewhere to go (D is written) and the cells
-// are long enough to be worth splitting. MM_SPLITK / MM_SB_A / MM_SB_B in the environment override the choice (tuning).
-Raster choose_raster(int n_cell_tiles, int n_lib_tiles, int n_chunks, bool can_split);
-// D[0][i] += D[1][i] + ... + D[n_segs-1][i] (fixed order); seg_stride in floats
-cudaError_t launch_sum_segments(float *D, int n_segs, size_t seg_stride, size_t n, cudaStream_t stream);
 
 // ---- diff_kernels.cu
-// raster.n_segs > 1: one launch per pixel segment, D holds n_segs partial matrices seg_stride floats apart (add them with
-// launch_sum_segments); best_key must then be null (the fused argmin needs complete sums)
+// Fused argmin launch (best_key, no D) or a complete D: whole cells per CTA, super-block raster (above).
 cudaError_t launch_diff_sum(int diff_type, const void *cells, const void *lib, float *D, unsigned long long *best_key,
                             int n_cell_tiles, int n_lib_tiles, int n_chunks, int n_lib, int n_cells, cudaStream_t stream,
-                            const int *cancel = nullptr, unsigned long long *progress = nullptr,
-                            Raster raster = Raster{1, 0, kSuperTiles, kSuperTiles}, size_t seg_stride = 0);
+                            const int *cancel = nullptr, unsigned long long *progress = nullptr);
+
+// CIEDE2000 launches that write D run the pixel axis as segment passes over row work lists. A row = one cell x one library tile
+// of 8 images (tile slot i holds image perm[i], the library's colour order). Each pass adds the segment's sum of every listed pair
+// into D[cell][perm[slot]] -- D stays in library index order and holds, for every pair, ((seg 0 + seg 1) + seg 2) + ... whichever
+// launches computed it. Buckets = columns of col_cells consecutive cells x library tiles, column-major, so a column's cells
+// stay hot in L2 while the library sweeps past them.
+struct RowList {
+    int *cells;        // [n_buckets][col_cells] listed cells of each bucket, cell order
+    int *count;        // [n_buckets] listed cells
+    int *groups;       // [n_buckets + 1] exclusive scan of the groups of <= 8 rows per bucket (one CTA each)
+    int n_buckets, col_cells;
+};
+// row states (uint8 [n_rows][n_lib_tiles]): still summing / candidate tile, completed before the threshold / pruned
+enum : uint8_t { kRowActive = 0, kRowComplete = 1, kRowDead = 2 };
+// one segment pass: chunks [k0, k0 + nk) of the n_groups groups of `rows`; progress += rows stored
+cudaError_t launch_diff_rows(const void *cells, const void *lib, float *D, int n_groups, int n_lib_tiles, int n_chunks, int k0, int nk,
+                             RowList rows, const int *perm, cudaStream_t stream, const int *cancel = nullptr,
+                             unsigned long long *progress = nullptr);
+// lists the rows in state `want` (state null: every row) into rows.cells / rows.count / rows.groups (rows.groups[n_buckets] = groups
+// in all); with T: active rows whose pairs all have partial sums > T die (pairs -> +inf, progress += segs_left); listed += rows listed
+size_t list_rows_scratch_bytes(int n_buckets);
+cudaError_t launch_list_rows(float *D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *state, int want, const float *T,
+                             const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
+                             unsigned long long *listed, unsigned long long *progress, cudaStream_t stream);
 
 // ---- prep_kernels.cu
 // u8 BGR -> working space f32 AoS [pixel][3]: Lab through the OpenCV-compatible LUT (is_lab) or a plain cast.
@@ -156,15 +170,20 @@ struct CubicTab {
 cudaError_t launch_cubic_u8(const uint8_t *src, int sh, int sw, int cn, uint8_t *dst, int dh, int dw, CubicTab xt, CubicTab yt,
                             cudaStream_t stream);
 // working f32 AoS library [n][P][3] -> packed float4 tiles (compacted pixel order, chroma in .w)
+// perm (CIEDE2000 layout only, optional): tile slot i holds image perm[i] (launch_library_order)
 cudaError_t launch_pack_library(const float *lib, void *packed, int64_t n, int P, const int *pix_list, int n_active,
-                                int n_chunks, int n_lib_tiles, PackLayout layout, cudaStream_t stream);
+                                int n_chunks, int n_lib_tiles, PackLayout layout, cudaStream_t stream, const int *perm = nullptr);
+// colour order of an 8U library of n S x S images: perm[n_pad] (slot -> image; padding slots -> themselves) and its inverse
+size_t library_order_scratch_bytes(int64_t n);
+cudaError_t launch_library_order(const uint8_t *lib, int S, int64_t n, int n_pad, int *perm, int *inv_perm, void *scratch,
+                                 size_t scratch_bytes, cudaStream_t stream);
 
 // CIEDE2000 layout straight from the 8U BGR library at the detail size (Lab conversion fused, no f32 intermediate) or from
 // the f32 working-space library; padding slots are written by the same pass
 // src_is_u8: src_size x src_size images reduced k-fold on the fly (8U INTER_AREA, integer ratio; src_size 0 = already P pixels)
 cudaError_t launch_pack_library_ciede(const void *src, bool src_is_u8, void *packed, int64_t n, int P, const int *pix_list,
                                       int n_active, int n_chunks, int n_lib_tiles, const short4 *lab_lut, cudaStream_t stream,
-                                      int src_size = 0, int k = 1);
+                                      int src_size = 0, int k = 1, const int *perm = nullptr);
 
 // Euclidean layout straight from the 8U BGR library (src_size x src_size images, reduced k-fold on the fly by the 8U INTER_AREA
 // arithmetic; plain cast, or the Lab conversion for CIE76, fused); padding slots are written by the same pass
@@ -217,6 +236,10 @@ cudaError_t launch_min_variants(float *D, int n_cells, int V, int n_lib_pad, cud
 // K smallest (score, index) per row, unsorted. cand_score/cand_idx: [n_cells][K]
 cudaError_t launch_topk(const float *D, int row_stride, int n_lib, int n_cells, int K, float *cand_score, int *cand_idx,
                         cudaStream_t stream);
+// exact pruning: mark = true sets the rows of the candidates' tiles to kRowComplete; mark = false writes T[cell], the k-th smallest
+// of the candidates' (by then complete) sums
+cudaError_t launch_prune_threshold(const float *D, int row_stride, const int *cand_idx, int n_rows, int M, int k, const int *inv_perm,
+                                   int n_lib_tiles, uint8_t *state, float *T, bool mark, cudaStream_t stream);
 // Repeat-penalised selection in raster order (CPUPhotomosaicGenerator.cpp:81-82, 137-169, 185-225).
 //   grid         : rows x cols int64, in: -1 invalid / >= 0 valid, out: best fit per valid cell
 //   cell_pos     : [n_cells] y * cols + x of each valid cell in raster order (= row order of the scores)

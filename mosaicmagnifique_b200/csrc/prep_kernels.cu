@@ -12,6 +12,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
+#include <cub/device/device_radix_sort.cuh>
+
 #include "colour_math.cuh"
 #include "host_model.h"
 #include "kernels.h"
@@ -481,7 +484,7 @@ cudaError_t launch_pack_library_euclid_u8(const uint8_t *lib, int src_size, int 
 template <bool kFromU8>
 __global__ void pack_library_ciede_kernel(const void *__restrict__ src, int S, int k, unsigned char *__restrict__ packed, int64_t n, int P,
                                           const int *__restrict__ pix_list, int n_active, int n_chunks, int64_t n_pair_slots,
-                                          const short4 *__restrict__ lut)
+                                          const short4 *__restrict__ lut, const int *__restrict__ perm)
 {
     const int slots_per_image = n_chunks * MM_KP;
     const size_t total = (size_t)n_pair_slots * slots_per_image;
@@ -493,9 +496,10 @@ __global__ void pack_library_ciede_kernel(const void *__restrict__ src, int S, i
             const int px = pix_list[q];
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
-                const int64_t im = pr * 2 + j;
-                if (im >= n)
+                const int64_t slot = pr * 2 + j;
+                if (slot >= n)
                     continue;
+                const int64_t im = perm ? perm[slot] : slot;
                 float L, a, b;
                 if (kFromU8) {
                     // S x S source, reduced k-fold on the fly (8U INTER_AREA as area_u8_kernel computes it; k == 1: a plain read)
@@ -523,7 +527,7 @@ __global__ void pack_library_ciede_kernel(const void *__restrict__ src, int S, i
 
 cudaError_t launch_pack_library_ciede(const void *src, bool src_is_u8, void *packed, int64_t n, int P, const int *pix_list,
                                       int n_active, int n_chunks, int n_lib_tiles, const short4 *lab_lut, cudaStream_t stream,
-                                      int src_size, int k)
+                                      int src_size, int k, const int *perm)
 {
     if (src_is_u8 && src_size == 0) {  // source already at the detail size
         src_size = 1;
@@ -539,18 +543,86 @@ cudaError_t launch_pack_library_ciede(const void *src, bool src_is_u8, void *pac
         return cudaSuccess;
     if (src_is_u8)
         pack_library_ciede_kernel<true><<<grid_for(total, 256), 256, 0, stream>>>(src, src_size, k, (unsigned char *)packed, n, P, pix_list,
-                                                                                  n_active, n_chunks, n_pair_slots, lab_lut);
+                                                                                  n_active, n_chunks, n_pair_slots, lab_lut, perm);
     else
         pack_library_ciede_kernel<false><<<grid_for(total, 256), 256, 0, stream>>>(src, 0, 1, (unsigned char *)packed, n, P, pix_list,
-                                                                                   n_active, n_chunks, n_pair_slots, lab_lut);
+                                                                                   n_active, n_chunks, n_pair_slots, lab_lut, perm);
+    return cudaGetLastError();
+}
+
+// Colour order of the library (exact pruning groups similar images into one tile): key = Morton code of each image's mean colour,
+// 10 bits per channel. The means are exact integer sums over the 8-bit pixels, so every rank and every run gets the same order;
+// the 5-bit Morton order is a prefix of the 10-bit one, so the key keeps locality at every scale however narrow the colour range.
+__global__ void __launch_bounds__(256) library_key_kernel(const uint8_t *__restrict__ lib, size_t image_bytes, unsigned *__restrict__ key,
+                                                          int *__restrict__ idx)
+{
+    __shared__ unsigned long long part[3][8];
+    const uint8_t *img = lib + (size_t)blockIdx.x * image_bytes;
+    unsigned long long sum[3] = {0, 0, 0};
+    for (size_t i = threadIdx.x; i < image_bytes; i += blockDim.x)
+        sum[i % 3] += img[i];
+    for (int c = 0; c < 3; ++c) {
+        unsigned long long v = sum[c];
+        for (int o = 16; o > 0; o >>= 1)
+            v += __shfl_xor_sync(0xffffffffu, v, o);
+        if ((threadIdx.x & 31) == 0)
+            part[c][threadIdx.x >> 5] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned code = 0;
+        for (int c = 0; c < 3; ++c) {
+            unsigned long long t = 0;
+            for (int w = 0; w < 8; ++w)
+                t += part[c][w];
+            const unsigned q = (unsigned)min(1023ull, t * 1024 / (image_bytes / 3 * 256));  // mean / 256, 10 bits
+            for (int b = 0; b < 10; ++b)
+                code |= ((q >> b) & 1u) << (3 * b + c);
+        }
+        key[blockIdx.x] = code;
+        idx[blockIdx.x] = blockIdx.x;
+    }
+}
+
+__global__ void finish_order_kernel(int *__restrict__ perm, int *__restrict__ inv, int n, int n_pad)
+{
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pad; i += gridDim.x * blockDim.x) {
+        if (i >= n)
+            perm[i] = i;  // padding slots keep padding columns
+        inv[perm[i]] = i;
+    }
+}
+
+size_t library_order_scratch_bytes(int64_t n)
+{
+    size_t temp = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, temp, (const unsigned *)nullptr, (unsigned *)nullptr, (const int *)nullptr, (int *)nullptr,
+                                    (int)n, 0, 30);
+    return (size_t)n * 12 + 256 + temp;
+}
+
+cudaError_t launch_library_order(const uint8_t *lib, int S, int64_t n, int n_pad, int *perm, int *inv_perm, void *scratch,
+                                 size_t scratch_bytes, cudaStream_t stream)
+{
+    if (n <= 0)
+        return cudaSuccess;
+    unsigned *key_in = (unsigned *)scratch, *key_out = key_in + n;
+    int *idx = (int *)(key_out + n);
+    void *temp = (unsigned char *)scratch + (((size_t)n * 12 + 255) & ~(size_t)255);
+    size_t temp_bytes = scratch_bytes - (((size_t)n * 12 + 255) & ~(size_t)255);
+    library_key_kernel<<<(unsigned)n, 256, 0, stream>>>(lib, (size_t)S * S * 3, key_in, idx);
+    cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_in, key_out, idx, perm, (int)n, 0, 30, stream);  // stable
+    if (e != cudaSuccess)
+        return e;
+    finish_order_kernel<<<(unsigned)std::min<int64_t>((n_pad + 255) / 256, 1024), 256, 0, stream>>>(perm, inv_perm, (int)n, n_pad);
     return cudaGetLastError();
 }
 
 cudaError_t launch_pack_library(const float *lib, void *packed, int64_t n, int P, const int *pix_list, int n_active,
-                                int n_chunks, int n_lib_tiles, PackLayout layout, cudaStream_t stream)
+                                int n_chunks, int n_lib_tiles, PackLayout layout, cudaStream_t stream, const int *perm)
 {
     if (layout == kLayoutCiede)
-        return launch_pack_library_ciede(lib, false, packed, n, P, pix_list, n_active, n_chunks, n_lib_tiles, nullptr, stream);
+        return launch_pack_library_ciede(lib, false, packed, n, P, pix_list, n_active, n_chunks, n_lib_tiles, nullptr, stream, 0, 1, perm);
     cudaError_t e = cudaMemsetAsync(packed, 0, (size_t)n_lib_tiles * n_chunks * tile_geom(layout).lib_block, stream);
     if (e != cudaSuccess)
         return e;

@@ -15,6 +15,8 @@
 #include <float.h>
 #include <stdint.h>
 
+#include <algorithm>
+
 #include "kernels.h"
 
 namespace mm {
@@ -178,6 +180,54 @@ cudaError_t launch_topk(const float *D, int row_stride, int n_lib, int n_cells, 
     if (K > n_lib)
         return cudaErrorInvalidValue;
     topk_kernel<<<n_cells, kTopkThreads, 0, stream>>>(D, row_stride, n_lib, K, cand_score, cand_idx);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ pruning threshold
+
+// After pass 0 the M smallest partial sums of a cell name its candidates; their library tiles are completed before anything is
+// pruned. Marking: state[cell][tile of the candidate] = kRowComplete.
+__global__ void mark_candidates_kernel(const int *__restrict__ cand_idx, int M, int n_rows, const int *__restrict__ inv_perm, int n_lib_tiles,
+                                       uint8_t *__restrict__ state)
+{
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < (size_t)n_rows * M; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t cell = i / M;
+        state[cell * n_lib_tiles + inv_perm[cand_idx[i]] / MM_TNB] = kRowComplete;
+    }
+}
+
+// T[cell] = k-th smallest complete sum among the cell's M candidates: at least k complete sums are <= T, so the k-th smallest
+// sum of the whole row is <= T, and a pair whose (monotone) partial sum is already > T cannot be among the k smallest.
+__global__ void threshold_kernel(const float *__restrict__ D, int row_stride, const int *__restrict__ cand_idx, int M, int k,
+                                 float *__restrict__ T)
+{
+    const float *row = D + (size_t)blockIdx.x * row_stride;
+    const int *idx = cand_idx + (size_t)blockIdx.x * M;
+    for (int j = threadIdx.x; j < M; j += blockDim.x) {
+        const float v = row[idx[j]];
+        int lt = 0, le = 0;
+        for (int i = 0; i < M; ++i) {
+            const float u = row[idx[i]];
+            lt += u < v;
+            le += u <= v;
+        }
+        if (lt < k && k <= le)
+            T[blockIdx.x] = v;  // every thread that writes holds the same value
+    }
+}
+
+cudaError_t launch_prune_threshold(const float *D, int row_stride, const int *cand_idx, int n_rows, int M, int k, const int *inv_perm,
+                                   int n_lib_tiles, uint8_t *state, float *T, bool mark, cudaStream_t stream)
+{
+    if (n_rows <= 0)
+        return cudaSuccess;
+    if (k < 1 || k > M)
+        return cudaErrorInvalidValue;
+    if (mark)
+        mark_candidates_kernel<<<(unsigned)std::min<size_t>(((size_t)n_rows * M + 255) / 256, 4096), 256, 0, stream>>>(
+            cand_idx, M, n_rows, inv_perm, n_lib_tiles, state);
+    else
+        threshold_kernel<<<(unsigned)n_rows, 128, 0, stream>>>(D, row_stride, cand_idx, M, k, T);
     return cudaGetLastError();
 }
 

@@ -27,7 +27,9 @@ LIB = os.path.join(ROOT, "mosaicmagnifique_b200", "libmosaic_b200.so")
 
 # kernel name pattern -> (short name, pixel-differences per lane per loop iteration, how that is derived)
 KERNELS = {
-    r"diff_sum_kernelILi2E": ("diff_sum", 8, "one pixel of the lane's cell x the 8 library images of the tile (4 packed pairs), diff_kernels.cu"),
+    # the CIEDE2000 launches that write D (every penalised / top-K step) run diff_rows_kernel; its consumer loop is the same code as
+    # diff_sum_kernel's (consume_ring), which now only serves the fused-argmin launch
+    r"diff_rows_kernel": ("diff_sum", 8, "one pixel of the lane's cell x the 8 library images of the tile (4 packed pairs), diff_kernels.cu diff_rows_kernel"),
     r"diff_euclid_kernel": ("diff_euclid", None, "4 cells x 4 images per pixel, x the loop's pixel unroll (derived from the MUFU.SQRT count: 1 per pair)"),
 }
 PACKED = ("FFMA2", "FMUL2", "FADD2")
