@@ -129,11 +129,28 @@ void mosaic_set_progress_callback(mosaic_generator *g, mosaic_progress_fn fn, vo
 void mosaic_cancel(mosaic_generator *g);
 void mosaic_reset_cancel(mosaic_generator *g);
 
+/* ---- mirrored library tiles (no reference counterpart: the reference mirrors cell masks, CellShape alternate*Flip*, never the
+ * tile placed in a cell). flips is a mask: 1 = horizontal (columns mirrored, cv::flip code 1), 2 = vertical (rows mirrored, code 0);
+ * 0 (the default) compares the library as it is. The candidates of a cell are then the O = 1, 2, 2 or 4 enabled orientations
+ * {0 none, 1 H, 2 V, 3 HV} (in increasing code) of every image: O * N slots, orientation-major, slot = j * N + i for the j-th
+ * orientation of image i -- exactly a library given as [lib, flip_1(lib), ...]. Everything up to the difference matrix is that run's;
+ * ties go to the lowest slot, so an image that is its own mirror image is placed unflipped. Repeats count per source image: all
+ * orientations of image i share one count and the penalty of slot s is addition * count[s mod N]. mosaic_get_best_fits keeps
+ * returning image indices in [0, N); mosaic_get_best_fit_flips gives the orientation; mosaic_get_differences has O * N columns in
+ * slot order; pixel_diffs count the O * N work; buildPhotomosaic places each tile mirrored by its orientation.
+ * MOSAIC_ERR_INVALID_ARGUMENT outside 0..3. A library from mosaic_set_library_shard cannot be combined with flips
+ * (MOSAIC_ERR_UNSUPPORTED): it is stored at the detail size, where mirroring is no longer exact. */
+int mosaic_set_tile_flips(mosaic_generator *g, int flips);
+/* out[r*cols+c] = orientation of the tile chosen for the cell (flip_h + 2 * flip_v, as mosaic_flip_at), -1 = std::nullopt;
+ * MOSAIC_ERR_NOT_READY before a generate on the current grid state */
+int mosaic_get_best_fit_flips(const mosaic_generator *g, int step, int8_t *out, int rows, int cols);
+
 /* ---- parity / measurement taps (no reference counterpart; used by tests and bench.py) */
 /* keep the full difference matrix of every step on the device so it can be read back */
 int mosaic_set_keep_differences(mosaic_generator *g, int keep);
 int64_t mosaic_get_valid_cell_count(const mosaic_generator *g, int step);
-/* D[cell][lib] = min over variants of the masked difference sum (no repeat penalty), cells in raster order */
+/* D[cell][lib] = min over variants of the masked difference sum (no repeat penalty), cells in raster order; with tile flips the
+ * columns are the O * N slots and n_lib must equal O * N */
 int mosaic_get_differences(const mosaic_generator *g, int step, float *out, int64_t n_cells, int64_t n_lib);
 /* Tie-band reporting (BASELINE.json: cells whose best two candidates differ by less than the FP32 tolerance): when switched
  * on, generate() records for every valid cell the best and the second-best PENALISED score it compared (the fused-argmin

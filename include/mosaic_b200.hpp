@@ -295,6 +295,26 @@ public:
         }
         return out;
     }
+    // ---- mirrored library tiles (no reference counterpart; see mosaic_b200.h "mirrored library tiles"): the best fit may place an
+    // image mirrored horizontally and/or vertically. getBestFits() keeps returning image indices; getBestFitFlips() gives, per step,
+    // the orientation of every cell's tile (flip_h + 2 * flip_v, -1 = no best fit).
+    void setTileFlips(bool horizontal, bool vertical) { ck(mosaic_set_tile_flips(m_g, (horizontal ? 1 : 0) | (vertical ? 2 : 0))); }
+    std::vector<std::vector<std::vector<int8_t>>> getBestFitFlips() const
+    {
+        std::vector<std::vector<std::vector<int8_t>>> out(static_cast<size_t>(mosaic_get_grid_steps(m_g)));
+        for (size_t s = 0; s < out.size(); ++s) {
+            int rows = 0, cols = 0;
+            mosaic_get_grid_size(m_g, static_cast<int>(s), &rows, &cols);
+            std::vector<int8_t> v(static_cast<size_t>(rows) * cols);
+            if (mosaic_get_best_fit_flips(m_g, static_cast<int>(s), v.data(), rows, cols) != MOSAIC_OK)
+                throw std::runtime_error("getBestFitFlips: no best fits on the current grid state");
+            out[s].assign(rows, std::vector<int8_t>(cols));
+            for (int y = 0; y < rows; ++y)
+                for (int x = 0; x < cols; ++x)
+                    out[s][y][x] = v[static_cast<size_t>(y) * cols + x];
+        }
+        return out;
+    }
     // cv::Mat buildPhotomosaic(const cv::Scalar&): fills a rows x cols BGRA buffer (step = bytes per row)
     void buildPhotomosaic(const uint8_t backgroundBGRA[4], uint8_t *outBGRA, int rows, int cols, size_t step)
     {

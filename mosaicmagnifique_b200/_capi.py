@@ -68,6 +68,8 @@ def capi():
         "mosaic_set_variant_quirk": (i, [vp, i]),
         "mosaic_generate": (i, [vp]),
         "mosaic_get_best_fits": (i, [vp, i, vp, i, i]),
+        "mosaic_set_tile_flips": (i, [vp, i]),
+        "mosaic_get_best_fit_flips": (i, [vp, i, vp, i, i]),
         "mosaic_build_photomosaic": (i, [vp, vp, vp, i, i, sz]),
         "mosaic_get_max_progress": (i, [vp]),
         "mosaic_set_progress_callback": (None, [vp, PROGRESS_FN, vp]),

@@ -41,7 +41,10 @@ __global__ void build_gather_kernel(const unsigned long long *__restrict__ owner
         if (key != 0ull) {
             const BuildStep st = steps[n_steps - (int)(key >> 40)];  // the high field stores n_steps - step (>= 1)
             const BuildCell c = st.cells[(key & 0xffffffffffull) - 1];
-            const uint8_t *src = st.lib + ((size_t)c.lib_index * st.S * st.S + (size_t)(y - c.y0) * st.S + (x - c.x0)) * 3;
+            // tile pixel (r, c) of the cell, read at the mirrored coordinates of the tile's orientation
+            const int ty = (c.orient & 2) ? st.S - 1 - (y - c.y0) : y - c.y0;
+            const int tx = (c.orient & 1) ? st.S - 1 - (x - c.x0) : x - c.x0;
+            const uint8_t *src = st.lib + ((size_t)c.lib_index * st.S * st.S + (size_t)ty * st.S + tx) * 3;
             px = make_uchar4(src[0], src[1], src[2], 255);
         }
         out[(size_t)y * out_stride_px + x] = px;

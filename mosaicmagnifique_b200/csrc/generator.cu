@@ -152,6 +152,13 @@ struct mosaic_generator {
     bool keep_D = false;
     bool report_margins = false;
     int rank = 0, world = 1;
+    // mirrored library tiles (mosaic_set_tile_flips): the candidate set is the O * N oriented library, orientation-major
+    int flips = 0;
+    bool lib_sharded = false;      // the library came from mosaic_set_library_shard (stored at the detail size, filled by the caller)
+    DevBuf d_lib_oriented;         // [O][N][size][size][3] 8U, built by launch_orient_library
+    int lib_oriented_flips = 0;    // flips d_lib_oriented holds (0 = stale: rebuilt by the next generate)
+    int fits_flips = -1;           // flips of the generate whose slots the grid holds (-1: no generate since the grid was set)
+    int64_t n_slots = 0;           // candidate slots O * N of the last generate (columns of D)
 
     mosaic_progress_fn progress_fn = nullptr;
     void *progress_user = nullptr;
@@ -264,6 +271,16 @@ Shape shape_params_only(const mosaic_cell_shape &c)
     s.alt_row_flip_h = c.alt_row_flip_h != 0;
     s.alt_row_flip_v = c.alt_row_flip_v != 0;
     return s;
+}
+
+// orientations of a flips mask (mosaic_set_tile_flips): the enabled subset of the codes {0, 1 = H, 2 = V, 3 = HV}, in increasing code
+int orient_count(int flips) { return 1 << __builtin_popcount((unsigned)flips & 3u); }
+int orient_code(int flips, int j)
+{
+    for (int c = 0; c < 4; ++c)
+        if ((c & ~flips) == 0 && j-- == 0)
+            return c;
+    return -1;
 }
 
 // Phase timing without host synchronisation inside the pipeline: every begin/end pair records two CUDA events on the
@@ -500,7 +517,18 @@ void run_pipeline(G *g, bool candidates_only)
     }
     const int V = (int)rotations.size();
     g->V_eff = V;
-    const int64_t N = g->n_lib;
+    // candidate slots: the O orientations of the N library images, orientation-major (slot = j * N + i); every stage up to D runs
+    // on the oriented library as if it were the library itself
+    const int O = orient_count(g->flips);
+    if (O > 1 && g->lib_sharded)
+        throw Fail{MOSAIC_ERR_UNSUPPORTED, "tile flips need the library from mosaic_set_library: a library stored at the detail size "
+                                           "cannot be re-oriented exactly"};
+    const int64_t N = g->n_lib * O;
+    if (N * g->lib_size > INT32_MAX)
+        throw Fail{MOSAIC_ERR_UNSUPPORTED, "library too large with tile flips (orientations * n * size must fit 31 bits)"};
+    g->n_slots = N;
+    if (!candidates_only)
+        g->fits_flips = g->flips;
     const int n_lib_tiles = (int)((N + tg.tnb - 1) / tg.tnb);
     const int n_lib_pad = n_lib_tiles * tg.tnb;
     const size_t n_steps = g->grid.size();
@@ -543,6 +571,19 @@ void run_pipeline(G *g, bool candidates_only)
         tm.kernel_launches++;
     }
 
+    // ---- Preprocess: oriented library (rebuilt only when the library or the flips changed)
+    const uint8_t *lib_src = g->d_lib_u8.as<uint8_t>();
+    if (O > 1) {
+        if (g->lib_oriented_flips != g->flips) {
+            g->lib_oriented_flips = 0;
+            g->d_lib_oriented.alloc((size_t)N * g->lib_size * g->lib_size * 3, st);
+            CU(launch_orient_library(lib_src, g->d_lib_oriented.as<uint8_t>(), g->n_lib, g->lib_size, g->flips, st));
+            tm.kernel_launches++;
+            g->lib_oriented_flips = g->flips;
+        }
+        lib_src = g->d_lib_oriented.as<uint8_t>();
+    }
+
     // ---- Preprocess: library -> working space at the detail size of step 0 (:255-290)
     DevBuf &d_lib_work = g->ws.lib_work, &d_lib_small = g->ws.lib_small;
     int lib_ds = g->lib_size;
@@ -550,7 +591,7 @@ void run_pipeline(G *g, bool candidates_only)
     bool fuse_lib_conversion = false;
     int fused_k = 1;
     {
-        const uint8_t *src = g->d_lib_u8.as<uint8_t>();
+        const uint8_t *src = lib_src;
         if (g->group.detail != 1.0) {
             lib_ds = g->plans[0].ds;
             if (g->lib_stored_size != g->lib_size) {
@@ -614,8 +655,7 @@ void run_pipeline(G *g, bool candidates_only)
         g->ws.perm.alloc((size_t)n_lib_pad * sizeof(int), st);
         g->ws.inv_perm.alloc((size_t)n_lib_pad * sizeof(int), st);
         g->ws.order_scratch.alloc(library_order_scratch_bytes(N), st);
-        const uint8_t *src = g->d_lib_u8.as<uint8_t>();
-        CU(launch_library_order(src, g->lib_stored_size, N, n_lib_pad, g->ws.perm.as<int>(), g->ws.inv_perm.as<int>(), g->ws.order_scratch.p,
+        CU(launch_library_order(lib_src, g->lib_stored_size, N, n_lib_pad, g->ws.perm.as<int>(), g->ws.inv_perm.as<int>(), g->ws.order_scratch.p,
                                 g->ws.order_scratch.bytes, st));
         tm.kernel_launches += 3;
     }
@@ -755,10 +795,16 @@ void run_pipeline(G *g, bool candidates_only)
             tm.kernel_launches++;
         }
         // top-K count of the selection below; when D only feeds top-K (and need not be complete), pairs that cannot be among the
-        // k_need smallest are pruned (launch_prune_threshold)
+        // k_need smallest are pruned (launch_prune_threshold).
+        // Grouped K: the window holds W = 2r^2 + 2r cells, so at most W distinct images and, as the O orientations of an image share
+        // its count, at most O * W of the O * N slots carry a penalty. Among the O * W + 1 smallest (score, slot) pairs at least one
+        // slot u is unpenalised. The penalised winner w has D[w] + A * count >= D[w] and must beat or tie u, so D[w] <= D[u], and at
+        // D[w] == D[u] the lower slot wins: (D[w], w) <= (D[u], u), so w is among the O * W + 1 smallest. The runner-up is among the
+        // O * W + 2 smallest by the same argument with two unpenalised slots. O = 1 is SURVEY.md 8e's bound.
         const int64_t rr = g->repeat_range;
-        const int64_t k_need = candidates_only ? (penalise ? std::min<int64_t>(N, 2 * rr * rr + 2 * rr + 1) : 1)
-                                               : std::min<int64_t>(N, 2 * rr * rr + 2 * rr + 1 + (g->report_margins ? 1 : 0));
+        const int64_t n_win = 2 * rr * rr + 2 * rr;
+        const int64_t k_need = candidates_only ? (penalise ? std::min<int64_t>(N, O * n_win + 1) : 1)
+                                               : std::min<int64_t>(N, O * n_win + 1 + (g->report_margins ? 1 : 0));
         const bool via_topk = candidates_only || (penalise && k_need * 4 <= N);
         const int M = (int)std::min<int64_t>(N, k_need + k_need / 4 + 8);  // candidates of the first segment: 1.25 k_need + 8
         const bool prune = row_passes && via_topk && V == 1 && !g->keep_D && k_need * 4 <= N && M <= 4096 && n_rows_local > 0;
@@ -901,7 +947,7 @@ void run_pipeline(G *g, bool candidates_only)
             tm.kernel_launches++;
         }
         if (candidates_only) {
-            // K = min(N, 2r^2 + 2r + 1) smallest entries always contain the penalised winner (SURVEY.md 8e)
+            // K = min(O * N, O * (2r^2 + 2r) + 1) smallest entries always contain the penalised winner (k_need above)
             const int K = (int)k_need;
             g->cand_k[s] = K;
             // one block per rank: float scores [per_rank][K] followed by int32 indices [per_rank][K]; every rank's block has the
@@ -931,7 +977,7 @@ void run_pipeline(G *g, bool candidates_only)
                 d_prog.alloc((size_t)p.rows * sizeof(int), st);
                 CU(cudaMemcpyAsync(d_prog.p, p.row_first.data(), (size_t)p.rows * sizeof(int), cudaMemcpyHostToDevice, st));
                 const int n_ctas = (int)std::max<int64_t>(1, std::min<int64_t>(n_all, select_max_ctas(g->device)));
-                d_counts.alloc((size_t)n_ctas * N * sizeof(int), st);
+                d_counts.alloc((size_t)n_ctas * g->n_lib * sizeof(int), st);  // per source image
                 CU(cudaMemsetAsync(d_counts.p, 0, d_counts.bytes, st));
                 float *margins = nullptr;
                 if (g->report_margins) {
@@ -949,11 +995,11 @@ void run_pipeline(G *g, bool candidates_only)
                                    g->d_cand_idx[s].as<int>(), st));
                     tm.kernel_launches++;
                     CU(launch_select(d_grid.as<long long>(), d_pos.as<int>(), d_next.as<int>(), (int)n_all, p.rows, p.cols,
-                                     g->d_cand_score[s].as<float>(), g->d_cand_idx[s].as<int>(), K, K, (int)N, g->repeat_range,
+                                     g->d_cand_score[s].as<float>(), g->d_cand_idx[s].as<int>(), K, K, (int)g->n_lib, g->repeat_range,
                                      g->repeat_addition, d_prog.as<int>(), d_counts.as<int>(), n_ctas, margins, st));
                 } else {
                     CU(launch_select(d_grid.as<long long>(), d_pos.as<int>(), d_next.as<int>(), (int)n_all, p.rows, p.cols,
-                                     D.as<float>(), nullptr, (int)N, V * n_lib_pad, (int)N, g->repeat_range, g->repeat_addition,
+                                     D.as<float>(), nullptr, (int)N, V * n_lib_pad, (int)g->n_lib, g->repeat_range, g->repeat_addition,
                                      d_prog.as<int>(), d_counts.as<int>(), n_ctas, margins, st));
                 }
                 if (n_all > 0)
@@ -1037,6 +1083,7 @@ void mosaic_destroy(mosaic_generator *g)
         cudaStreamSynchronize(g->stream);
     g->d_main_u8.release();
     g->d_lib_u8.release();
+    g->d_lib_oriented.release();
     g->d_lut.release();
     g->ws = Workspace();
     g->d_D.clear();
@@ -1150,6 +1197,8 @@ int mosaic_set_library(mosaic_generator *g, const uint8_t *bgr, int64_t n, int s
         g->lib_size = a.size;
         g->lib_stored_size = a.size;
         g->lib_capacity = a.n;
+        g->lib_sharded = false;
+        g->lib_oriented_flips = 0;
     }, &a);
 }
 
@@ -1167,6 +1216,9 @@ int mosaic_set_library_shard(mosaic_generator *g, const uint8_t *bgr_slice, int6
             throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "need 0 <= first, first + count <= n_total <= capacity and a slice pointer"};
         if (a.n * a.size > INT32_MAX)
             throw Fail{MOSAIC_ERR_UNSUPPORTED, "library too large (n * size must fit 31 bits)"};
+        if (g->flips != 0)
+            throw Fail{MOSAIC_ERR_UNSUPPORTED, "tile flips are set: a library stored at the detail size cannot be re-oriented exactly "
+                                               "(use mosaic_set_library, or mosaic_set_tile_flips(g, 0))"};
         if (!g->have_group)
             throw Fail{MOSAIC_ERR_NOT_READY, "the cell group must be set first (its detail level decides the stored size)"};
         if (a.size != g->group.cells[0].size)
@@ -1198,6 +1250,8 @@ int mosaic_set_library_shard(mosaic_generator *g, const uint8_t *bgr_slice, int6
         g->lib_size = a.size;
         g->lib_stored_size = ds;
         g->lib_capacity = a.cap;
+        g->lib_sharded = true;
+        g->lib_oriented_flips = 0;
     }, &a);
 }
 
@@ -1271,6 +1325,7 @@ int mosaic_set_cell_group_ex(mosaic_generator *g, const mosaic_cell_shape *shape
         g->group = grp;
         g->have_group = true;
         g->grid.clear();
+        g->fits_flips = -1;
         return MOSAIC_OK;
     } catch (const std::bad_alloc &) {
         return g->fail(MOSAIC_ERR_OUT_OF_MEMORY, "setCellGroup: host allocation failed");
@@ -1345,6 +1400,7 @@ int mosaic_set_grid_state(mosaic_generator *g, int step, int rows, int cols, con
         for (size_t i = 0; i < gs.v.size(); ++i)
             gs.v[i] = valid[i] ? 0 : -1;  // valid cells start as 0 (GridGenerator.cpp:192)
         g->grid.resize(step + 1);
+        g->fits_flips = -1;
     } catch (...) {
         g->grid.clear();
         return g->fail(MOSAIC_ERR_OUT_OF_MEMORY, "setGridState: host allocation failed");
@@ -1391,6 +1447,7 @@ int mosaic_compute_grid_state(mosaic_generator *g)
             return false;
         }
     };
+    g->fits_flips = -1;
     if (!compute_grid_state(g->group, g->img_rows, g->img_cols, gpu_eval, g->grid, err))
         return g->fail(MOSAIC_ERR_UNSUPPORTED, "getGridState: " + err);
     return MOSAIC_OK;
@@ -1434,7 +1491,36 @@ int mosaic_get_best_fits(const mosaic_generator *g, int step, int64_t *out, int 
     const GridStep &gs = g->grid[step];
     if (rows != gs.rows || cols != gs.cols)
         return MOSAIC_ERR_INVALID_ARGUMENT;
-    memcpy(out, gs.v.data(), gs.v.size() * sizeof(int64_t));
+    if (g->fits_flips > 0) {  // the grid holds slots j * N + i: report the image i
+        for (size_t i = 0; i < gs.v.size(); ++i)
+            out[i] = gs.v[i] >= 0 ? gs.v[i] % g->n_lib : gs.v[i];
+    } else {
+        memcpy(out, gs.v.data(), gs.v.size() * sizeof(int64_t));
+    }
+    return MOSAIC_OK;
+}
+
+int mosaic_set_tile_flips(mosaic_generator *g, int flips)
+{
+    if (!g)
+        return MOSAIC_ERR_INVALID_ARGUMENT;
+    if (flips < 0 || flips > 3)
+        return g->fail(MOSAIC_ERR_INVALID_ARGUMENT, "setTileFlips: flips is a mask of 1 (horizontal) and 2 (vertical)");
+    g->flips = flips;
+    return MOSAIC_OK;
+}
+
+int mosaic_get_best_fit_flips(const mosaic_generator *g, int step, int8_t *out, int rows, int cols)
+{
+    if (!g || !out || step < 0 || step >= (int)g->grid.size())
+        return MOSAIC_ERR_INVALID_ARGUMENT;
+    if (g->fits_flips < 0)
+        return MOSAIC_ERR_NOT_READY;
+    const GridStep &gs = g->grid[step];
+    if (rows != gs.rows || cols != gs.cols)
+        return MOSAIC_ERR_INVALID_ARGUMENT;
+    for (size_t i = 0; i < gs.v.size(); ++i)
+        out[i] = (int8_t)(gs.v[i] >= 0 ? orient_code(g->fits_flips, (int)(gs.v[i] / g->n_lib)) : -1);
     return MOSAIC_OK;
 }
 
@@ -1502,12 +1588,12 @@ int mosaic_get_differences(const mosaic_generator *g, int step, float *out, int6
         return MOSAIC_ERR_NOT_READY;
     const StepPlan &p = g->plans[step];
     const int64_t n_local = p.cell_end - p.cell_begin;
-    if (n_cells != n_local || n_lib != g->n_lib)
+    if (n_cells != n_local || n_lib != g->n_slots)  // n_slots = O * N: D has a column per slot
         return MOSAIC_ERR_INVALID_ARGUMENT;
     if (n_local == 0)
         return MOSAIC_OK;
     const int tnb = tile_geom(g->diff_type == MOSAIC_CIEDE2000 ? kLayoutCiede : kLayoutEuclid).tnb;
-    const int n_lib_pad = (int)((g->n_lib + tnb - 1) / tnb) * tnb;
+    const int n_lib_pad = (int)((g->n_slots + tnb - 1) / tnb) * tnb;
     cudaSetDevice(g->device);
     cudaError_t e = cudaMemcpy2D(out, (size_t)n_lib * sizeof(float), g->d_D[step].p, (size_t)g->V_eff * n_lib_pad * sizeof(float),
                                  (size_t)n_lib * sizeof(float), (size_t)n_local, cudaMemcpyDeviceToHost);
@@ -1573,6 +1659,8 @@ int mosaic_build_photomosaic(mosaic_generator *g, const uint8_t background_bgra[
         cudaStream_t st = g->stream;
         const int H = g->img_rows, W = g->img_cols, n_steps = (int)g->grid.size();
         const int64_t N = g->n_lib;
+        // the grid holds slots j * N + i of the generate's orientations: image i, placed mirrored by orientation j
+        const int fl = std::max(g->fits_flips, 0), O = orient_count(fl);
         DevBuf owner, out, d_steps;
         std::vector<DevBuf> libs(n_steps), cells(n_steps), masks(n_steps);
         std::vector<BuildStep> hsteps(n_steps);
@@ -1588,6 +1676,10 @@ int mosaic_build_photomosaic(mosaic_generator *g, const uint8_t background_bgra[
             int S = S_prev;
             if (s > 0) {
                 S = (int)lround(0.5 * S_prev);
+                // the 2 x 2 halving is exact in integers and commutes with mirroring; the fractional table of an odd size need not
+                if (O > 1 && S_prev % 2 != 0)
+                    throw Fail{MOSAIC_ERR_UNSUPPORTED, "mirrored tiles at an odd cell size (" + std::to_string(S_prev) + ") of step " +
+                                                           std::to_string(s - 1) + ": halving it does not commute with mirroring"};
                 libs[s].alloc((size_t)N * S * S * 3, st);
                 if (S_prev % 2 == 0) {
                     CU(launch_area_u8(lib_prev, libs[s].as<uint8_t>(), N, S_prev, 2, st));
@@ -1614,10 +1706,11 @@ int mosaic_build_photomosaic(mosaic_generator *g, const uint8_t background_bgra[
                     const int64_t v = gs.v[(size_t)y * gs.cols + x];
                     if (v < 0)
                         continue;
-                    if (v >= N)
+                    if (v >= O * N)
                         throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "best fit index outside the library"};
                     const Rect r = rect_at(shape, x - kPadGrid, y - kPadGrid);
-                    hc.push_back(BuildCell{r.x, r.y, flip_at(shape, x - kPadGrid, y - kPadGrid), (int)hc.size() + 1, (int)v});
+                    hc.push_back(BuildCell{r.x, r.y, flip_at(shape, x - kPadGrid, y - kPadGrid), (int)hc.size() + 1, (int)(v % N),
+                                           orient_code(fl, (int)(v / N))});
                 }
             const std::vector<uint8_t> m4 = shape.masks4();
             masks[s].alloc(m4.size(), st);
@@ -1743,8 +1836,9 @@ int select_impl(mosaic_generator *g, int step, const void *scores, const void *i
         d_prog.alloc((size_t)p.rows * sizeof(int), st);
         CU(cudaMemcpyAsync(d_prog.p, p.row_first.data(), (size_t)p.rows * sizeof(int), cudaMemcpyHostToDevice, st));
         const int n_ctas = (int)std::max<int64_t>(1, std::min<int64_t>(n_all, select_max_ctas(g->device)));
-        d_counts.alloc((size_t)n_ctas * g->n_lib * sizeof(int), st);
+        d_counts.alloc((size_t)n_ctas * g->n_lib * sizeof(int), st);  // per source image: candidates are slots of g->flips
         CU(cudaMemsetAsync(d_counts.p, 0, d_counts.bytes, st));
+        g->fits_flips = g->flips;
         const float *sc = (const float *)a.scores;
         const int *ix = (const int *)a.indices;
         int64_t block_stride = 0;

@@ -150,6 +150,9 @@ inline std::vector<int16_t> expand_lab_lut(const int16_t *lut3)
 cudaError_t launch_hue_rotate(const uint8_t *in, uint8_t *out, int rows, int cols, float rot, cudaStream_t stream);
 // INTER_AREA for integer ratios, 8U 3-channel, batch of n square images (src size s -> dst size s / k)
 cudaError_t launch_area_u8(const uint8_t *src, uint8_t *dst, int64_t n, int src_size, int k, cudaStream_t stream);
+// oriented 8U BGR library for mosaic_set_tile_flips: dst [O][n][S][S][3], orientation-major, the enabled subset of the codes
+// {0 none, 1 = H (columns mirrored), 2 = V (rows mirrored), 3 = HV} of `flips` in increasing code (O = 1, 2, 2 or 4)
+cudaError_t launch_orient_library(const uint8_t *src, uint8_t *dst, int64_t n, int S, int flips, cudaStream_t stream);
 // INTER_AREA for integer ratios, f32 3-channel, batch of n square images
 cudaError_t launch_area_f32(const float *src, float *dst, int64_t n, int src_size, int k, cudaStream_t stream);
 // INTER_AREA for any down-scaling ratio (OpenCV's resizeArea_): device CSR table of host_model's make_area_table
@@ -218,6 +221,7 @@ struct BuildCell {
     int flip;        // mask index
     int raster;      // 1-based raster index of the cell inside its step (0 = "no cell" in the owner map)
     int lib_index;   // chosen library image
+    int orient;      // mirroring of the tile (mosaic_set_tile_flips): flip_h + 2 * flip_v
 };
 struct BuildStep {
     const BuildCell *cells;  // indexed by raster - 1
@@ -244,13 +248,16 @@ cudaError_t launch_prune_threshold(const float *D, int row_stride, const int *ca
 //   grid         : rows x cols int64, in: -1 invalid / >= 0 valid, out: best fit per valid cell
 //   cell_pos     : [n_cells] y * cols + x of each valid cell in raster order (= row order of the scores)
 //   next_x       : [n_cells] column of the next valid cell in the same grid row (cols if none)
-//   scores / idx : per cell M entries; idx == nullptr means "entry j is library image j" (rows of D, stride M_stride)
+//   scores / idx : per cell M entries; idx == nullptr means "entry j is slot j" (rows of D, stride M_stride)
+//   n_images     : library images N. Slots are orientation-major (slot = j * N + i for orientation j of image i, mosaic_set_tile_flips)
+//                  and repeats count per source image: the penalty of slot s is addition * count[s % N], and a chosen slot s in the
+//                  window adds to count[s % N]. With one orientation slot = image and this is the reference's rule.
 //   row_progress : [rows] initialised to the column of the first valid cell of each row (cols if none)
-//   counts       : [n_ctas][n_lib] zero-filled scratch
+//   counts       : [n_ctas][n_images] zero-filled scratch
 //   margins      : optional [n_cells][2] best / second-best penalised score of every cell
 //   rows_per_block / block_stride : candidate lists all-gathered from several GPUs (see SelArgs); 0 = one plain array
 cudaError_t launch_select(long long *grid, const int *cell_pos, const int *next_x, int n_cells, int rows, int cols,
-                          const float *scores, const int *idx, int M, int M_stride, int n_lib, int repeat_range,
+                          const float *scores, const int *idx, int M, int M_stride, int n_images, int repeat_range,
                           int repeat_addition, int *row_progress, int *counts, int n_ctas, float *margins,
                           cudaStream_t stream, long long rows_per_block = 0, long long block_stride = 0);
 int select_max_ctas(int device);

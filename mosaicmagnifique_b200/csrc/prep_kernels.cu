@@ -199,6 +199,48 @@ cudaError_t launch_area_u8(const uint8_t *src, uint8_t *dst, int64_t n, int src_
     return cudaGetLastError();
 }
 
+// Oriented library: dst[j][i] = source image i mirrored by the j-th orientation of `codes` (2 bits each, code = flip_h + 2 * flip_v;
+// flip_h mirrors the columns like cv::flip code 1, flip_v the rows like code 0). One thread per output pixel of 3 bytes.
+__global__ void orient_library_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int64_t n, int S, int n_orient,
+                                      unsigned codes)
+{
+    const size_t img_px = (size_t)S * S;
+    const size_t total = (size_t)n_orient * n * img_px;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t im = i / img_px;  // output image = j * n + source image
+        const int p = (int)(i - im * img_px);
+        const int j = (int)(im / n);
+        const size_t si = im - (size_t)j * n;
+        const unsigned code = (codes >> (2 * j)) & 3u;
+        int y = p / S, x = p - (p / S) * S;
+        if (code & 1u)
+            x = S - 1 - x;
+        if (code & 2u)
+            y = S - 1 - y;
+        const uint8_t *s = src + (si * img_px + (size_t)y * S + x) * 3;
+        uint8_t *d = dst + i * 3;
+        d[0] = s[0];
+        d[1] = s[1];
+        d[2] = s[2];
+    }
+}
+
+cudaError_t launch_orient_library(const uint8_t *src, uint8_t *dst, int64_t n, int S, int flips, cudaStream_t stream)
+{
+    if (flips < 0 || flips > 3)
+        return cudaErrorInvalidValue;
+    int n_orient = 0;
+    unsigned codes = 0;
+    for (int c = 0; c < 4; ++c)
+        if ((c & ~flips) == 0)
+            codes |= (unsigned)c << (2 * n_orient++);
+    const size_t total = (size_t)n_orient * n * S * S;
+    if (total == 0)
+        return cudaSuccess;
+    orient_library_kernel<<<grid_for(total, 256), 256, 0, stream>>>(src, dst, n, S, n_orient, codes);
+    return cudaGetLastError();
+}
+
 // One output pixel of the same 8U INTER_AREA (integer ratio k) straight from the source image: what the fused library packers read
 // when the resize to the detail size has not been materialised (k == 1: the pixel itself)
 __device__ __forceinline__ void area_pixel_u8(const uint8_t *__restrict__ img, int S, int k, int py, int px, int out[3])

@@ -242,10 +242,11 @@ struct SelArgs {
     int n_cells, rows, cols;
     const float *scores;   // per cell M entries, row stride M_stride
     const int *idx;        // per cell M entries (stride M) or nullptr: entry j is library image j
-    int M, M_stride, n_lib;
+    int M, M_stride;
+    int n_images;          // library images: entry id v is slot v of an orientation-major candidate set, image v % n_images
     int range, addition;
     int *row_progress;     // [rows], initialised to the column of the first valid cell (cols if none)
-    int *counts;           // [gridDim.x][n_lib] zeroed scratch: occurrences of each library image in the window
+    int *counts;           // [gridDim.x][n_images] zeroed scratch: occurrences of each library image in the window
     float *margins;        // optional [n_cells][2]: best and second-best PENALISED score (tie-band reporting)
     // all-gathered candidate blocks (multi-GPU): cell c lives in block c / rows_per_block at row c % rows_per_block; blocks are
     // block_stride 4-byte elements apart (scores and indices alike). rows_per_block == 0: one plain array.
@@ -268,7 +269,8 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(SelArgs a)
     __shared__ double s_val[kSelThreads / 32];
     __shared__ int s_id[kSelThreads / 32];
     __shared__ double s_second[kSelThreads / 32];
-    int *cnt = a.counts + (size_t)blockIdx.x * a.n_lib;
+    // repeats count per source image: every orientation of image i shares cnt[i] (kernels.h: launch_select)
+    int *cnt = a.counts + (size_t)blockIdx.x * a.n_images;
     const int tid = threadIdx.x;
 
     for (int c = blockIdx.x; c < a.n_cells; c += gridDim.x) {
@@ -306,7 +308,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(SelArgs a)
             }
             const long long v = __ldcg(a.grid + (size_t)ry * a.cols + rx);
             if (v >= 0)
-                atomicAdd(cnt + v, 1);
+                atomicAdd(cnt + v % a.n_images, 1);
         }
         __syncthreads();
 
@@ -323,7 +325,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(SelArgs a)
         for (int j = tid; j < a.M; j += kSelThreads) {
             const int id = ids ? ids[j] : j;
             const float s = sc[j];
-            const int k = penalise ? __ldcg(cnt + id) : 0;
+            const int k = penalise ? __ldcg(cnt + id % a.n_images) : 0;
             const double v = (double)s + (double)a.addition * (double)k;
             if (v < best || (v == best && id < best_id)) {
                 second = best;
@@ -365,7 +367,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(SelArgs a)
             }
             const long long v = __ldcg(a.grid + (size_t)ry * a.cols + rx);
             if (v >= 0)
-                cnt[v] = 0;
+                cnt[v % a.n_images] = 0;
         }
 
         if (tid == 0) {
@@ -394,13 +396,15 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(SelArgs a)
 }
 
 cudaError_t launch_select(long long *grid, const int *cell_pos, const int *next_x, int n_cells, int rows, int cols,
-                          const float *scores, const int *idx, int M, int M_stride, int n_lib, int repeat_range,
+                          const float *scores, const int *idx, int M, int M_stride, int n_images, int repeat_range,
                           int repeat_addition, int *row_progress, int *counts, int n_ctas, float *margins,
                           cudaStream_t stream, long long rows_per_block, long long block_stride)
 {
     if (n_cells == 0)
         return cudaSuccess;
-    SelArgs a{grid, cell_pos, next_x, n_cells, rows, cols, scores, idx, M, M_stride, n_lib, repeat_range, repeat_addition,
+    if (n_images < 1)
+        return cudaErrorInvalidValue;
+    SelArgs a{grid, cell_pos, next_x, n_cells, rows, cols, scores, idx, M, M_stride, n_images, repeat_range, repeat_addition,
               row_progress, counts, margins, rows_per_block, block_stride};
     void *args[] = {&a};
     // cooperative launch: fails instead of deadlocking if the CTAs could not all be resident

@@ -300,6 +300,26 @@ class PhotomosaicGenerator:
             out.append(g)
         return out
 
+    # ---- mirrored library tiles (no reference counterpart, include/mosaic_b200.h "mirrored library tiles")
+    def setTileFlips(self, horizontal: bool = False, vertical: bool = False):
+        """Lets the best fit place a library image mirrored horizontally and/or vertically. getBestFits() keeps returning image
+        indices; getBestFitFlips() the orientation; getDifferences() has a column per (orientation, image) slot, orientation-major."""
+        self._flips = int(bool(horizontal)) | 2 * int(bool(vertical))
+        self._ck(self._L.mosaic_set_tile_flips(self._h, self._flips))
+
+    def getBestFitFlips(self):
+        """Per step an int8 array: orientation of each cell's tile, flip_h + 2 * flip_v (as mosaic_flip_at), -1 = no best fit."""
+        out = []
+        for step in range(self._L.mosaic_get_grid_steps(self._h)):
+            r, c = ctypes.c_int(), ctypes.c_int()
+            self._ck(self._L.mosaic_get_grid_size(self._h, step, ctypes.byref(r), ctypes.byref(c)))
+            g = np.empty((r.value, c.value), np.int8)
+            rc = self._L.mosaic_get_best_fit_flips(self._h, step, g.ctypes.data, r.value, c.value)
+            if rc:
+                raise MosaicError(rc, "getBestFitFlips: no best fits on the current grid state")
+            out.append(g)
+        return out
+
     def buildPhotomosaic(self, backgroundColour=(0, 0, 0, 0)) -> np.ndarray:
         """PhotomosaicGeneratorBase::buildPhotomosaic(const cv::Scalar&): H x W x 4 uint8 BGRA mosaic."""
         rows, cols = self._main_shape
@@ -330,8 +350,9 @@ class PhotomosaicGenerator:
         first, n, k = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int()
         rc = self._L.mosaic_get_candidate_count(self._h, step, ctypes.byref(first), ctypes.byref(n), ctypes.byref(k))
         n_cells = n.value if rc == 0 else self._L.mosaic_get_valid_cell_count(self._h, step)
-        out = np.empty((n_cells, self._n_lib), np.float32)
-        self._ck(self._L.mosaic_get_differences(self._h, step, out.ctypes.data, n_cells, self._n_lib))
+        n_slots = self._n_lib << bin(getattr(self, "_flips", 0)).count("1")  # O * N columns with tile flips
+        out = np.empty((n_cells, n_slots), np.float32)
+        self._ck(self._L.mosaic_get_differences(self._h, step, out.ctypes.data, n_cells, n_slots))
         return out
 
     def setReportMargins(self, report: bool = True):
