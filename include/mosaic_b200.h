@@ -145,6 +145,22 @@ int mosaic_set_tile_flips(mosaic_generator *g, int flips);
  * MOSAIC_ERR_NOT_READY before a generate on the current grid state */
 int mosaic_get_best_fit_flips(const mosaic_generator *g, int step, int8_t *out, int rows, int cols);
 
+/* ---- usage limit (no reference counterpart: the reference limits repetition only through the windowed penalty of setRepeat).
+ * max_uses = M >= 1 lets each library image be chosen at most M times in one generate, over all size steps (M = 1: no duplicates);
+ * 0 (the default) is unlimited and changes nothing. Cells are decided in the engine's order -- size step 0, 1, ..., and inside a
+ * step the reference's raster order over valid cells -- and a cell takes the lowest (D[s] + addition * count[s mod N], s) over the
+ * slots s whose image s mod N has been chosen fewer than M times so far in this generate (ties to the lowest slot, the value in
+ * f64 as without the limit; the window penalty is unchanged). With tile flips all orientations of an image share one use count.
+ * If M * N is less than the number of valid cells of all steps, generate fails with MOSAIC_ERR_INVALID_ARGUMENT before any work
+ * (the text gives both numbers); otherwise every cell has an allowed image, so the limit never leaves a cell without a fit.
+ * mosaic_get_best_fits, mosaic_get_best_fit_flips and mosaic_get_differences keep their meaning; margins are the best and
+ * second-best ALLOWED penalised scores. Sharded handles: mosaic_generate_candidates uses the limit set at that call; the steps
+ * must then be selected in increasing order (steps without cells may be skipped) -- use counts restart when a step at or below
+ * the last selected one is selected, and selecting a step before an earlier step with cells gives MOSAIC_ERR_NOT_READY.
+ * Candidates handed to mosaic_select_from_candidates / _gathered must be the engine's own (their rows start with a sorted prefix).
+ * MOSAIC_ERR_INVALID_ARGUMENT for M < 0. */
+int mosaic_set_usage_limit(mosaic_generator *g, int max_uses);
+
 /* ---- parity / measurement taps (no reference counterpart; used by tests and bench.py) */
 /* keep the full difference matrix of every step on the device so it can be read back */
 int mosaic_set_keep_differences(mosaic_generator *g, int keep);

@@ -315,6 +315,10 @@ public:
         }
         return out;
     }
+    // ---- usage limit (no reference counterpart; see mosaic_b200.h "usage limit"): each library image is chosen at most maxUses times
+    // per generate, over all size steps (1 = no duplicates, 0 = unlimited); generateBestFits() returns false (lastError() says why)
+    // when maxUses * library size is less than the number of cells.
+    void setUsageLimit(int maxUses) { ck(mosaic_set_usage_limit(m_g, maxUses)); }
     // cv::Mat buildPhotomosaic(const cv::Scalar&): fills a rows x cols BGRA buffer (step = bytes per row)
     void buildPhotomosaic(const uint8_t backgroundBGRA[4], uint8_t *outBGRA, int rows, int cols, size_t step)
     {

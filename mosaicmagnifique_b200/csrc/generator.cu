@@ -109,6 +109,7 @@ struct Workspace {
     // segment passes over row work lists (kernels.h: RowList) and exact pruning
     DevBuf perm, inv_perm, order_scratch, row_cells, row_count, row_groups, list_scratch, row_state, listed, prune_score, prune_idx,
         threshold;
+    DevBuf prefix_score, prefix_idx;  // usage limit: sorted prefixes of D rows, or launch_topk's pick for a candidate list's prefix
 };
 
 struct StepPlan {
@@ -159,6 +160,11 @@ struct mosaic_generator {
     int lib_oriented_flips = 0;    // flips d_lib_oriented holds (0 = stale: rebuilt by the next generate)
     int fits_flips = -1;           // flips of the generate whose slots the grid holds (-1: no generate since the grid was set)
     int64_t n_slots = 0;           // candidate slots O * N of the last generate (columns of D)
+    // usage limit (mosaic_set_usage_limit): each image is chosen at most max_uses times per generate (0 = unlimited)
+    int max_uses = 0;
+    int cand_max_uses = 0;         // max_uses of the last mosaic_generate_candidates: its K and sorted prefixes were built for it
+    int cap_last_step = -1;        // sharded selection: last step selected since `used` was reset (-1: none)
+    DevBuf d_used;                 // [N] choices per source image so far in this generate
 
     mosaic_progress_fn progress_fn = nullptr;
     void *progress_user = nullptr;
@@ -470,6 +476,49 @@ void needed_rows(const G *g, int &row_lo, int &row_hi)
         row_lo = row_hi = 0;
 }
 
+// usage limit: valid cells of all steps, and E_s = the most images that can be exhausted before the last cell of step s
+int64_t total_valid_cells(const G *g)
+{
+    int64_t n = 0;
+    for (const StepPlan &p : g->plans)
+        n += (int64_t)p.cell_pos.size();
+    return n;
+}
+
+int64_t exhausted_bound(const G *g, size_t step)
+{
+    int64_t before = 0;
+    for (size_t t = 0; t < step; ++t)
+        before += (int64_t)g->plans[t].cell_pos.size();
+    return std::max<int64_t>(0, before + (int64_t)g->plans[step].cell_pos.size() - 1) / g->max_uses;
+}
+
+// a cap below the number of cells would leave cells without any allowed image: refused before any work
+void check_usage_limit(const G *g)
+{
+    const int64_t cells = total_valid_cells(g);
+    if (g->max_uses > 0 && (int64_t)g->max_uses * g->n_lib < cells)
+        throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "usage limit " + std::to_string(g->max_uses) + " x " + std::to_string(g->n_lib) +
+                                                    " images = " + std::to_string((int64_t)g->max_uses * g->n_lib) +
+                                                    " placements is less than the " + std::to_string(cells) +
+                                                    " valid cells of all size steps"};
+}
+
+// sorted prefixes of candidate lists [n_rows][K] (launch_topk output), in place: the first min(K, kPrefixMax) entries of every row
+// become its smallest (score, slot) pairs in ascending order
+void sort_list_prefixes(G *g, float *cs, int *ci, int n_rows, int K, mosaic_timings &tm)
+{
+    if (n_rows == 0)
+        return;
+    const int k0 = std::min(K, kPrefixMax);
+    cudaStream_t st = g->stream;
+    g->ws.prefix_score.alloc((size_t)n_rows * k0 * sizeof(float), st);
+    g->ws.prefix_idx.alloc((size_t)n_rows * k0 * sizeof(int), st);
+    CU(launch_topk(cs, K, K, n_rows, k0, g->ws.prefix_score.as<float>(), g->ws.prefix_idx.as<int>(), st));
+    CU(launch_sort_prefix(g->ws.prefix_score.as<float>(), g->ws.prefix_idx.as<int>(), n_rows, k0, cs, ci, K, st));
+    tm.kernel_launches += 2;
+}
+
 // ------------------------------------------------------------------ the pipeline
 
 AreaTab upload_area_table(G *g, int ssize, int dsize, mosaic_timings &tm)
@@ -493,6 +542,7 @@ void run_pipeline(G *g, bool candidates_only)
     if (g->is_cancelled())  // sticky like m_wasCanceled (never reset by the reference): nothing runs until mosaic_reset_cancel
         throw Fail{MOSAIC_ERR_CANCELLED, "cancelled"};
     make_plans(g);
+    check_usage_limit(g);
     cudaStream_t st = g->stream;
     const auto t_host0 = std::chrono::steady_clock::now();
     g->timings = mosaic_timings{};
@@ -647,7 +697,15 @@ void run_pipeline(G *g, bool candidates_only)
     g->cand_k.assign(n_steps, 0);
 
     const bool penalise = g->repeat_range > 0 && g->repeat_addition != 0;
-    const bool fused_argmin = !penalise && V == 1 && !candidates_only && g->world == 1 && !g->report_margins;
+    const bool capped = g->max_uses > 0;
+    const bool fused_argmin = !penalise && !capped && V == 1 && !candidates_only && g->world == 1 && !g->report_margins;
+    if (candidates_only) {
+        g->cand_max_uses = g->max_uses;
+        g->cap_last_step = -1;
+    } else if (capped) {  // `used` starts at 0 for every generate and carries across its steps
+        g->d_used.alloc((size_t)g->n_lib * sizeof(int), st);
+        CU(cudaMemsetAsync(g->d_used.p, 0, g->d_used.bytes, st));
+    }
     // CIEDE2000 steps that need D run as segment passes over row work lists; the library tiles then hold the library in colour
     // order (kernels.h: RowList), which is what lets exact pruning drop whole tiles of a cell
     const bool row_passes = layout == kLayoutCiede && !fused_argmin;
@@ -801,11 +859,14 @@ void run_pipeline(G *g, bool candidates_only)
         // slot u is unpenalised. The penalised winner w has D[w] + A * count >= D[w] and must beat or tie u, so D[w] <= D[u], and at
         // D[w] == D[u] the lower slot wins: (D[w], w) <= (D[u], u), so w is among the O * W + 1 smallest. The runner-up is among the
         // O * W + 2 smallest by the same argument with two unpenalised slots. O = 1 is SURVEY.md 8e's bound.
+        // With a usage limit at most E_s images are exhausted before the step's last cell, so O * E_s more slots may be excluded and
+        // the same argument holds with O * (W + E_s) (DESIGN.md 4.4).
         const int64_t rr = g->repeat_range;
         const int64_t n_win = 2 * rr * rr + 2 * rr;
-        const int64_t k_need = candidates_only ? (penalise ? std::min<int64_t>(N, O * n_win + 1) : 1)
-                                               : std::min<int64_t>(N, O * n_win + 1 + (g->report_margins ? 1 : 0));
-        const bool via_topk = candidates_only || (penalise && k_need * 4 <= N);
+        const int64_t n_excl = capped ? O * exhausted_bound(g, s) : 0;
+        const int64_t k_need = candidates_only ? ((penalise || capped) ? std::min<int64_t>(N, O * n_win + n_excl + 1) : 1)
+                                               : std::min<int64_t>(N, O * n_win + n_excl + 1 + (g->report_margins ? 1 : 0));
+        const bool via_topk = candidates_only || ((penalise || capped) && k_need * 4 <= N);
         const int M = (int)std::min<int64_t>(N, k_need + k_need / 4 + 8);  // candidates of the first segment: 1.25 k_need + 8
         const bool prune = row_passes && via_topk && V == 1 && !g->keep_D && k_need * 4 <= N && M <= 4096 && n_rows_local > 0;
         // segments: 8 (or MM_SPLITK) passes over the pixel axis, chunk-aligned
@@ -959,6 +1020,8 @@ void run_pipeline(G *g, bool candidates_only)
             CU(launch_topk(D.as<float>(), V * n_lib_pad, (int)N, (int)n_local, K, cs, ci, st));
             if (n_local > 0)
                 tm.kernel_launches++;
+            if (capped)  // the capped selection on the gathered blocks reads every row's sorted prefix first
+                sort_list_prefixes(g, cs, ci, (int)n_local, K, tm);
         } else {
             DevBuf &d_grid = d.grid, &d_pos = d.pos, &d_next = d.next, &d_prog = d.prog, &d_counts = d.counts;
             d_grid.alloc(gs.v.size() * sizeof(long long), st);
@@ -987,7 +1050,37 @@ void run_pipeline(G *g, bool candidates_only)
                 }
                 // With a penalty the winner (and the runner-up) lies among the K (+1) smallest unpenalised scores
                 // (SURVEY.md 8e), so the wavefront scans candidate lists instead of whole D rows when that is shorter.
-                if (via_topk) {
+                if (capped) {
+                    // sequential capped selection: every cell's sorted prefix first, its full row (K list or D row) as the fallback
+                    const int k0 = (int)std::min<int64_t>(k_need, kPrefixMax);
+                    const float *row_s = D.as<float>(), *ps;
+                    const int *row_i = nullptr, *pi;
+                    int row_n = (int)N, row_stride = V * n_lib_pad, p_stride = k0;
+                    if (via_topk) {
+                        const int K = (int)k_need;
+                        g->d_cand_score[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(float), st);
+                        g->d_cand_idx[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(int), st);
+                        CU(launch_topk(D.as<float>(), V * n_lib_pad, (int)N, (int)n_all, K, g->d_cand_score[s].as<float>(),
+                                       g->d_cand_idx[s].as<int>(), st));
+                        tm.kernel_launches++;
+                        sort_list_prefixes(g, g->d_cand_score[s].as<float>(), g->d_cand_idx[s].as<int>(), (int)n_all, K, tm);
+                        row_s = ps = g->d_cand_score[s].as<float>();
+                        row_i = pi = g->d_cand_idx[s].as<int>();
+                        row_n = row_stride = p_stride = K;
+                    } else {
+                        d.prefix_score.alloc((size_t)std::max<int64_t>(n_all, 1) * k0 * sizeof(float), st);
+                        d.prefix_idx.alloc((size_t)std::max<int64_t>(n_all, 1) * k0 * sizeof(int), st);
+                        CU(launch_topk(D.as<float>(), V * n_lib_pad, (int)N, (int)n_all, k0, d.prefix_score.as<float>(),
+                                       d.prefix_idx.as<int>(), st));
+                        CU(launch_sort_prefix(d.prefix_score.as<float>(), d.prefix_idx.as<int>(), (int)n_all, k0, nullptr, nullptr, 0, st));
+                        tm.kernel_launches += n_all > 0 ? 2 : 0;
+                        ps = d.prefix_score.as<float>();
+                        pi = d.prefix_idx.as<int>();
+                    }
+                    CU(launch_select_capped(d_grid.as<long long>(), d_pos.as<int>(), (int)n_all, p.rows, p.cols, row_s, row_i, row_n,
+                                            row_stride, ps, pi, k0, p_stride, (int)g->n_lib, g->repeat_range, g->repeat_addition,
+                                            g->max_uses, d_counts.as<int>(), g->d_used.as<int>(), margins, st));
+                } else if (via_topk) {
                     const int K = (int)k_need;
                     g->d_cand_score[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(float), st);
                     g->d_cand_idx[s].alloc((size_t)std::max<int64_t>(n_all, 1) * K * sizeof(int), st);
@@ -1084,6 +1177,7 @@ void mosaic_destroy(mosaic_generator *g)
     g->d_main_u8.release();
     g->d_lib_u8.release();
     g->d_lib_oriented.release();
+    g->d_used.release();
     g->d_lut.release();
     g->ws = Workspace();
     g->d_D.clear();
@@ -1510,6 +1604,16 @@ int mosaic_set_tile_flips(mosaic_generator *g, int flips)
     return MOSAIC_OK;
 }
 
+int mosaic_set_usage_limit(mosaic_generator *g, int max_uses)
+{
+    if (!g)
+        return MOSAIC_ERR_INVALID_ARGUMENT;
+    if (max_uses < 0)
+        return g->fail(MOSAIC_ERR_INVALID_ARGUMENT, "setUsageLimit: max_uses must be >= 0 (0 = unlimited)");
+    g->max_uses = max_uses;
+    return MOSAIC_OK;
+}
+
 int mosaic_get_best_fit_flips(const mosaic_generator *g, int step, int8_t *out, int rows, int cols)
 {
     if (!g || !out || step < 0 || step >= (int)g->grid.size())
@@ -1847,11 +1951,32 @@ int select_impl(mosaic_generator *g, int step, const void *scores, const void *i
             block_stride = 2 * a.rpb * a.k;                                 // in 4-byte elements
         }
         Timer t(st);
-        t.start();
-        CU(launch_select(d_grid.as<long long>(), d_pos.as<int>(), d_next.as<int>(), (int)n_all, p.rows, p.cols, sc, ix, a.k, a.k,
-                         (int)g->n_lib, g->repeat_range, g->repeat_addition, d_prog.as<int>(), d_counts.as<int>(), n_ctas, nullptr,
-                         st, a.rpb, block_stride));
-        t.stop();
+        if (g->cand_max_uses > 0) {
+            // `used` carries across the steps of one generate: selecting a step at or below the last one starts a new generate, and
+            // every earlier step with cells must have been selected since
+            if (a.step <= g->cap_last_step)
+                g->cap_last_step = -1;
+            for (int s = g->cap_last_step + 1; s < a.step; ++s)
+                if (!g->plans[s].cell_pos.empty())
+                    throw Fail{MOSAIC_ERR_NOT_READY, "usage limit: step " + std::to_string(s) + " must be selected before step " +
+                                                         std::to_string(a.step) + " (image uses carry across the steps in order)"};
+            if (g->cap_last_step < 0) {
+                g->d_used.alloc((size_t)g->n_lib * sizeof(int), st);
+                CU(cudaMemsetAsync(g->d_used.p, 0, g->d_used.bytes, st));
+            }
+            t.start();
+            CU(launch_select_capped(d_grid.as<long long>(), d_pos.as<int>(), (int)n_all, p.rows, p.cols, sc, ix, a.k, a.k, sc, ix,
+                                    std::min(a.k, kPrefixMax), a.k, (int)g->n_lib, g->repeat_range, g->repeat_addition, g->cand_max_uses,
+                                    d_counts.as<int>(), g->d_used.as<int>(), nullptr, st, a.rpb, block_stride));
+            t.stop();
+            g->cap_last_step = a.step;
+        } else {
+            t.start();
+            CU(launch_select(d_grid.as<long long>(), d_pos.as<int>(), d_next.as<int>(), (int)n_all, p.rows, p.cols, sc, ix, a.k, a.k,
+                             (int)g->n_lib, g->repeat_range, g->repeat_addition, d_prog.as<int>(), d_counts.as<int>(), n_ctas, nullptr,
+                             st, a.rpb, block_stride));
+            t.stop();
+        }
         CU(cudaMemcpyAsync(gs.v.data(), d_grid.p, gs.v.size() * sizeof(long long), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         g->timings.select_ms += t.ms();

@@ -261,6 +261,22 @@ cudaError_t launch_select(long long *grid, const int *cell_pos, const int *next_
                           int repeat_addition, int *row_progress, int *counts, int n_ctas, float *margins,
                           cudaStream_t stream, long long rows_per_block = 0, long long block_stride = 0);
 int select_max_ctas(int device);
+// Usage limit (mosaic_set_usage_limit, DESIGN.md 4.4). Sorted prefixes: every cell's k0 = min(K, kPrefixMax) smallest (score, slot)
+// pairs in ascending order, the part of its candidates the capped selection scans first.
+constexpr int kPrefixMax = 1024;
+// sel_s / sel_pos [n_rows][k0]: launch_topk's k0 smallest of each row's source. list_s == nullptr: the source is a D row and
+// sel_s / sel_pos become its sorted prefix (score, slot). Otherwise the source is the candidate list list_s / list_i [n_rows][K]
+// (launch_topk output, slots ascending) and its first k0 entries become the sorted prefix; the row keeps its K entries.
+cudaError_t launch_sort_prefix(float *sel_s, int *sel_pos, int n_rows, int k0, float *list_s, int *list_i, int K, cudaStream_t stream);
+// Capped selection in raster order, one CTA: a cell takes the lowest (D[s] + A * count[s % N], s) over the slots s whose image
+// s % N has used[s % N] < max_uses, then used[s % N] += 1. scores / idx: the full candidate row of each cell as launch_select's
+// (M entries, stride M_stride; idx nullptr = D rows); pscores / pidx: its sorted prefix of k0 entries, stride p_stride. All-gathered
+// blocks address prefix and row alike (rows_per_block, block_stride as launch_select). counts: [n_images] zeroed scratch;
+// used: [n_images], carried across the steps of one generate. margins: best / second-best ALLOWED penalised score.
+cudaError_t launch_select_capped(long long *grid, const int *cell_pos, int n_cells, int rows, int cols, const float *scores, const int *idx,
+                                 int M, int M_stride, const float *pscores, const int *pidx, int k0, int p_stride, int n_images,
+                                 int repeat_range, int repeat_addition, int max_uses, int *counts, int *used, float *margins,
+                                 cudaStream_t stream, long long rows_per_block = 0, long long block_stride = 0);
 // best_key (from the diff epilogue) -> grid
 cudaError_t launch_keys_to_grid(const unsigned long long *best_key, const int *cell_pos, long long *grid, int n_cells,
                                 float *best_score, cudaStream_t stream);

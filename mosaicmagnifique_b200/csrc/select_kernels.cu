@@ -419,4 +419,302 @@ int select_max_ctas(int device)
     return sms * (per_sm > 0 ? 1 : 0);
 }
 
+// ------------------------------------------------------------------ usage limit: sorted candidate prefixes
+
+constexpr int kSortThreads = 512;
+
+// One CTA per row. sel_s / sel_pos hold the k0 smallest entries of the row's source by (score bits, position), positions ascending
+// (launch_topk). Without a list the source is a D row (position = slot) and sel_s / sel_pos are sorted in place by (score, slot).
+// With a list (a top-K candidate row of K entries, slots ascending, so position order is slot order) the k0 entries move to the
+// front of the list, sorted; the list entries they displace take the positions the k0 entries left, so the row keeps its K entries.
+__global__ void __launch_bounds__(kSortThreads)
+sort_prefix_kernel(float *__restrict__ sel_s, int *__restrict__ sel_pos, int k0, float *__restrict__ list_s, int *__restrict__ list_i, int K)
+{
+    __shared__ unsigned long long key[kPrefixMax];
+    __shared__ unsigned char in_front[kPrefixMax];  // list position < k0 holds one of the k0 entries
+    __shared__ int word_base[kPrefixMax / 32];
+    const int tid = threadIdx.x, lane = tid & 31;
+    float *ss = sel_s + (size_t)blockIdx.x * k0;
+    int *sp = sel_pos + (size_t)blockIdx.x * k0;
+    float *ls = list_s ? list_s + (size_t)blockIdx.x * K : nullptr;
+    int *li = list_s ? list_i + (size_t)blockIdx.x * K : nullptr;
+    int n2 = 1;
+    while (n2 < k0)
+        n2 <<= 1;
+    for (int j = tid; j < kPrefixMax; j += kSortThreads) {
+        unsigned long long k = ~0ull;
+        if (j < k0) {
+            const int p = sp[j];
+            k = (unsigned long long)__float_as_uint(ss[j]) << 32 | (unsigned)(ls ? li[p] : p);
+        }
+        key[j] = k;
+        in_front[j] = 0;
+    }
+    __syncthreads();
+    // bitonic sort of the n2 keys (scores are sums of non-negative terms, +inf when pruned: their bits order like the values)
+    for (int k = 2; k <= n2; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < n2; i += kSortThreads) {
+                const int o = i ^ j;
+                if (o > i) {
+                    const unsigned long long a = key[i], b = key[o];
+                    if ((a > b) == ((i & k) == 0)) {
+                        key[i] = b;
+                        key[o] = a;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    if (!ls) {
+        for (int j = tid; j < k0; j += kSortThreads) {
+            ss[j] = __uint_as_float((unsigned)(key[j] >> 32));
+            sp[j] = (int)(key[j] & 0xffffffffu);
+        }
+        return;
+    }
+    // t of the k0 entries already sit in front; the other k0 - t (sel_pos[t..k0), ascending) sit behind it. They swap places with
+    // the k0 - t front entries that are not among them, paired in position order.
+    for (int j = tid; j < k0; j += kSortThreads)
+        if (sp[j] < k0)
+            in_front[sp[j]] = 1;
+    __syncthreads();
+    unsigned m[kPrefixMax / kSortThreads];
+    for (int r = 0; r < kPrefixMax / kSortThreads; ++r) {
+        const int a = tid + r * kSortThreads;
+        m[r] = __ballot_sync(0xffffffffu, a < k0 && !in_front[a]);
+        if (lane == 0)
+            word_base[a >> 5] = __popc(m[r]);
+    }
+    __shared__ int s_leaving;
+    __syncthreads();
+    if (tid == 0) {
+        int acc = 0;
+        for (int w = 0; w < kPrefixMax / 32; ++w) {
+            const int c = word_base[w];
+            word_base[w] = acc;
+            acc += c;
+        }
+        s_leaving = acc;
+    }
+    __syncthreads();
+    const int t = k0 - s_leaving;
+    float out_s[kPrefixMax / kSortThreads];
+    int out_i[kPrefixMax / kSortThreads], out_to[kPrefixMax / kSortThreads];
+    for (int r = 0; r < kPrefixMax / kSortThreads; ++r) {
+        const int a = tid + r * kSortThreads;
+        out_to[r] = -1;
+        if (m[r] >> lane & 1u) {  // the rank-th front entry that leaves goes to sel_pos[t + rank]
+            out_to[r] = sp[t + word_base[a >> 5] + __popc(m[r] & ((1u << lane) - 1u))];
+            out_s[r] = ls[a];
+            out_i[r] = li[a];
+        }
+    }
+    __syncthreads();  // every displaced entry is read before the front is overwritten
+    for (int r = 0; r < kPrefixMax / kSortThreads; ++r)
+        if (out_to[r] >= 0) {
+            ls[out_to[r]] = out_s[r];
+            li[out_to[r]] = out_i[r];
+        }
+    for (int j = tid; j < k0; j += kSortThreads) {
+        ls[j] = __uint_as_float((unsigned)(key[j] >> 32));
+        li[j] = (int)(key[j] & 0xffffffffu);
+    }
+}
+
+cudaError_t launch_sort_prefix(float *sel_s, int *sel_pos, int n_rows, int k0, float *list_s, int *list_i, int K, cudaStream_t stream)
+{
+    if (n_rows == 0)
+        return cudaSuccess;
+    if (k0 < 1 || k0 > kPrefixMax || (list_s && (!list_i || K < k0)))
+        return cudaErrorInvalidValue;
+    sort_prefix_kernel<<<n_rows, kSortThreads, 0, stream>>>(sel_s, sel_pos, k0, list_s, list_i, K);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ usage limit: sequential capped selection
+
+constexpr int kCapThreads = 256;
+
+struct CapArgs {
+    long long *grid;
+    const int *cell_pos;
+    int n_cells, rows, cols;
+    const float *scores;   // full candidate row of every cell (M entries, stride M_stride): the fallback
+    const int *idx;        // nullptr: entry j is slot j (a D row)
+    int M, M_stride;
+    const float *pscores;  // sorted prefix of every cell: the k0 smallest (score, slot), stride p_stride
+    const int *pidx;
+    int k0, p_stride;
+    int n_images, range, addition, max_uses;
+    int *counts;           // [n_images] zeroed scratch: window occurrences
+    int *used;             // [n_images] choices so far in this generate
+    float *margins;
+    long long rows_per_block, block_stride;  // all-gathered candidate blocks, as SelArgs (prefix and row share them)
+};
+
+// (best, id, second) of the union of two disjoint candidate sets: lexicographic (value, slot) minimum, second-best value
+__device__ __forceinline__ void merge_best(double &best, int &id, double &second, double ob, int oid, double os)
+{
+    if (ob < best || (ob == best && oid < id)) {
+        second = fmin(best, os);
+        best = ob;
+        id = oid;
+    } else {
+        second = fmin(second, ob);
+    }
+}
+
+__device__ __forceinline__ void warp_best(double &best, int &id, double &second)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(0xffffffffu, best, o);
+        const int oid = __shfl_xor_sync(0xffffffffu, id, o);
+        const double os = __shfl_xor_sync(0xffffffffu, second, o);
+        merge_best(best, id, second, ob, oid, os);
+    }
+}
+
+// One CTA walks the step's valid cells in raster order (every choice depends on all earlier ones through `used`). Per cell: window
+// counts as select_kernel; warp 0 scans the sorted prefix 32 entries at a time and stops once the next entry's unpenalised score is
+// strictly above the best (with margins: second-best) allowed penalised score -- every later entry scores at least that much, and
+// an equal one can only win on a lower slot if it is unpenalised, so it is still examined. A prefix that ends first means the
+// answer may lie behind it: the whole block then scans the cell's full row.
+__global__ void __launch_bounds__(kCapThreads) select_capped_kernel(CapArgs a)
+{
+    __shared__ double s_val[kCapThreads / 32], s_second[kCapThreads / 32];
+    __shared__ int s_id[kCapThreads / 32];
+    __shared__ int s_fallback;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const bool penalise = a.range > 0 && a.addition != 0;
+    const bool margins = a.margins != nullptr;
+
+    for (int c = 0; c < a.n_cells; ++c) {
+        const int pos = a.cell_pos[c];
+        const int y = pos / a.cols, x = pos - y * a.cols;
+        const int y0 = min(max(y - a.range, 0), a.rows);
+        const int x0 = min(max(x - a.range, 0), a.cols);
+        const int x1 = min(max(x + a.range, 0), a.cols - 1);
+        const int ww = x1 - x0 + 1;
+        const int n_above = (y - y0) * ww;
+        const int n_win = penalise ? n_above + (x - x0) : 0;
+        for (int j = tid; j < n_win; j += kCapThreads) {
+            const int ry = j < n_above ? y0 + j / ww : y, rx = j < n_above ? x0 + j % ww : x0 + (j - n_above);
+            const long long v = a.grid[(size_t)ry * a.cols + rx];
+            if (v >= 0)
+                atomicAdd(a.counts + v % a.n_images, 1);
+        }
+        __syncthreads();
+
+        size_t row = (size_t)c, base = 0;
+        if (a.rows_per_block > 0) {
+            base = (size_t)(c / a.rows_per_block) * (size_t)a.block_stride;
+            row = (size_t)(c % a.rows_per_block);
+        }
+        if (warp == 0) {
+            const float *ps = a.pscores + base + row * a.p_stride;
+            const int *pi = a.pidx + base + row * a.p_stride;
+            double best = DBL_MAX, second = DBL_MAX;
+            int best_id = 0x7fffffff;
+            bool stopped = false;
+            float s = lane < a.k0 ? ps[lane] : 0.0f;
+            int id = lane < a.k0 ? pi[lane] : 0;
+            for (int j0 = 0; j0 < a.k0; j0 += 32) {
+                const float first = __shfl_sync(0xffffffffu, s, 0);
+                if ((double)first > (margins ? second : best)) {
+                    stopped = true;
+                    break;
+                }
+                const bool have = j0 + lane < a.k0;
+                const float cs = s;
+                const int cid = id;
+                if (j0 + 32 + lane < a.k0) {  // next chunk's loads overlap this chunk's reduction
+                    s = ps[j0 + 32 + lane];
+                    id = pi[j0 + 32 + lane];
+                }
+                double v = DBL_MAX;
+                int vid = 0x7fffffff;
+                if (have) {
+                    const int img = cid % a.n_images;
+                    if (a.used[img] < a.max_uses) {
+                        v = (double)cs + (double)a.addition * (double)(penalise ? __ldcg(a.counts + img) : 0);
+                        vid = cid;
+                    }
+                }
+                double vs = DBL_MAX;
+                warp_best(v, vid, vs);
+                merge_best(best, best_id, second, v, vid, vs);
+            }
+            if (lane == 0) {
+                s_val[0] = best;
+                s_id[0] = best_id;
+                s_second[0] = second;
+                s_fallback = !stopped && a.k0 < a.M;
+            }
+        }
+        __syncthreads();
+
+        if (s_fallback) {  // uniform: the block scans the full row
+            const float *sc = a.scores + base + row * a.M_stride;
+            const int *ids = a.idx ? a.idx + base + row * a.M : nullptr;
+            double best = DBL_MAX, second = DBL_MAX;
+            int best_id = 0x7fffffff;
+            for (int j = tid; j < a.M; j += kCapThreads) {
+                const int id = ids ? ids[j] : j;
+                const int img = id % a.n_images;
+                if (a.used[img] < a.max_uses)
+                    merge_best(best, best_id, second, (double)sc[j] + (double)a.addition * (double)(penalise ? __ldcg(a.counts + img) : 0), id,
+                               DBL_MAX);
+            }
+            warp_best(best, best_id, second);
+            if (lane == 0) {
+                s_val[warp] = best;
+                s_id[warp] = best_id;
+                s_second[warp] = second;
+            }
+            __syncthreads();
+            if (tid == 0)
+                for (int w = 1; w < kCapThreads / 32; ++w)
+                    merge_best(s_val[0], s_id[0], s_second[0], s_val[w], s_id[w], s_second[w]);
+        }
+
+        // undo the window counts (every thread revisits its own window entries); then the choice
+        for (int j = tid; j < n_win; j += kCapThreads) {
+            const int ry = j < n_above ? y0 + j / ww : y, rx = j < n_above ? x0 + j % ww : x0 + (j - n_above);
+            const long long v = a.grid[(size_t)ry * a.cols + rx];
+            if (v >= 0)
+                a.counts[v % a.n_images] = 0;
+        }
+        if (tid == 0) {
+            const double best = s_val[0];
+            const int best_id = s_id[0];
+            const long long result = (best < DBL_MAX && best_id != 0x7fffffff) ? (long long)best_id : -1ll;
+            a.grid[pos] = result;
+            if (result >= 0)
+                a.used[best_id % a.n_images] += 1;
+            if (margins) {
+                a.margins[2 * c] = (float)best;
+                a.margins[2 * c + 1] = (float)s_second[0];
+            }
+        }
+        __syncthreads();  // counts reset, grid and used updated before the next cell reads them
+    }
+}
+
+cudaError_t launch_select_capped(long long *grid, const int *cell_pos, int n_cells, int rows, int cols, const float *scores, const int *idx,
+                                 int M, int M_stride, const float *pscores, const int *pidx, int k0, int p_stride, int n_images,
+                                 int repeat_range, int repeat_addition, int max_uses, int *counts, int *used, float *margins,
+                                 cudaStream_t stream, long long rows_per_block, long long block_stride)
+{
+    if (n_cells == 0)
+        return cudaSuccess;
+    if (n_images < 1 || max_uses < 1 || k0 < 1 || k0 > M)
+        return cudaErrorInvalidValue;
+    CapArgs a{grid, cell_pos, n_cells, rows, cols, scores, idx, M, M_stride, pscores, pidx, k0, p_stride, n_images, repeat_range,
+              repeat_addition, max_uses, counts, used, margins, rows_per_block, block_stride};
+    select_capped_kernel<<<1, kCapThreads, 0, stream>>>(a);
+    return cudaGetLastError();
+}
+
 }  // namespace mm

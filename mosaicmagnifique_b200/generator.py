@@ -320,6 +320,13 @@ class PhotomosaicGenerator:
             out.append(g)
         return out
 
+    # ---- usage limit (no reference counterpart, include/mosaic_b200.h "usage limit")
+    def setUsageLimit(self, maxUses: int = 0):
+        """Lets each library image be chosen at most maxUses times per generate, over all size steps (1 = no duplicates, 0 = unlimited).
+        Cells are decided in step and raster order, each taking the best image that is still allowed; generateBestFits() raises
+        MosaicError when maxUses * library size is less than the number of cells."""
+        self._ck(self._L.mosaic_set_usage_limit(self._h, int(maxUses)))
+
     def buildPhotomosaic(self, backgroundColour=(0, 0, 0, 0)) -> np.ndarray:
         """PhotomosaicGeneratorBase::buildPhotomosaic(const cv::Scalar&): H x W x 4 uint8 BGRA mosaic."""
         rows, cols = self._main_shape
