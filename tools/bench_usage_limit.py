@@ -34,7 +34,7 @@ def gpu_info():
 
 
 def step_bounds(cells, N, rr, ra, M):
-    """K_s and the (prefix length, candidate row length) the engine uses per step (generator.cu::run_pipeline)"""
+    """K_s and the (prefix length, candidate row length) the engine uses per step (generator.cu::plan_step)"""
     from tests.helpers.usage_limit import PREFIX_MAX, exhausted_bound, k_bound
     out, before = [], 0
     for n in cells:
