@@ -220,6 +220,11 @@ int mosaic_kernel_colour_difference(int device, int type, const float *a, const 
  * of diff(cell[p], lib[i][p]) -- imageDifference(+Edge) + reduceAdd + flatten */
 int mosaic_kernel_image_difference_sum(int device, int type, const float *cell, const float *lib, int64_t n_lib,
                                        const uint8_t *mask, int size, const int32_t *target_area, float *out);
+/* CIEDE2000 pruning bound (no reference counterpart): n_cells cells against n_lib images, pixel axis cut into segments of
+   seg_chunks 128-pixel chunks of the compacted mask; out [n_segs - 1][n_cells][n_lib] = R[s - 1], a lower bound of what
+   segments s .. n_segs - 1 add to the pair's difference sum */
+int mosaic_kernel_prune_bound(int device, const float *cells, int n_cells, const float *lib, int64_t n_lib, const uint8_t *mask,
+                              int size, const int32_t *target_area, int seg_chunks, float *out);
 /* calculateRepeats + findLowest over a whole grid: scores [n_valid][n_lib] (raster order of valid cells) */
 int mosaic_kernel_select(int device, const float *scores, int64_t n_lib, int64_t *grid, int rows, int cols,
                          int repeat_range, int repeat_addition);

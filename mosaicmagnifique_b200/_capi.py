@@ -96,6 +96,7 @@ def capi():
         "mosaic_get_library_device": (i, [vp, c.POINTER(vp), ip, i64p]),
         "mosaic_kernel_colour_difference": (i, [i, i, vp, vp, i64, vp]),
         "mosaic_kernel_image_difference_sum": (i, [i, i, vp, vp, i64, vp, i, vp, vp]),
+        "mosaic_kernel_prune_bound": (i, [i, vp, i, vp, i64, vp, i, vp, i, vp]),
         "mosaic_kernel_select": (i, [i, vp, i64, vp, i, i, i, i]),
         "mosaic_kernel_topk": (i, [i, vp, i64, i64, i, vp, vp]),
         "mosaic_kernel_bgr_to_lab": (i, [i, vp, i64, vp]),

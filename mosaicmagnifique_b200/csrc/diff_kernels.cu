@@ -378,13 +378,104 @@ cudaError_t launch_diff_rows(const void *cells, const void *lib, float *D, int n
     return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------- lightness bound of the segments not yet summed (DESIGN.md 4.1)
+
+// Per pixel the kernel's value is sqrt(N) / den25 with N = X^2 + Y (Y + R_T Z) + Z^2 (colour_math.cuh). For |R_T| < 2 the part
+// after X^2 is a positive semi-definite form, so N >= X^2 and dE/50 >= |X| / den25 = |dLh| / sl25, sl25 = 25 S_L(lm), lm = Lbar - 50
+// = Lh_cell + Lh_lib. S_L = 1 + 0.015 lm^2 / sqrt(20 + lm^2) <= 1 + 0.015 |lm| because sqrt(20 + lm^2) >= |lm|, and S_L grows with
+// |lm|. Over a block of MM_BB compacted pixels where every cell weight is w, the triangle inequality gives
+//     sum_p w |dLh_p| / sl25_p  >=  w |sum_p Lh_lib,p - sum_p Lh_cell,p| / (25 + 0.375 m),   m = max(|lo|, |hi|),
+// with lo = min Lh_cell + min Lh_lib <= lm_p <= max Lh_cell + max Lh_lib = hi. A block whose weights differ contributes 0.
+//
+// Rounding. The block sums are FP32 sums of 16 values |Lh| <= 25: each is within 15 * 2^-24 * 400 < 3.6e-4 of its exact value and
+// their difference adds < 4.8e-5, so kSumErr = 2^-10 is subtracted from every |difference| (this also covers pixels whose |dLh| <
+// 1e-19 flush to a zero N under ftz). What remains is relative: the kernel's per-pixel value is within ~1e-5 of the formula
+// (rsqrt.approx / sqrt.approx, colour_math.cuh; the tiny terms only raise t and leave rsq(N den^2 + tiny) within 1e-18 of
+// rsq(N den^2) since N >= 1e-12 whenever dLh != 0), a pair's FP32 sums of at most 16,384 non-negative terms lose < 1e-3 -- all
+// in the direction that could put a computed sum below its exact value -- and this kernel's own rcp.approx and FP32 sums of
+// non-negative terms lose < 3e-4. kSlack = 1 - 2^-8 covers all of it: R stays below what the kernels will sum. The dropped dTheta
+// Gaussian and the R_T polynomial enter only through R_T, and the bound holds for any |R_T| < 2.
+constexpr int kBoundThreads = 128, kBoundRows = 8;
+constexpr float kSumErr = 0x1p-10f, kSlack = 1.0f - 0x1p-8f;
+
+// One thread per library slot (coalesced over lib_stats and R) and kBoundRows cell rows (their statistics are warp-uniform loads).
+// Segments are walked from the last, so that every R[s] is the running suffix sum.
+__global__ void __launch_bounds__(kBoundThreads)
+prune_bound_kernel(const float4 *__restrict__ lib_stats, const float4 *__restrict__ cell_stats, int n_rows, int n_lib_pad, int n_blocks,
+                   int seg_blocks, int n_segs, float *__restrict__ R, const float *__restrict__ D, const int *__restrict__ perm,
+                   float *__restrict__ score)
+{
+    const int slot = blockIdx.x * kBoundThreads + threadIdx.x;
+    const int row0 = blockIdx.y * kBoundRows;
+    if (slot >= n_lib_pad)
+        return;
+    const int nr = min(kBoundRows, n_rows - row0);
+    const size_t plane = (size_t)n_rows * n_lib_pad;
+    float suffix[kBoundRows];
+#pragma unroll
+    for (int r = 0; r < kBoundRows; ++r)
+        suffix[r] = 0.0f;
+    for (int seg = n_segs - 1; seg >= 1; --seg) {
+        float acc[kBoundRows];
+#pragma unroll
+        for (int r = 0; r < kBoundRows; ++r)
+            acc[r] = 0.0f;
+        const int b1 = min(n_blocks, (seg + 1) * seg_blocks);
+        for (int b = seg * seg_blocks; b < b1; ++b) {
+            const float4 l = lib_stats[(size_t)b * n_lib_pad + slot];
+#pragma unroll
+            for (int r = 0; r < kBoundRows; ++r) {
+                const float4 c = cell_stats[(size_t)min(row0 + r, n_rows - 1) * n_blocks + b];  // (sum, min, max, w)
+                const float d = fmaxf(fabsf(l.x - c.x) - kSumErr, 0.0f);
+                const float m = fmaxf(fabsf(l.y + c.y), fabsf(l.z + c.z));
+                acc[r] = fmaf(c.w * d, mm_rcp(fmaf(25.0f * 0.015f, m, 25.0f)), acc[r]);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < kBoundRows; ++r) {
+            suffix[r] += acc[r];
+            if (r < nr)
+                R[(size_t)(seg - 1) * plane + (size_t)(row0 + r) * n_lib_pad + slot] = suffix[r] * kSlack;
+        }
+    }
+    if (score) {
+        const int j = perm[slot];
+#pragma unroll
+        for (int r = 0; r < kBoundRows; ++r)
+            if (r < nr) {
+                const size_t e = (size_t)(row0 + r) * n_lib_pad + j;
+                score[e] = D[e] + suffix[r] * kSlack;
+            }
+    }
+}
+
+cudaError_t launch_prune_bound(const float4 *lib_stats, const float4 *cell_stats, int n_rows, int n_lib_pad, int n_blocks, int seg_blocks,
+                               int n_segs, float *R, const float *D, const int *perm, float *score, cudaStream_t stream)
+{
+    if (n_rows <= 0 || n_lib_pad <= 0 || n_segs < 2)
+        return cudaSuccess;
+    if (seg_blocks <= 0 || (score && (!D || !perm)))
+        return cudaErrorInvalidValue;
+    const dim3 grid((unsigned)((n_lib_pad + kBoundThreads - 1) / kBoundThreads), (unsigned)((n_rows + kBoundRows - 1) / kBoundRows));
+    prune_bound_kernel<<<grid, kBoundThreads, 0, stream>>>(lib_stats, cell_stats, n_rows, n_lib_pad, n_blocks, seg_blocks, n_segs, R, D, perm,
+                                                           score);
+    return cudaGetLastError();
+}
+
 // One CTA per bucket (column of col_cells cells x one library tile), one thread per cell. A cell is listed when its row is in
-// state `want`; with a threshold T (pruning) an active row is listed only while one of its pairs still has a partial sum <= T[cell]
-// -- otherwise it dies: its pairs become +inf (their complete sums are > T, top-K can never take them) and its remaining segments
-// count as done. Listing keeps cell order, so the lists do not depend on scheduling.
+// state `want`; with a threshold T (pruning) an active row is listed only while one of its pairs still has a partial sum plus R,
+// the bound of the segments not yet summed, <= T[cell] -- otherwise it dies: its pairs become +inf (their complete sums are > T,
+// top-K can never take them) and its remaining segments count as done. Listing keeps cell order, so the lists do not depend on
+// scheduling.
+//
+// Why a pair with fl(P + R) > T has a complete sum C > T (P = partial sum, C its continuation in FP32): the later segments'
+// computed sums add up to at least R (1 - 1.01e-3) / ((1 - 2^-8)(1 + 3e-4)) > R (1 + 2.6e-3) (kSlack above), and C and fl(P + R)
+// round each of their n <= n_segs additions of non-negative terms by <= 2^-24 of the result, so C - fl(P + R) >= 2.6e-3 R -
+// n 2^-24 (P + R) > 0 whenever R >= 2^-8 P and n <= 168. A smaller R is not used (the test is then the plain P > T, exact because
+// partial sums only grow); at under 1/256 of the partial sum it would prune next to nothing anyway.
 __global__ void __launch_bounds__(1024)
 list_rows_kernel(float *__restrict__ D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *__restrict__ state, int want,
-                 const float *__restrict__ T, const int *__restrict__ perm, int segs_left, RowList rows,
+                 const float *__restrict__ T, const float *__restrict__ R, const int *__restrict__ perm, int segs_left, RowList rows,
                  int *__restrict__ group_count, unsigned long long *__restrict__ listed, unsigned long long *__restrict__ progress)
 {
     __shared__ int warp_sum[32];
@@ -398,10 +489,14 @@ list_rows_kernel(float *__restrict__ D, int n_lib_pad, int n_lib, int n_rows, in
         if (on && T) {
             const float t = T[cell];
             float *row = D + (size_t)cell * n_lib_pad;
+            const float *rest = R ? R + (size_t)cell * n_lib_pad + lib_tile * MM_TNB : nullptr;
             bool alive = false;
             for (int i = 0; i < MM_TNB; ++i) {
                 const int j = perm[lib_tile * MM_TNB + i];
-                alive = alive || (j < n_lib && row[j] <= t);
+                if (j < n_lib) {
+                    const float p = row[j], r = rest ? rest[i] : 0.0f;
+                    alive = alive || p + (r >= p * 0x1p-8f ? r : 0.0f) <= t;
+                }
             }
             if (!alive) {
                 for (int i = 0; i < MM_TNB; ++i)
@@ -442,7 +537,7 @@ size_t list_rows_scratch_bytes(int n_buckets)
 }
 
 cudaError_t launch_list_rows(float *D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *state, int want, const float *T,
-                             const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
+                             const float *R, const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
                              unsigned long long *listed, unsigned long long *progress, cudaStream_t stream)
 {
     const int n_cols = (n_rows + rows.col_cells - 1) / rows.col_cells;
@@ -457,7 +552,7 @@ cudaError_t launch_list_rows(float *D, int n_lib_pad, int n_lib, int n_rows, int
     if (e != cudaSuccess)
         return e;
     list_rows_kernel<<<dim3((unsigned)n_lib_tiles, (unsigned)n_cols), rows.col_cells, 0, stream>>>(
-        D, n_lib_pad, n_lib, n_rows, n_lib_tiles, state, want, T, perm, segs_left, rows, group_count, listed, progress);
+        D, n_lib_pad, n_lib, n_rows, n_lib_tiles, state, want, T, R, perm, segs_left, rows, group_count, listed, progress);
     if ((e = cudaGetLastError()) != cudaSuccess)
         return e;
     size_t temp = scratch_bytes - head;

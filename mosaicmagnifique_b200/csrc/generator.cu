@@ -109,6 +109,7 @@ struct Workspace {
     // segment passes over row work lists (kernels.h: RowList) and exact pruning
     DevBuf perm, inv_perm, order_scratch, row_cells, row_count, row_groups, list_scratch, row_state, listed, prune_score, prune_idx,
         threshold;
+    DevBuf lib_stats, cell_stats, prune_rest, prune_rank;  // lightness bound of the segments not yet summed (launch_prune_bound)
     DevBuf prefix_score, prefix_idx;  // usage limit: sorted prefixes of D rows, or launch_topk's pick for a candidate list's prefix
 };
 
@@ -982,9 +983,9 @@ double difference_sums(G *g, const Run &r, size_t s, const StepWork &w, Progress
     }
     double units = 0;  // rows x chunks evaluated
     int n_groups = 0;
-    auto list = [&](uint8_t *st8, int want, const float *T, int segs_left) {
+    auto list = [&](uint8_t *st8, int want, const float *T, const float *R, int segs_left) {
         CU(cudaMemsetAsync(d.listed.p, 0, sizeof(unsigned long long), st));
-        CU(launch_list_rows(D.as<float>(), r.n_lib_pad, (int)r.N, w.n_rows_local, r.n_lib_tiles, st8, want, T, perm, segs_left, rows,
+        CU(launch_list_rows(D.as<float>(), r.n_lib_pad, (int)r.N, w.n_rows_local, r.n_lib_tiles, st8, want, T, R, perm, segs_left, rows,
                             d.list_scratch.p, d.list_scratch.bytes, d.listed.as<unsigned long long>(), prog.d_done, st));
         CU(cudaMemcpyAsync(g->h_progress + 1, rows.groups + rows.n_buckets, sizeof(int), cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(g->h_progress + 2, d.listed.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
@@ -1000,23 +1001,44 @@ double difference_sums(G *g, const Run &r, size_t s, const StepWork &w, Progress
         tm.kernel_launches += n_groups > 0;
         units += n_listed * nk;
     };
-    double n_listed = list(nullptr, kRowActive, nullptr, 0);  // every row
+    double n_listed = list(nullptr, kRowActive, nullptr, nullptr, 0);  // every row
     if (!w.prune) {
         for (int seg = 0; seg < w.n_segs; ++seg)
             pass(seg, n_listed);
     } else {
         pass(0, n_listed);
-        // candidates = the M smallest partial sums of segment 0; their tiles are completed first, T[cell] = the k_need-th smallest
-        // of their complete sums, and every later pass lists only the rows that still have a pair <= T
+        // R[s - 1][cell][slot]: lower bound of what segments s .. n_segs - 1 add to a pair (launch_prune_bound; its rounding argument
+        // holds up to 168 segments), and the candidates' ranking D + R[0]
+        const float *rank = D.as<float>();
+        const float *rest = nullptr;
+        const size_t plane = (size_t)w.n_rows_local * r.n_lib_pad;
+        if (w.n_segs > 1 && w.n_segs <= 168) {
+            const int n_blocks = p.n_chunks * (MM_KP / MM_BB);
+            d.lib_stats.alloc((size_t)n_blocks * r.n_lib_pad * sizeof(float4), st);
+            d.cell_stats.alloc((size_t)w.n_rows_local * n_blocks * sizeof(float4), st);
+            d.prune_rest.alloc((w.n_segs - 1) * plane * sizeof(float), st);
+            d.prune_rank.alloc(plane * sizeof(float), st);
+            CU(launch_block_stats(d.lib_packed.p, r.n_lib_tiles, d.cells_packed.p, w.n_rows_local, p.n_chunks, d.lib_stats.as<float4>(),
+                                  d.cell_stats.as<float4>(), st));
+            CU(launch_prune_bound(d.lib_stats.as<float4>(), d.cell_stats.as<float4>(), w.n_rows_local, r.n_lib_pad, n_blocks,
+                                  w.seg_chunks * (MM_KP / MM_BB), w.n_segs, d.prune_rest.as<float>(), D.as<float>(), perm,
+                                  d.prune_rank.as<float>(), st));
+            tm.kernel_launches += 2;
+            rank = d.prune_rank.as<float>();
+            rest = d.prune_rest.as<float>();
+        }
+        // candidates = the M smallest of pass 0's partial sum + R[0]; their tiles are completed first, T[cell] = the k_need-th
+        // smallest of their complete sums, and every later pass lists only the rows that still have a pair with partial sum + the
+        // bound of the segments not yet summed <= T
         d.prune_score.alloc((size_t)w.n_rows_local * w.M * sizeof(float), st);
         d.prune_idx.alloc((size_t)w.n_rows_local * w.M * sizeof(int), st);
         d.threshold.alloc((size_t)w.n_rows_local * sizeof(float), st);
-        CU(launch_topk(D.as<float>(), r.n_lib_pad, (int)r.N, w.n_rows_local, w.M, d.prune_score.as<float>(), d.prune_idx.as<int>(), st));
+        CU(launch_topk(rank, r.n_lib_pad, (int)r.N, w.n_rows_local, w.M, d.prune_score.as<float>(), d.prune_idx.as<int>(), st));
         CU(launch_prune_threshold(D.as<float>(), r.n_lib_pad, d.prune_idx.as<int>(), w.n_rows_local, w.M, (int)w.k_need,
                                   d.inv_perm.as<int>(), r.n_lib_tiles, state, nullptr, true, st));
         tm.kernel_launches += 2;
         if (w.n_segs > 1) {
-            n_listed = list(state, kRowComplete, nullptr, 0);
+            n_listed = list(state, kRowComplete, nullptr, nullptr, 0);
             for (int seg = 1; seg < w.n_segs; ++seg)
                 pass(seg, n_listed);
         }
@@ -1024,7 +1046,7 @@ double difference_sums(G *g, const Run &r, size_t s, const StepWork &w, Progress
                                   d.inv_perm.as<int>(), r.n_lib_tiles, state, d.threshold.as<float>(), false, st));
         tm.kernel_launches++;
         for (int seg = 1; seg < w.n_segs; ++seg) {
-            n_listed = list(state, kRowActive, d.threshold.as<float>(), w.n_segs - seg);
+            n_listed = list(state, kRowActive, d.threshold.as<float>(), rest ? rest + (size_t)(seg - 1) * plane : nullptr, w.n_segs - seg);
             pass(seg, n_listed);
         }
     }

@@ -55,8 +55,10 @@ int use_device(int device)
 }
 
 // cells: n_cells images [size*size][3] f32 treated as "main images" of their own; lib: n_lib images
+// seg_chunks > 0 (CIEDE2000): instead of the sums, the pruning bound R of segments of seg_chunks chunks (launch_prune_bound) goes to
+// out [n_segs - 1][n_cells][n_lib]
 int difference_sums(int type, const float *cells, int n_cells, const float *lib, int64_t n_lib, const uint8_t *mask, int size,
-                    const int32_t *target_area, float *out /* [n_cells][n_lib] */)
+                    const int32_t *target_area, float *out /* [n_cells][n_lib] */, int seg_chunks = 0)
 {
     const int P = size * size;
     std::vector<int> pix;
@@ -106,6 +108,21 @@ int difference_sums(int type, const float *cells, int n_cells, const float *lib,
     KCHECK(launch_extract_cells(d_cells.as<float>(), n_cells * size, size, d_desc.as<CellDesc>(), n_cells, size, size, 1,
                                 AreaTab{nullptr, nullptr, nullptr}, d_m4.as<uint8_t>(), d_pix.as<int>(), n_active, n_chunks, d_cp.p,
                                 layout, 0));
+    if (chroma && seg_chunks > 0) {
+        const int n_blocks = n_chunks * (MM_KP / MM_BB), n_segs = (n_chunks + seg_chunks - 1) / seg_chunks;
+        if (n_segs < 2)
+            return MOSAIC_ERR_INVALID_ARGUMENT;
+        Dev d_ls, d_cs, d_R;
+        KCHECK(d_ls.alloc((size_t)n_blocks * n_lib_pad * sizeof(float4)));
+        KCHECK(d_cs.alloc((size_t)n_cells * n_blocks * sizeof(float4)));
+        KCHECK(d_R.alloc((size_t)(n_segs - 1) * n_cells * n_lib_pad * sizeof(float)));
+        KCHECK(launch_block_stats(d_lp.p, n_lib_tiles, d_cp.p, n_cells, n_chunks, d_ls.as<float4>(), d_cs.as<float4>(), 0));
+        KCHECK(launch_prune_bound(d_ls.as<float4>(), d_cs.as<float4>(), n_cells, n_lib_pad, n_blocks, seg_chunks * (MM_KP / MM_BB), n_segs,
+                                  d_R.as<float>(), nullptr, nullptr, nullptr, 0));
+        KCHECK(cudaMemcpy2D(out, (size_t)n_lib * sizeof(float), d_R.p, (size_t)n_lib_pad * sizeof(float), (size_t)n_lib * sizeof(float),
+                            (size_t)(n_segs - 1) * n_cells, cudaMemcpyDeviceToHost));
+        return MOSAIC_OK;
+    }
     if (chroma)
         KCHECK(launch_diff_sum(MM_DIFF_CIEDE2000, d_cp.p, d_lp.p, d_D.as<float>(), nullptr, n_cell_tiles, n_lib_tiles, n_chunks, (int)n_lib,
                                n_cells, 0));
@@ -128,6 +145,16 @@ int mosaic_kernel_image_difference_sum(int device, int type, const float *cell, 
     if (int rc = use_device(device))
         return rc;
     return difference_sums(type, cell, 1, lib, n_lib, mask, size, target_area, out);
+}
+
+int mosaic_kernel_prune_bound(int device, const float *cells, int n_cells, const float *lib, int64_t n_lib, const uint8_t *mask, int size,
+                              const int32_t *target_area, int seg_chunks, float *out)
+{
+    if (!cells || !lib || !mask || !out || n_cells <= 0 || n_lib <= 0 || size <= 0 || seg_chunks <= 0)
+        return MOSAIC_ERR_INVALID_ARGUMENT;
+    if (int rc = use_device(device))
+        return rc;
+    return difference_sums(MOSAIC_CIEDE2000, cells, n_cells, lib, n_lib, mask, size, target_area, out, seg_chunks);
 }
 
 int mosaic_kernel_colour_difference(int device, int type, const float *a, const float *b, int64_t n, float *out)

@@ -125,11 +125,18 @@ cudaError_t launch_diff_rows(const void *cells, const void *lib, float *D, int n
                              RowList rows, const int *perm, cudaStream_t stream, const int *cancel = nullptr,
                              unsigned long long *progress = nullptr);
 // lists the rows in state `want` (state null: every row) into rows.cells / rows.count / rows.groups (rows.groups[n_buckets] = groups
-// in all); with T: active rows whose pairs all have partial sums > T die (pairs -> +inf, progress += segs_left); listed += rows listed
+// in all); with T: active rows whose pairs all have partial sum + R > T die (pairs -> +inf, progress += segs_left); listed += rows
+// listed. R (optional, [n_rows][n_lib_pad] in SLOT order): launch_prune_bound's lower bound of the segments not yet summed.
 size_t list_rows_scratch_bytes(int n_buckets);
 cudaError_t launch_list_rows(float *D, int n_lib_pad, int n_lib, int n_rows, int n_lib_tiles, uint8_t *state, int want, const float *T,
-                             const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
+                             const float *R, const int *perm, int segs_left, RowList rows, void *scratch, size_t scratch_bytes,
                              unsigned long long *listed, unsigned long long *progress, cudaStream_t stream);
+// Lightness lower bound of the CIEDE2000 segments not yet summed (DESIGN.md 4.1), from launch_block_stats' statistics.
+// R [n_segs - 1][n_rows][n_lib_pad], slot order: R[s - 1][row][slot] <= the sum that segments s .. n_segs - 1 will add to the pair
+// (row, image perm[slot]), s = 1 .. n_segs - 1. score (optional, [n_rows][n_lib_pad], image order): D + R[0], pass 0's partial
+// sum plus the bound of the rest, which ranks the pruning candidates.
+cudaError_t launch_prune_bound(const float4 *lib_stats, const float4 *cell_stats, int n_rows, int n_lib_pad, int n_blocks, int seg_blocks,
+                               int n_segs, float *R, const float *D, const int *perm, float *score, cudaStream_t stream);
 
 // ---- prep_kernels.cu
 // u8 BGR -> working space f32 AoS [pixel][3]: Lab through the OpenCV-compatible LUT (is_lab) or a plain cast.
@@ -193,6 +200,15 @@ cudaError_t launch_pack_library_ciede(const void *src, bool src_is_u8, void *pac
 cudaError_t launch_pack_library_euclid_u8(const uint8_t *lib, int src_size, int k, bool is_lab, void *packed, int64_t n, int P,
                                           const int *pix_list, int n_active, int n_chunks, int n_lib_tiles, const short4 *lab_lut,
                                           cudaStream_t stream);
+
+// Block statistics of the packed CIEDE2000 tiles for the pruning bound (launch_prune_bound): a block is a run of MM_BB compacted
+// pixels inside a chunk, n_blocks = n_chunks * MM_KP / MM_BB. Stored lightness Lh = L/2 - 25.
+//   lib_stats  [n_blocks][n_lib_tiles * MM_TNB] (sum Lh, min Lh, max Lh, 0) per library slot
+//   cell_stats [n_rows][n_blocks]             (sum Lh, min Lh, max Lh, w) per cell row; w = the weight every pixel of the block has,
+//                                              0 when the weights differ (clipped edges, flipped masks, detail-space bounds)
+#define MM_BB 16
+cudaError_t launch_block_stats(const void *lib_packed, int n_lib_tiles, const void *cells_packed, int n_rows, int n_chunks,
+                               float4 *lib_stats, float4 *cell_stats, cudaStream_t stream);
 
 struct CellDesc {
     int x0, y0;          // top-left of the (unclipped) cell rect in main-image space

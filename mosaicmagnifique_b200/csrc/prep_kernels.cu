@@ -592,6 +592,74 @@ cudaError_t launch_pack_library_ciede(const void *src, bool src_is_u8, void *pac
     return cudaGetLastError();
 }
 
+// Block statistics for the pruning bound (kernels.h: launch_block_stats), read from the packed tiles so that they follow the tiles'
+// compacted pixel order and slot order. One thread per (library pair slot, block) -- both images of the pair share the float4 that
+// holds their L -- then one per (cell row, block). Sums run in FP32, in pixel order; launch_prune_bound allows for their rounding.
+__global__ void block_stats_kernel(const unsigned char *__restrict__ lib, int64_t n_pair_slots, const unsigned char *__restrict__ cells,
+                                   int n_rows, int n_chunks, float4 *__restrict__ lib_stats, float4 *__restrict__ cell_stats)
+{
+    constexpr int kBlocksPerChunk = MM_KP / MM_BB;
+    const int n_blocks = n_chunks * kBlocksPerChunk;
+    const size_t n_lib_items = (size_t)n_blocks * n_pair_slots;
+    const size_t total = n_lib_items + (size_t)n_rows * n_blocks;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        if (i < n_lib_items) {
+            const int b = (int)(i / n_pair_slots);
+            const int64_t pr = (int64_t)(i % n_pair_slots);
+            const int64_t tile = pr / (MM_TNB / 2);
+            const int tp = (int)(pr % (MM_TNB / 2)), chunk = b / kBlocksPerChunk, p0 = (b % kBlocksPerChunk) * MM_BB;
+            // [pair][0][p] = (L0, L1, a0, a1) (pack_library_ciede_kernel)
+            const float4 *v = reinterpret_cast<const float4 *>(lib + ((size_t)tile * n_chunks + chunk) * (size_t)(MM_TNB * MM_KP * 16)) +
+                              (tp * 2) * MM_KP + p0;
+            float s0 = 0.0f, s1 = 0.0f, lo0 = INFINITY, lo1 = INFINITY, hi0 = -INFINITY, hi1 = -INFINITY;
+#pragma unroll
+            for (int p = 0; p < MM_BB; ++p) {
+                const float4 q = v[p];
+                s0 += q.x;
+                s1 += q.y;
+                lo0 = fminf(lo0, q.x);
+                hi0 = fmaxf(hi0, q.x);
+                lo1 = fminf(lo1, q.y);
+                hi1 = fmaxf(hi1, q.y);
+            }
+            float4 *out = lib_stats + (size_t)b * n_pair_slots * 2 + pr * 2;
+            out[0] = make_float4(s0, lo0, hi0, 0.0f);
+            out[1] = make_float4(s1, lo1, hi1, 0.0f);
+        } else {
+            const size_t j = i - n_lib_items;
+            const int row = (int)(j / n_blocks), b = (int)(j % n_blocks);
+            const int chunk = b / kBlocksPerChunk, p0 = (b % kBlocksPerChunk) * MM_BB;
+            const unsigned char *blk = cells + ((size_t)(row / MM_TCB) * n_chunks + chunk) * (size_t)(MM_TCB * MM_KP * 20);
+            const float4 *c = reinterpret_cast<const float4 *>(blk) + (row % MM_TCB) * MM_KP + p0;
+            const float *w = reinterpret_cast<const float *>(blk + (size_t)MM_TCB * MM_KP * 16) + (row % MM_TCB) * MM_KP + p0;
+            const float w0 = w[0];
+            float s = 0.0f, lo = INFINITY, hi = -INFINITY;
+            bool uniform = true;
+#pragma unroll
+            for (int p = 0; p < MM_BB; ++p) {
+                const float x = c[p].x;
+                s += x;
+                lo = fminf(lo, x);
+                hi = fmaxf(hi, x);
+                uniform = uniform && w[p] == w0;
+            }
+            cell_stats[j] = make_float4(s, lo, hi, uniform ? w0 : 0.0f);
+        }
+    }
+}
+
+cudaError_t launch_block_stats(const void *lib_packed, int n_lib_tiles, const void *cells_packed, int n_rows, int n_chunks,
+                               float4 *lib_stats, float4 *cell_stats, cudaStream_t stream)
+{
+    static_assert(MM_KP % MM_BB == 0, "a block lies inside one chunk");
+    const size_t total = ((size_t)n_lib_tiles * (MM_TNB / 2) + (size_t)n_rows) * n_chunks * (MM_KP / MM_BB);
+    if (total == 0)
+        return cudaSuccess;
+    block_stats_kernel<<<grid_for(total, 256), 256, 0, stream>>>((const unsigned char *)lib_packed, (int64_t)n_lib_tiles * (MM_TNB / 2),
+                                                                 (const unsigned char *)cells_packed, n_rows, n_chunks, lib_stats, cell_stats);
+    return cudaGetLastError();
+}
+
 // Colour order of the library (exact pruning groups similar images into one tile): key = Morton code of each image's mean colour,
 // 10 bits per channel. The means are exact integer sums over the 8-bit pixels, so every rank and every run gets the same order;
 // the 5-bit Morton order is a prefix of the 10-bit one, so the key keeps locality at every scale however narrow the colour range.
