@@ -161,6 +161,36 @@ int mosaic_get_best_fit_flips(const mosaic_generator *g, int step, int8_t *out, 
  * MOSAIC_ERR_INVALID_ARGUMENT for M < 0. */
 int mosaic_set_usage_limit(mosaic_generator *g, int max_uses);
 
+/* ---- scaled compositing (no reference counterpart: the reference composites at the main image's size, from the library it
+ * matched with). Print wants tiles with far more pixels than matching needs; these two calls build the mosaic at k times the main
+ * image's size without matching at that size.
+ * mosaic_set_render_library: the render library -- the SAME n images as the library, in the same index order, square 8U BGR at
+ *   side size = R, contiguous, host OR device pointer. It is copied to the device and stays resident until replaced; n = 0 clears it.
+ *   The copy runs on the handle's own stream, which does not wait for work on other streams: device data must be complete when the
+ *   call is made (e.g. torch.cuda.synchronize() after the kernels that wrote it).
+ *   Nothing is checked against the cell group here (it may be set later), and the plain build never uses it.
+ *   MOSAIC_ERR_INVALID_ARGUMENT for n < 0, size < 1, or bgr == NULL with n > 0.
+ * mosaic_build_photomosaic_scaled: with S the cell size of step 0 and k = R / S, writes a (k * H) x (k * W) 8U BGRA image (rows, cols)
+ *   that is exactly what buildPhotomosaic (PhotomosaicGeneratorBase.cpp:110-207) produces from
+ *     - a main image of k * H x k * W, the render library and the same best fits (slots with tile flips) and background;
+ *     - the k-scaled cell group: per step the normal cell with size, row / col spacing, alternate spacings and alternate offsets
+ *       times k (flip flags unchanged) and its mask upsampled by nearest neighbour (every mask pixel a k x k block).
+ *   So each cell's rect is k times its rect at scale 1 and the output pixel (Y, X) comes from the tile of the cell that owns base
+ *   pixel (Y / k, X / k), at (Y - k * y0, X - k * x0) of the render tile. The render tiles of size step s are the step s - 1 tiles
+ *   halved with 8U INTER_AREA (side k * S_s); a step after an odd cell size gives MOSAIC_ERR_UNSUPPORTED, as the plain build does.
+ *   With tile flips slot j * N + i places render image i mirrored by orientation j. Tile pixels get alpha 255, uncovered pixels the
+ *   background. k = 1 with the render library equal to the library is byte-identical to mosaic_build_photomosaic.
+ *   The library at the cell size is not needed, so a handle loaded with mosaic_set_library_shard can build (after
+ *   mosaic_select_from_gathered). out: 4-byte aligned device memory of the handle's GPU is written in place; any other pointer
+ *   (pinned or pageable host memory, an unaligned address) is filled through device bands of about 256 MB. Bytes past cols * 4 in
+ *   each row are left untouched.
+ *   MOSAIC_ERR_NOT_READY: no render library, or no best fits on the current grid state. MOSAIC_ERR_INVALID_ARGUMENT (the text gives
+ *   the numbers): render n != the library's N (n_total of a sharded handle), R not a multiple of S, rows != k * H or cols != k * W,
+ *   k * H or k * W above INT_MAX, row_stride < cols * 4 or not a multiple of 4. */
+int mosaic_set_render_library(mosaic_generator *g, const uint8_t *bgr, int64_t n, int size);
+int mosaic_build_photomosaic_scaled(mosaic_generator *g, const uint8_t background_bgra[4], uint8_t *out_bgra, int rows, int cols,
+                                    size_t row_stride);
+
 /* ---- parity / measurement taps (no reference counterpart; used by tests and bench.py) */
 /* keep the full difference matrix of every step on the device so it can be read back */
 int mosaic_set_keep_differences(mosaic_generator *g, int keep);

@@ -324,6 +324,13 @@ public:
     {
         ck(mosaic_build_photomosaic(m_g, backgroundBGRA, outBGRA, rows, cols, step));
     }
+    // ---- scaled compositing (no reference counterpart; see mosaic_b200.h "scaled compositing"): the library's images, same order, at
+    // side R = k * cell size; buildPhotomosaicScaled then fills a (k * rows) x (k * cols) BGRA buffer (host or device memory)
+    void setRenderLibrary(const uint8_t *bgr, int64_t n, int size) { ck(mosaic_set_render_library(m_g, bgr, n, size)); }
+    void buildPhotomosaicScaled(const uint8_t backgroundBGRA[4], uint8_t *outBGRA, int rows, int cols, size_t step)
+    {
+        ck(mosaic_build_photomosaic_scaled(m_g, backgroundBGRA, outBGRA, rows, cols, step));
+    }
     int getMaxProgress() { return mosaic_get_max_progress(m_g); }
     // slot cancel(): callable from any thread or from inside the progress callback; the running kernel drains within milliseconds
     // and generateBestFits() returns false. Sticky like the reference's m_wasCanceled until resetCancel().

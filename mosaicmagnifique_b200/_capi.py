@@ -72,6 +72,8 @@ def capi():
         "mosaic_get_best_fit_flips": (i, [vp, i, vp, i, i]),
         "mosaic_set_usage_limit": (i, [vp, i]),
         "mosaic_build_photomosaic": (i, [vp, vp, vp, i, i, sz]),
+        "mosaic_set_render_library": (i, [vp, vp, i64, i]),
+        "mosaic_build_photomosaic_scaled": (i, [vp, vp, vp, i, i, sz]),
         "mosaic_get_max_progress": (i, [vp]),
         "mosaic_set_progress_callback": (None, [vp, PROGRESS_FN, vp]),
         "mosaic_cancel": (None, [vp]),

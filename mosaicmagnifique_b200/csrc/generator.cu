@@ -209,6 +209,10 @@ struct mosaic_generator : Handles {
     int cand_max_uses = 0;         // max_uses of the last mosaic_generate_candidates: its K and sorted prefixes were built for it
     int cap_last_step = -1;        // sharded selection: last step selected since `used` was reset (-1: none)
     DevBuf d_used;                 // [N] choices per source image so far in this generate
+    // render library (mosaic_set_render_library): the library's images at render_size = k * S for mosaic_build_photomosaic_scaled
+    DevBuf d_render;
+    int64_t render_n = 0;          // 0: none set
+    int render_size = 0;
 
     mosaic_progress_fn progress_fn = nullptr;
     void *progress_user = nullptr;
@@ -1823,6 +1827,100 @@ int mosaic_get_timings(const mosaic_generator *g, mosaic_timings *out)
 
 // ---- buildPhotomosaic (PhotomosaicGeneratorBase.cpp:110-207)
 
+}  // extern "C"
+
+namespace {
+
+// buildPhotomosaic at k times the main image's size from `lib`, the library's N images at side k * S (S = the cell size of step 0):
+// the reference procedure on a k-times larger main image with the k-scaled cell group (every tiling parameter times k, masks
+// upsampled by nearest neighbour). k = 1 with the matching library is buildPhotomosaic itself. A cell covers output pixel (Y, X)
+// exactly when it covers base pixel (Y / k, X / k) at scale 1, with the same step / raster priority, so the owner map is scattered at
+// the main image's size and only the gather runs at the output size.
+void build_mosaic(G *g, const uint8_t *lib, int k, const uint8_t background_bgra[4], uint8_t *out_bgra, size_t row_stride)
+{
+    // MM_BUILD_BAND_ROWS: rows per device band of a host-memory output (default: about 256 MB per band)
+    const char *eb = getenv("MM_BUILD_BAND_ROWS");
+    const int band_override = eb ? atoi(eb) : 0;
+    cudaStream_t st = g->stream;
+    const int H = g->img_rows, W = g->img_cols, n_steps = (int)g->grid.size();
+    const int rows = k * H, cols = k * W;
+    const int64_t N = g->n_lib;
+    // the grid holds slots j * N + i of the generate's orientations: image i, placed mirrored by orientation j
+    const int fl = std::max(g->fits_flips, 0), O = orient_count(fl);
+    DevBuf owner, d_steps, band;
+    std::vector<DevBuf> libs(n_steps), cells(n_steps), masks(n_steps);
+    std::vector<BuildStep> hsteps(n_steps);
+    owner.alloc((size_t)H * W * sizeof(unsigned long long), st);
+    CU(cudaMemsetAsync(owner.p, 0, owner.bytes, st));
+    const uint8_t *lib_s = lib;
+    for (int s = 0; s < n_steps; ++s) {
+        const Shape &shape = g->group.cells[s];
+        const GridStep &gs = g->grid[s];
+        if (s > 0) {
+            // the library at this step: halved like batchResizeMat(libImg) (8U INTER_AREA, round(0.5 * size)). The cell halves with
+            // integer division, so an odd previous cell size leaves library and cell a pixel apart.
+            const int S_prev = g->group.cells[s - 1].size;
+            if (S_prev % 2 != 0)
+                throw Fail{MOSAIC_ERR_UNSUPPORTED, "library and cell size disagree at step " + std::to_string(s) + " (cell size " +
+                                                       std::to_string(S_prev) + " of step " + std::to_string(s - 1) +
+                                                       " is odd; the reference copies out of range here)"};
+            const int side = k * shape.size;
+            libs[s].alloc((size_t)N * side * side * 3, st);
+            CU(launch_area_u8(lib_s, libs[s].as<uint8_t>(), N, 2 * side, 2, st));  // exact 2 x 2 means: commutes with mirroring
+            lib_s = libs[s].as<uint8_t>();
+        }
+        std::vector<BuildCell> hc;
+        for (int y = 0; y < gs.rows; ++y)
+            for (int x = 0; x < gs.cols; ++x) {
+                const int64_t v = gs.v[(size_t)y * gs.cols + x];
+                if (v < 0)
+                    continue;
+                if (v >= O * N)
+                    throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "best fit index outside the library"};
+                const Rect r = rect_at(shape, x - kPadGrid, y - kPadGrid);
+                hc.push_back(BuildCell{r.x, r.y, flip_at(shape, x - kPadGrid, y - kPadGrid), (int)hc.size() + 1, (int)(v % N),
+                                       orient_code(fl, (int)(v / N))});
+            }
+        const std::vector<uint8_t> m4 = shape.masks4();
+        masks[s].alloc(m4.size(), st);
+        CU(cudaMemcpyAsync(masks[s].p, m4.data(), m4.size(), cudaMemcpyHostToDevice, st));
+        cells[s].alloc(std::max<size_t>(hc.size(), 1) * sizeof(BuildCell), st);
+        CU(cudaMemcpyAsync(cells[s].p, hc.data(), hc.size() * sizeof(BuildCell), cudaMemcpyHostToDevice, st));
+        CU(launch_build_scatter(cells[s].as<BuildCell>(), (int)hc.size(), shape.size, masks[s].as<uint8_t>(), H, W, s, n_steps,
+                                owner.as<unsigned long long>(), st));
+        hsteps[s] = BuildStep{cells[s].as<BuildCell>(), lib_s, k * shape.size};
+    }
+    d_steps.alloc(hsteps.size() * sizeof(BuildStep), st);
+    CU(cudaMemcpyAsync(d_steps.p, hsteps.data(), d_steps.bytes, cudaMemcpyHostToDevice, st));
+    // 4-byte aligned device memory of this handle's GPU is written in place at the caller's stride (the callers check that the stride
+    // is a multiple of 4); anything else (pinned or pageable host memory, another device, an unaligned address) through device bands
+    // of bounded size and cudaMemcpy2DAsync, which takes any alignment, so device memory does not grow with the output
+    cudaPointerAttributes pa{};
+    const bool direct = ((uintptr_t)out_bgra & 3) == 0 && cudaPointerGetAttributes(&pa, out_bgra) == cudaSuccess &&
+                        pa.type == cudaMemoryTypeDevice && pa.device == g->device;
+    cudaGetLastError();
+    const unsigned long long *own = owner.as<unsigned long long>();
+    if (direct) {
+        CU(launch_build_gather(own, W, k, n_steps, d_steps.as<BuildStep>(), background_bgra, 0, rows, cols, out_bgra, row_stride, st));
+    } else {
+        const size_t row_bytes = (size_t)cols * 4;
+        const int band_rows = std::min<int64_t>(rows, band_override > 0 ? band_override : std::max<size_t>(1, (size_t(256) << 20) / row_bytes));
+        band.alloc((size_t)band_rows * row_bytes, st);
+        for (int y0 = 0; y0 < rows; y0 += band_rows) {
+            const int y1 = std::min(rows, y0 + band_rows);
+            CU(launch_build_gather(own, W, k, n_steps, d_steps.as<BuildStep>(), background_bgra, y0, y1, cols, band.as<uint8_t>(), row_bytes,
+                                   st));
+            CU(cudaMemcpy2DAsync(out_bgra + (size_t)y0 * row_stride, row_stride, band.p, row_bytes, row_bytes, (size_t)(y1 - y0),
+                                 cudaMemcpyDefault, st));
+        }
+    }
+    CU(cudaStreamSynchronize(st));
+}
+
+}  // namespace
+
+extern "C" {
+
 int mosaic_build_photomosaic(mosaic_generator *g, const uint8_t background_bgra[4], uint8_t *out_bgra, int rows, int cols, size_t row_stride)
 {
     return guard(g, "buildPhotomosaic", [&] {
@@ -1834,74 +1932,58 @@ int mosaic_build_photomosaic(mosaic_generator *g, const uint8_t background_bgra[
             throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "library images must be at the cell size"};
         if (g->lib_stored_size != g->lib_size)
             throw Fail{MOSAIC_ERR_NOT_READY, "buildPhotomosaic needs the library at the cell size (it was uploaded at the detail size "
-                                             "by mosaic_set_library_shard)"};
-        cudaStream_t st = g->stream;
-        const int H = g->img_rows, W = g->img_cols, n_steps = (int)g->grid.size();
-        const int64_t N = g->n_lib;
-        // the grid holds slots j * N + i of the generate's orientations: image i, placed mirrored by orientation j
-        const int fl = std::max(g->fits_flips, 0), O = orient_count(fl);
-        DevBuf owner, out, d_steps;
-        std::vector<DevBuf> libs(n_steps), cells(n_steps), masks(n_steps);
-        std::vector<BuildStep> hsteps(n_steps);
-        owner.alloc((size_t)H * W * sizeof(unsigned long long), st);
-        CU(cudaMemsetAsync(owner.p, 0, owner.bytes, st));
-        const uint8_t *lib_prev = g->d_lib_u8.as<uint8_t>();
-        int S_prev = g->lib_size;
-        for (int s = 0; s < n_steps; ++s) {
-            const Shape &shape = g->group.cells[s];
-            const GridStep &gs = g->grid[s];
-            // library at this step: halved like batchResizeMat(libImg) (8U INTER_AREA, round(0.5 * size))
-            const uint8_t *lib_s = lib_prev;
-            int S = S_prev;
-            if (s > 0) {
-                S = (int)lround(0.5 * S_prev);
-                // the 2 x 2 halving is exact in integers and commutes with mirroring; the fractional table of an odd size need not
-                if (O > 1 && S_prev % 2 != 0)
-                    throw Fail{MOSAIC_ERR_UNSUPPORTED, "mirrored tiles at an odd cell size (" + std::to_string(S_prev) + ") of step " +
-                                                           std::to_string(s - 1) + ": halving it does not commute with mirroring"};
-                libs[s].alloc((size_t)N * S * S * 3, st);
-                if (S_prev % 2 == 0) {
-                    CU(launch_area_u8(lib_prev, libs[s].as<uint8_t>(), N, S_prev, 2, st));
-                } else {
-                    mosaic_timings scratch{};
-                    const AreaTab tab = upload_area_table(g, S_prev, S, scratch);
-                    CU(launch_area_general_u8(lib_prev, libs[s].as<uint8_t>(), N, S_prev, S, tab, st));
-                }
-                lib_s = libs[s].as<uint8_t>();
-            }
-            if (S != shape.size)
-                throw Fail{MOSAIC_ERR_UNSUPPORTED, "library and cell size disagree at step " + std::to_string(s) +
-                                                       " (the reference copies out of range here)"};
-            std::vector<BuildCell> hc;
-            for (int y = 0; y < gs.rows; ++y)
-                for (int x = 0; x < gs.cols; ++x) {
-                    const int64_t v = gs.v[(size_t)y * gs.cols + x];
-                    if (v < 0)
-                        continue;
-                    if (v >= O * N)
-                        throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "best fit index outside the library"};
-                    const Rect r = rect_at(shape, x - kPadGrid, y - kPadGrid);
-                    hc.push_back(BuildCell{r.x, r.y, flip_at(shape, x - kPadGrid, y - kPadGrid), (int)hc.size() + 1, (int)(v % N),
-                                           orient_code(fl, (int)(v / N))});
-                }
-            const std::vector<uint8_t> m4 = shape.masks4();
-            masks[s].alloc(m4.size(), st);
-            CU(cudaMemcpyAsync(masks[s].p, m4.data(), m4.size(), cudaMemcpyHostToDevice, st));
-            cells[s].alloc(std::max<size_t>(hc.size(), 1) * sizeof(BuildCell), st);
-            CU(cudaMemcpyAsync(cells[s].p, hc.data(), hc.size() * sizeof(BuildCell), cudaMemcpyHostToDevice, st));
-            CU(launch_build_scatter(cells[s].as<BuildCell>(), (int)hc.size(), S, masks[s].as<uint8_t>(), H, W, s, n_steps,
-                                    owner.as<unsigned long long>(), st));
-            hsteps[s] = BuildStep{cells[s].as<BuildCell>(), lib_s, S};
-            lib_prev = lib_s;
-            S_prev = S;
+                                             "by mosaic_set_library_shard; mosaic_build_photomosaic_scaled builds from a render library)"};
+        build_mosaic(g, g->d_lib_u8.as<uint8_t>(), 1, background_bgra, out_bgra, row_stride);
+    });
+}
+
+int mosaic_set_render_library(mosaic_generator *g, const uint8_t *bgr, int64_t n, int size)
+{
+    return guard(g, "setRenderLibrary", [&] {
+        if (n < 0 || size < 1 || (n > 0 && !bgr))
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "render library must hold n >= 0 square 8U BGR images of size >= 1 (n = 0 clears it)"};
+        g->render_n = 0;
+        g->render_size = 0;
+        if (n == 0) {
+            g->d_render.release();
+            return;
         }
-        d_steps.alloc(hsteps.size() * sizeof(BuildStep), st);
-        CU(cudaMemcpyAsync(d_steps.p, hsteps.data(), d_steps.bytes, cudaMemcpyHostToDevice, st));
-        out.alloc((size_t)H * W * 4, st);
-        CU(launch_build_gather(owner.as<unsigned long long>(), H, W, n_steps, d_steps.as<BuildStep>(), background_bgra, out.as<uint8_t>(),
-                               (size_t)W, st));
-        CU(cudaMemcpy2DAsync(out_bgra, row_stride, out.p, (size_t)W * 4, (size_t)W * 4, H, cudaMemcpyDefault, st));
-        CU(cudaStreamSynchronize(st));
+        g->d_render.alloc((size_t)n * size * size * 3, g->stream);
+        CU(cudaMemcpyAsync(g->d_render.p, bgr, g->d_render.bytes, cudaMemcpyDefault, g->stream));  // host or device pointer
+        CU(cudaStreamSynchronize(g->stream));
+        g->render_n = n;
+        g->render_size = size;
+    });
+}
+
+int mosaic_build_photomosaic_scaled(mosaic_generator *g, const uint8_t background_bgra[4], uint8_t *out_bgra, int rows, int cols,
+                                    size_t row_stride)
+{
+    return guard(g, "buildPhotomosaicScaled", [&] {
+        if (!background_bgra || !out_bgra)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "background and output must not be NULL"};
+        if (g->render_n == 0)
+            throw Fail{MOSAIC_ERR_NOT_READY, "no render library (mosaic_set_render_library)"};
+        if (g->grid.empty() || !g->have_group || g->n_lib == 0 || g->fits_flips < 0)
+            throw Fail{MOSAIC_ERR_NOT_READY, "no best fits on the current grid state to build from"};
+        const int S = g->group.cells[0].size;
+        if (g->render_n != g->n_lib)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "render library holds " + std::to_string(g->render_n) + " images, the library " +
+                                                        std::to_string(g->n_lib)};
+        if (g->render_size % S != 0)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "render size " + std::to_string(g->render_size) + " is not a multiple of the cell size " +
+                                                        std::to_string(S)};
+        const int64_t k = g->render_size / S, kH = k * g->img_rows, kW = k * g->img_cols;
+        if (kH > INT32_MAX || kW > INT32_MAX)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "output of " + std::to_string(kH) + " x " + std::to_string(kW) + " (scale " +
+                                                        std::to_string(k) + ") does not fit int"};
+        if (rows != kH || cols != kW)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "output must be " + std::to_string(kH) + " x " + std::to_string(kW) + " (scale " +
+                                                        std::to_string(k) + "), got " + std::to_string(rows) + " x " + std::to_string(cols)};
+        if (row_stride < (size_t)cols * 4 || row_stride % 4 != 0)
+            throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "row stride " + std::to_string(row_stride) + " must be a multiple of 4 and at least " +
+                                                        std::to_string((size_t)cols * 4)};
+        build_mosaic(g, g->d_render.as<uint8_t>(), (int)k, background_bgra, out_bgra, row_stride);
     });
 }
 

@@ -241,13 +241,15 @@ struct BuildCell {
 };
 struct BuildStep {
     const BuildCell *cells;  // indexed by raster - 1
-    const uint8_t *lib;      // 8U BGR library at this step's cell size, [N][S][S][3]
-    int S;
+    const uint8_t *lib;      // 8U BGR (render) library of this step, [N][side][side][3]
+    int side;                // k * S_s: the step's cell size at the output scale k
 };
 cudaError_t launch_build_scatter(const BuildCell *cells, int n_cells, int S, const uint8_t *masks4, int H, int W, int step, int n_steps,
                                  unsigned long long *owner, cudaStream_t stream);
-cudaError_t launch_build_gather(const unsigned long long *owner, int H, int W, int n_steps, const BuildStep *steps, const uint8_t bgra[4],
-                                uint8_t *out, size_t out_stride_px, cudaStream_t stream);
+// rows [y_begin, y_end) of the BGRA mosaic at k times the owner map's size (cols = k * W) into out, row y_begin first, out_stride
+// bytes per row; bytes past cols * 4 in a row are not written. out and out_stride must be multiples of 4 bytes.
+cudaError_t launch_build_gather(const unsigned long long *owner, int W, int k, int n_steps, const BuildStep *steps, const uint8_t bgra[4],
+                                int y_begin, int y_end, int cols, uint8_t *out, size_t out_stride, cudaStream_t stream);
 
 // ---- select_kernels.cu
 cudaError_t launch_fill_u64(unsigned long long *p, size_t n, unsigned long long v, cudaStream_t stream);

@@ -335,6 +335,54 @@ class PhotomosaicGenerator:
         self._ck(self._L.mosaic_build_photomosaic(self._h, bg.ctypes.data, out.ctypes.data, rows, cols, out.strides[0]))
         return out
 
+    # ---- scaled compositing (no reference counterpart, include/mosaic_b200.h "scaled compositing")
+    def setRenderLibrary(self, lib):
+        """lib: N x R x R x 3 uint8, the library's images in the same order at R = k * cell size (or None to clear). The build at k
+        times the main image's size places these tiles; matching is unchanged. An aligned pair comes from two ImageLibrary objects
+        with the same seed, fed the same images, at sizes S and k * S: ImageLibrary(S), ImageLibrary(k * S), addImage on both."""
+        if lib is None:
+            self._render_size = None
+            self._ck(self._L.mosaic_set_render_library(self._h, None, 0, 1))
+            return
+        arr = np.ascontiguousarray(np.stack(lib) if isinstance(lib, (list, tuple)) else lib)
+        if arr.dtype != np.uint8 or arr.ndim != 4 or arr.shape[3] != 3 or arr.shape[1] != arr.shape[2]:
+            raise ValueError("render library must be N x R x R x 3 uint8")
+        self.setRenderLibraryPtr(arr.ctypes.data, arr.shape[0], arr.shape[1])
+
+    def setRenderLibraryPtr(self, ptr: int, n: int, size: int):
+        """Same as setRenderLibrary from a raw host or device pointer (e.g. a torch tensor's data_ptr()). The handle copies on its
+        own stream, which does not wait for torch's: call torch.cuda.synchronize() after the kernels that wrote device data."""
+        self._render_size = None
+        self._ck(self._L.mosaic_set_render_library(self._h, ptr, n, size))
+        self._render_size = int(size) if n else None
+
+    def buildPhotomosaicScaled(self, backgroundColour=(0, 0, 0, 0), out=None):
+        """buildPhotomosaic at k = R / S times the main image's size from the render library: (k * H) x (k * W) x 4 uint8 BGRA.
+        out: a preallocated array of that shape -- numpy, or a torch tensor on the host or the GPU -- with 4-byte pixels and any row
+        stride (bytes past the pixels of a row are left alone); it is filled and returned, so a multi-GB mosaic needs no second buffer.
+        The handle writes it on its own stream: work of other streams on a CUDA `out` must be finished first."""
+        rows, cols = self._main_shape
+        k = self._render_size // self._cell_size() if getattr(self, "_render_size", None) else 1
+        shape = (k * rows, k * cols, 4)
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        if tuple(out.shape) != shape:
+            raise ValueError("out must be %d x %d x 4" % shape[:2])
+        if isinstance(out, np.ndarray):
+            ptr, strides, itemsize = out.ctypes.data, out.strides, out.itemsize
+        else:  # torch.Tensor: strides in elements
+            ptr, strides, itemsize = out.data_ptr(), tuple(s * out.element_size() for s in out.stride()), out.element_size()
+        if itemsize != 1 or strides[1] != 4 or strides[2] != 1:
+            raise ValueError("out must be uint8 with contiguous BGRA pixels")
+        bg = np.asarray(backgroundColour, np.uint8)
+        self._ck(self._L.mosaic_build_photomosaic_scaled(self._h, bg.ctypes.data, ptr, shape[0], shape[1], strides[0]))
+        return out
+
+    def _cell_size(self) -> int:
+        c = CellShapeC()
+        self._ck(self._L.mosaic_get_cell_shape(self._h, 0, 0, ctypes.byref(c), None, 0))
+        return c.size
+
     def getMaxProgress(self) -> int:
         return self._L.mosaic_get_max_progress(self._h)
 
