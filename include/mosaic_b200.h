@@ -268,6 +268,29 @@ int mosaic_kernel_hue_rotate(int device, const uint8_t *bgr, int rows, int cols,
 int mosaic_kernel_resize_area_u8(int device, const uint8_t *src, int64_t n, int size, int k, uint8_t *dst);
 int mosaic_kernel_resize_area_f32(int device, const float *src, int64_t n, int size, int k, float *dst);
 int mosaic_kernel_resize_cubic_u8(int device, const uint8_t *src, int src_h, int src_w, int cn, uint8_t *dst, int dst_h, int dst_w);
+/* The packed inputs of the difference kernels at size step `step`, as a generate on this handle would build them (test tap of the
+ * preprocessing): main image variants, library preparation and colour order, and the packing of steps 0 .. step (the working
+ * library is halved step by step). No difference or selection kernel runs and the handle's results are kept.
+ * info always; cells / lib (cell_bytes / lib_bytes, raw tile layout of csrc/diff_kernels.cu or csrc/diff_euclid.cu),
+ * pix_list (n_active compacted pixel indices) and perm (n_lib_tiles * slots_per_tile slot -> image, only when has_perm) when
+ * non-NULL. Call with NULL buffers first to size them (the preprocessing runs either way); MOSAIC_ERR_INVALID_ARGUMENT when
+ * cells_cap or lib_cap is too small. */
+typedef struct mosaic_step_inputs {
+    int layout;       /* 0: CIEDE2000 tiles (csrc/diff_kernels.cu), 1: Euclidean tiles (csrc/diff_euclid.cu) */
+    int n_variants;   /* difference rows per cell (colour-scheme variants compared) */
+    int n_active, n_chunks;
+    int n_rows;       /* this handle's rows: its valid cells x n_variants, raster order, variant fastest */
+    int n_cell_tiles;
+    int64_t n_slots;  /* library slots: orientations x images, orientation-major */
+    int n_lib_tiles;
+    int cells_per_tile, slots_per_tile, pixels_per_chunk;
+    size_t cell_bytes, lib_bytes;
+    int fused;        /* one size step: the library packer reads the 8U library and converts on the fly */
+    int fused_k;      /* integer reduction the fused packer applies to the stored library (1: none) */
+    int has_perm;     /* library tiles in colour order (CIEDE2000 row passes): slot i holds image perm[i] */
+} mosaic_step_inputs;
+int mosaic_debug_step_inputs(mosaic_generator *g, int step, mosaic_step_inputs *info, void *cells, size_t cells_cap, void *lib,
+                             size_t lib_cap, int32_t *pix_list, int32_t *perm);
 
 /* ---- on-disk containers of the reference (Qt-free, OpenCV-free: QDataStream layout and PNG codec inside the library).
  * A file the reference would reject with std::invalid_argument gives MOSAIC_ERR_INVALID_ARGUMENT; mosaic_io_last_error() has

@@ -24,6 +24,14 @@ class Timings(ctypes.Structure):
                 ("kernel_launches", ctypes.c_int64), ("evaluated_pixel_diffs", ctypes.c_double)]
 
 
+class StepInputs(ctypes.Structure):
+    _fields_ = [("layout", ctypes.c_int), ("n_variants", ctypes.c_int), ("n_active", ctypes.c_int), ("n_chunks", ctypes.c_int),
+                ("n_rows", ctypes.c_int), ("n_cell_tiles", ctypes.c_int), ("n_slots", ctypes.c_int64), ("n_lib_tiles", ctypes.c_int),
+                ("cells_per_tile", ctypes.c_int), ("slots_per_tile", ctypes.c_int), ("pixels_per_chunk", ctypes.c_int),
+                ("cell_bytes", ctypes.c_size_t), ("lib_bytes", ctypes.c_size_t), ("fused", ctypes.c_int), ("fused_k", ctypes.c_int),
+                ("has_perm", ctypes.c_int)]
+
+
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_int, ctypes.c_void_p)
 
 _lib = None
@@ -120,6 +128,7 @@ def capi():
         "mosaic_host_resize_area_u8": (i, [vp, i, i, i, vp, i, i]),
         "mosaic_host_resize_cubic_u8": (i, [vp, i, i, i, vp, i, i]),
         "mosaic_kernel_resize_cubic_u8": (i, [i, vp, i, i, i, vp, i, i]),
+        "mosaic_debug_step_inputs": (i, [vp, i, c.POINTER(StepInputs), vp, sz, vp, sz, vp, vp]),
         "mosaic_library_ingest": (i, [i, vp, i, i, sz, i, vp]),
     }
     for name, (res, args) in sig.items():

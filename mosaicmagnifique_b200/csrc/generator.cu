@@ -1190,18 +1190,11 @@ void select_phase(G *g, const Run &r, size_t s, const StepWork &w, mosaic_timing
                 nullptr, tm);
 }
 
-void run_pipeline(G *g, bool candidates_only)
+// what a generate decides once (Run) and, on first use, the Lab LUT upload. Sets the handle's V_eff, n_slots and (unless
+// candidates_only) fits_flips.
+Run setup_run(G *g, bool candidates_only, mosaic_timings &tm)
 {
-    check_ready(g);
-    if (g->is_cancelled())  // sticky like m_wasCanceled (never reset by the reference): nothing runs until mosaic_reset_cancel
-        throw Fail{MOSAIC_ERR_CANCELLED, "cancelled"};
-    make_plans(g);
-    check_usage_limit(g);
     cudaStream_t st = g->stream;
-    const auto t_host0 = std::chrono::steady_clock::now();
-    g->timings = mosaic_timings{};
-    mosaic_timings &tm = g->timings;
-    const size_t n_steps = g->grid.size();
     Run r;
     r.candidates_only = candidates_only;
     r.rotations = colour_variants(g);
@@ -1229,8 +1222,6 @@ void run_pipeline(G *g, bool candidates_only)
     // CIEDE2000 steps that need D run as segment passes over row work lists; the library tiles then hold the library in colour
     // order (kernels.h: RowList), which is what lets exact pruning drop whole tiles of a cell
     r.row_passes = r.layout == kLayoutCiede && !r.fused_argmin;
-    PhaseClock clock(st);
-    enum { kPre = 0, kDiff = 1, kSel = 2 };
 
     if (!g->d_lut.p) {
         const std::vector<int16_t> lut4 = expand_lab_lut(mm_lab_lut_s16);
@@ -1239,6 +1230,38 @@ void run_pipeline(G *g, bool candidates_only)
         CU(cudaStreamSynchronize(st));  // lut4 is a local
         tm.h2d_bytes += (double)g->d_lut.bytes;
     }
+    return r;
+}
+
+// colour order of the library (kernels.h: RowList) when the CIEDE2000 steps run as row passes: ws.perm / ws.inv_perm
+void library_order(G *g, const Run &r, const LibSource &lib, mosaic_timings &tm)
+{
+    if (!r.row_passes)
+        return;
+    cudaStream_t st = g->stream;
+    g->ws.perm.alloc((size_t)r.n_lib_pad * sizeof(int), st);
+    g->ws.inv_perm.alloc((size_t)r.n_lib_pad * sizeof(int), st);
+    g->ws.order_scratch.alloc(library_order_scratch_bytes(r.N), st);
+    CU(launch_library_order(lib.oriented, g->lib_stored_size, r.N, r.n_lib_pad, g->ws.perm.as<int>(), g->ws.inv_perm.as<int>(),
+                            g->ws.order_scratch.p, g->ws.order_scratch.bytes, st));
+    tm.kernel_launches += 3;
+}
+
+void run_pipeline(G *g, bool candidates_only)
+{
+    check_ready(g);
+    if (g->is_cancelled())  // sticky like m_wasCanceled (never reset by the reference): nothing runs until mosaic_reset_cancel
+        throw Fail{MOSAIC_ERR_CANCELLED, "cancelled"};
+    make_plans(g);
+    check_usage_limit(g);
+    cudaStream_t st = g->stream;
+    const auto t_host0 = std::chrono::steady_clock::now();
+    g->timings = mosaic_timings{};
+    mosaic_timings &tm = g->timings;
+    const size_t n_steps = g->grid.size();
+    const Run r = setup_run(g, candidates_only, tm);
+    PhaseClock clock(st);
+    enum { kPre = 0, kDiff = 1, kSel = 2 };
 
     clock.begin(kPre);
     main_to_working_space(g, r, tm);
@@ -1257,14 +1280,7 @@ void run_pipeline(G *g, bool candidates_only)
         g->cand_max_uses = g->max_uses;
         g->cap_last_step = -1;
     }
-    if (r.row_passes) {
-        g->ws.perm.alloc((size_t)r.n_lib_pad * sizeof(int), st);
-        g->ws.inv_perm.alloc((size_t)r.n_lib_pad * sizeof(int), st);
-        g->ws.order_scratch.alloc(library_order_scratch_bytes(r.N), st);
-        CU(launch_library_order(lib.oriented, g->lib_stored_size, r.N, r.n_lib_pad, g->ws.perm.as<int>(), g->ws.inv_perm.as<int>(),
-                                g->ws.order_scratch.p, g->ws.order_scratch.bytes, st));
-        tm.kernel_launches += 3;
-    }
+    library_order(g, r, lib, tm);
     Progress prog(g);
     for (size_t s = 0; s < n_steps; ++s) {
         prog.check_cancel();
@@ -1291,6 +1307,75 @@ void run_pipeline(G *g, bool candidates_only)
     tm.diff_ms = clock.sum(kDiff);
     tm.select_ms = clock.sum(kSel);
     tm.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
+}
+
+// mosaic_debug_step_inputs: a generate's preprocessing up to the packing of `step`, then the packed tensors copied back. The
+// handle's results (plans, grid, D, margins, candidates, timings, the slot count and variant count of the last generate) are kept.
+void step_inputs(G *g, int step, mosaic_step_inputs *info, void *cells, size_t cells_cap, void *lib_out, size_t lib_cap,
+                 int32_t *pix_list, int32_t *perm)
+{
+    check_ready(g);
+    if (step < 0 || step >= (int)g->grid.size())
+        throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "step " + std::to_string(step) + " is outside the grid state's " +
+                                                    std::to_string(g->grid.size()) + " steps"};
+    struct Keep {
+        G *g;
+        std::vector<StepPlan> plans;
+        int V_eff, fits_flips;
+        int64_t n_slots;
+        ~Keep()
+        {
+            g->plans.swap(plans);
+            g->V_eff = V_eff;
+            g->fits_flips = fits_flips;
+            g->n_slots = n_slots;
+        }
+    } keep{g, g->plans, g->V_eff, g->fits_flips, g->n_slots};
+    make_plans(g);
+    check_usage_limit(g);
+    cudaStream_t st = g->stream;
+    mosaic_timings tm{};
+    const Run r = setup_run(g, false, tm);
+    main_to_working_space(g, r, tm);
+    const LibSource lib = prepare_library(g, r, tm);
+    library_order(g, r, lib, tm);
+    StepWork w;
+    for (int s = 0; s <= step; ++s)
+        prepare_step(g, r, lib, s, w, tm);
+
+    const StepPlan &p = g->plans[step];
+    mosaic_step_inputs in{};
+    in.layout = r.layout;
+    in.n_variants = r.V;
+    in.n_active = p.n_active;
+    in.n_chunks = p.n_chunks;
+    in.n_rows = w.n_rows_local;
+    in.n_cell_tiles = w.n_cell_tiles;
+    in.n_slots = r.N;
+    in.n_lib_tiles = r.n_lib_tiles;
+    in.cells_per_tile = r.tg.tcb;
+    in.slots_per_tile = r.tg.tnb;
+    in.pixels_per_chunk = r.tg.kp;
+    in.cell_bytes = (size_t)w.n_cell_tiles * p.n_chunks * r.tg.cell_block;
+    in.lib_bytes = (size_t)r.n_lib_tiles * p.n_chunks * r.tg.lib_block;
+    in.fused = lib.fused;
+    in.fused_k = lib.fused_k;
+    in.has_perm = r.row_passes;
+    if (info)
+        *info = in;
+    if ((cells && cells_cap < in.cell_bytes) || (lib_out && lib_cap < in.lib_bytes))
+        throw Fail{MOSAIC_ERR_INVALID_ARGUMENT, "buffers hold " + std::to_string(cells_cap) + " / " + std::to_string(lib_cap) +
+                                                    " bytes, the packed cells / library need " + std::to_string(in.cell_bytes) + " / " +
+                                                    std::to_string(in.lib_bytes)};
+    if (cells)
+        CU(cudaMemcpyAsync(cells, g->ws.cells_packed.p, in.cell_bytes, cudaMemcpyDeviceToHost, st));
+    if (lib_out)
+        CU(cudaMemcpyAsync(lib_out, g->ws.lib_packed.p, in.lib_bytes, cudaMemcpyDeviceToHost, st));
+    if (pix_list)
+        CU(cudaMemcpyAsync(pix_list, g->ws.pix_list.p, (size_t)p.n_active * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (perm && r.row_passes)
+        CU(cudaMemcpyAsync(perm, g->ws.perm.p, (size_t)r.n_lib_pad * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
 }
 
 }  // namespace
@@ -1823,6 +1908,12 @@ int mosaic_get_timings(const mosaic_generator *g, mosaic_timings *out)
         return MOSAIC_ERR_INVALID_ARGUMENT;
     *out = g->timings;
     return MOSAIC_OK;
+}
+
+int mosaic_debug_step_inputs(mosaic_generator *g, int step, mosaic_step_inputs *info, void *cells, size_t cells_cap, void *lib,
+                             size_t lib_cap, int32_t *pix_list, int32_t *perm)
+{
+    return guard(g, "debugStepInputs", [&] { step_inputs(g, step, info, cells, cells_cap, lib, lib_cap, pix_list, perm); });
 }
 
 // ---- buildPhotomosaic (PhotomosaicGeneratorBase.cpp:110-207)
